@@ -1,6 +1,6 @@
 """bench.py - DCT importance-score throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--net resnet_50]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--net resnet_50] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -24,6 +24,11 @@ all-reduce, the finalise kernel and the segmented top-k, all inside the timed re
 `--impl reference` times the reference's CPU implementation (oracle/reference_port.py: the
 reference is pure Python and its DCT dependency torch_dct is absent, so the port is the runnable
 form) on a bounded sample per step, rank 0 only.
+
+`--dump-outputs DIR` writes, after the timed steps of the headline net and of the U^2-Netp legs, what the timed run handed
+back: DIR/<net>_<side>.score.<file>.npy (float32, one per score file) and DIR/<net>_<side>.kept.<file>.npy (kept channel
+ids as float64, one per pruned layer).  Images, weights and the cuDNN forward that makes the scored activations are seeded
+and deterministic, so two runs or two builds with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -75,6 +80,9 @@ def parse():
     p.add_argument('--no-u2netp', action='store_true', help='skip the U^2-Netp 320/288 summary (BASELINE config 5)')
     p.add_argument('--per-site', action='store_true', help='one launch per hook site in the timed steps too (no multi-site launches): the form the ncu launch list is taken in, so that bytes per launch compare with the per-site algorithmic bytes')
     p.add_argument('--graph', action='store_true', help='replay CUDA graphs (hook launches of a step; forward + hooks in the e2e leg): takes the host out of launch-bound nets')
+    p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                   help='after the timed steps, write what they computed (per-file scores, kept channel ids) as DIR/<name>.npy, '
+                        'for comparing two builds output for output')
     return p.parse_args()
 
 
@@ -176,8 +184,20 @@ def site_roofline(shape, scored_channels, hbm_gbs, tflops):
     return nbytes, flops, max(t_mem, t_mma), ('hbm' if t_mem >= t_mma else 'tensor')
 
 
-def measure_net(args, net_name, side, B, rank, local_rank, world, device, lib, steps, with_e2e, npy_dir=None, clock_sampler=None):
-    """Kernel-only and end-to-end legs for one net at per-rank batch B.  Returns a dict (all times already max over ranks)."""
+def dump_outputs(directory, tag, session, plan, scores, kept):
+    """The result of the timed run as its caller receives it: every score file's vector (float32, what ScoreSession.finalize
+    returns) and every selection's kept channel ids (int64 on the device, stored as float64: exact).  A few hundred kB per net."""
+    os.makedirs(directory, exist_ok=True)
+    for stem, vec in session.split_files(scores.cpu().numpy()).items():
+        np.save(os.path.join(directory, '%s.score.%s.npy' % (tag, stem)), vec)
+    for sel, ids in zip(plan, kept):
+        np.save(os.path.join(directory, '%s.kept.%s.npy' % (tag, sel.stem)), ids.cpu().numpy().astype(np.float64))
+
+
+def measure_net(args, net_name, side, B, rank, local_rank, world, device, lib, steps, with_e2e, npy_dir=None, clock_sampler=None,
+                dump_dir=None):
+    """Kernel-only and end-to-end legs for one net at per-rank batch B.  Returns a dict (all times already max over ranks).
+    `dump_dir`: rank 0 writes the kernel-only leg's scores and kept ids there (dump_outputs)."""
     from dct_pruning_b200 import _lib
     from dct_pruning_b200.compress import get_compress_rate, selection_plan
     from dct_pruning_b200.generate import device_batches, write_score_files
@@ -204,7 +224,9 @@ def measure_net(args, net_name, side, B, rank, local_rank, world, device, lib, s
             def cap(module, inputs, output, idx=idx, take_input=(site.variant == VARIANT_INPUT)):
                 acts[idx] = (inputs[0] if take_input else output).detach().clone()
             handles.append(resolve_module(net, site.module).register_forward_hook(cap))
-        with torch.no_grad():
+        # deterministic cuDNN algorithms (not benchmark's timing-dependent pick): the same activations from run to run, so that
+        # --dump-outputs of two runs or two builds compare output for output.  This forward is not timed.
+        with torch.no_grad(), torch.backends.cudnn.flags(enabled=True, benchmark=False, deterministic=True, allow_tf32=False):
             net(host_batch.to(device))
         for h in handles:
             h.remove()
@@ -276,11 +298,13 @@ def measure_net(args, net_name, side, B, rank, local_rank, world, device, lib, s
                 session.images[i] += B
         else:
             one_step()
-    finish_run()
+    final_scores, final_kept = finish_run()
     t1.record()
     barrier(world)
     launches = lib.dctp_launch_count() - launches0 + (steps * graph_launches if step_graph is not None else 0)
     _lib.check(lib.dctp_check(None))
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, '%s_%d' % (net_name, side), session, plan, final_scores, final_kept)
     ms_total = max_over_ranks(t0.elapsed_time(t1), device, world)
     out.update(ms_per_step=ms_total / steps, gpu_launches=int(launches), hook_sites=len(session.sites),
                activation_bytes_per_step=act_bytes, algorithmic_bytes_per_step=alg_bytes_step,
@@ -512,7 +536,7 @@ def run_ours(args):
 
     # ---- headline: batch B per GPU (weak scaling: the work per GPU is fixed)
     main = measure_net(args, args.net, side, B, rank, local_rank, world, device, lib, steps, not args.no_e2e,
-                       npy_dir=os.path.join(tmp, 'weak') if tmp else None)
+                       npy_dir=os.path.join(tmp, 'weak') if tmp else None, dump_dir=args.dump_outputs)
     acts_cpu, acts_gpu, sites = main.pop('_acts_cpu'), main.pop('_acts'), main.pop('_sites')
     value = world * B * steps / (main['ms_per_step'] * steps / 1e3)
 
@@ -556,7 +580,8 @@ def run_ours(args):
         u2 = {}
         for s_side in (320, 288):
             r = measure_net(args, 'u2netp', s_side, WORKLOADS['u2netp']['batch'], rank, local_rank, world, device, lib, steps,
-                            (not args.no_e2e) and s_side == 320, npy_dir=os.path.join(tmp, 'u2netp%d' % s_side) if tmp else None)
+                            (not args.no_e2e) and s_side == 320, npy_dir=os.path.join(tmp, 'u2netp%d' % s_side) if tmp else None,
+                            dump_dir=args.dump_outputs)
             for k in ('_acts_cpu', '_acts', '_sites'):
                 r.pop(k)
             r['value'] = world * r['batch_per_gpu'] / (r['ms_per_step'] / 1e3)
@@ -703,6 +728,8 @@ def run_reference(args):
 if __name__ == '__main__':
     a = parse()
     if a.impl == 'reference':
+        if a.dump_outputs:
+            raise SystemExit('--dump-outputs writes what the CUDA path computed; it has no meaning with --impl reference')
         run_reference(a)
     else:
         if not torch.cuda.is_available():
