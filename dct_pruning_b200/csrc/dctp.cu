@@ -78,21 +78,9 @@ struct State {
     std::map<int, LargeBasis> large;                   // N
     std::map<int, StackBasis> stack;                   // N
     std::map<int, KronBasis> kron;                     // N
-    bool kron_on = true;                               // AUTO routes dense sides <= 8 to the Kronecker kernel (DCTP_KRON=0: round-1 kernels)
-    int stack_cfg = 0;                                 // role layout of the stacked-basis kernel (DCTP_STACK_CFG, see stack_kernel_fn; 0: per side)
-    bool stack_on = true;                              // AUTO routes dense even sides to the stacked-basis kernel (DCTP_STACK=0: round-1 kernels)
-    long long stack_min_bytes = 0;                     // ... for launches of at least this many bytes (DCTP_STACK_MIN_MB)
+    std::vector<void*> bases;                          // every device allocation of the basis caches above (dctp_shutdown frees them)
     void* encode_tiled = nullptr;                      // cuTensorMapEncodeTiled, resolved through the runtime (no libcuda link dependency)
-    int t_slots = 3;                                   // tile slots per CTA of the TMEM-operand kernel (DCTP_T_SLOTS=0 disables it)
-    bool t_all = false;
-    bool t_prod = true;                                // 3-slot TMEM-operand kernel with two producer warpgroups where the tile fits
-                                                       // (52x52, 56x56; DCTP_TP=0 turns it off): ResNet-50 step 3.30 -> 3.15 ms
     bool pdl = true;                                   // programmatic dependent launch of the score kernels (DCTP_PDL=0 disables)
-    int t_auto_lo = 52;                                // sides from here up always go to the TMEM-operand kernel under AUTO (DCTP_T_LO)
-    int large_lo = 80;                                 // smallest side AUTO routes to the tiled large-map kernel (DCTP_LARGE_LO);
-                                                       // measured vs the smem-operand kernel, [12,64,N,N]: 80 0.92 vs 0.67 TB/s (a tie in
-                                                       // round 1, before the large kernel lost a fifth of its instructions), 96 1.22 vs 0.73
-    long long t_min_bytes = 32ll << 20;                // smaller sides only for launches of at least this many bytes (DCTP_T_MIN_MB)
     int regs[2][6][2] = {};                            // registers/thread per (KP, load mode, prefetch) instantiation
     // scratch of dctp_score_host (grow-only)
     float* hx = nullptr; size_t hx_bytes = 0;
@@ -131,6 +119,17 @@ inline void split_bf16(double c, uint16_t& hi, uint16_t& lo) {
     lo = bf16_rn(static_cast<float>(c - static_cast<double>(bf16_to_f(hi))));
 }
 
+// device copy of a host-built basis table; the allocation is recorded before anything can fail, so dctp_shutdown frees it
+template <typename T>
+int upload(const std::vector<T>& host, T*& dev) {
+    void* p = nullptr;
+    CUDA_TRY(cudaMalloc(&p, host.size() * sizeof(T)));
+    g.bases.push_back(p);
+    dev = static_cast<T*>(p);
+    CUDA_TRY(cudaMemcpy(p, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice));
+    return DCTP_OK;
+}
+
 int get_umma_basis(int N, int KP, UmmaBasis& out) {
     auto key = std::make_pair(N, KP);
     auto it = g.umma.find(key);
@@ -142,10 +141,8 @@ int get_umma_basis(int N, int KP, UmmaBasis& out) {
             for (int w = 0; w < N; ++w)
                 split_bf16(dct_coef(v, w, N), hi[(size_t)(j * Ms + v) * KP + j * Ms + w], lo[(size_t)(j * Ms + v) * KP + j * Ms + w]);
     UmmaBasis b;
-    CUDA_TRY(cudaMalloc(&b.hi, hi.size() * 2));
-    CUDA_TRY(cudaMalloc(&b.lo, lo.size() * 2));
-    CUDA_TRY(cudaMemcpy(b.hi, hi.data(), hi.size() * 2, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.lo, lo.data(), lo.size() * 2, cudaMemcpyHostToDevice));
+    int rc;
+    if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
     // scatter table of the dense load path: where element e of a full tile (maps back to back) lands in A1
     const int G = 128 / Ms, MT = G * J, NN = N * N;
     if ((MT * NN) % 4 == 0) {
@@ -159,8 +156,7 @@ int get_umma_basis(int N, int KP, UmmaBasis& out) {
                 tab[(size_t)v * b.vpe + s] =
                     static_cast<uint16_t>(detail::kmajor_off((t / J) * Ms + r / N, (t % J) * Ms + r % N, 128));
             }
-        CUDA_TRY(cudaMalloc(&b.scatter, tab.size() * 2));
-        CUDA_TRY(cudaMemcpy(b.scatter, tab.data(), tab.size() * 2, cudaMemcpyHostToDevice));
+        if ((rc = upload(tab, b.scatter))) return rc;
     }
     g.umma[key] = b;
     out = b;
@@ -199,16 +195,10 @@ int get_t_basis(int N, TBasis& out) {
             const int e = 4 * v + sI * step, t = e / NN, r = e % NN, gI = t / J, j = t % J;
             tab[(size_t)v * b.vpe + sI] = static_cast<uint16_t>(detail::kmajor_off(j * Ms + r / N, gI * N + r % N, rows));
         }
-    CUDA_TRY(cudaMalloc(&b.a_hi, ahi.size() * 4));
-    CUDA_TRY(cudaMalloc(&b.a_lo, alo.size() * 4));
-    CUDA_TRY(cudaMalloc(&b.c_hi, chi.size() * 2));
-    CUDA_TRY(cudaMalloc(&b.c_lo, clo.size() * 2));
-    CUDA_TRY(cudaMalloc(&b.scatter, tab.size() * 2));
-    CUDA_TRY(cudaMemcpy(b.a_hi, ahi.data(), ahi.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.a_lo, alo.data(), alo.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.c_hi, chi.data(), chi.size() * 2, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.c_lo, clo.data(), clo.size() * 2, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.scatter, tab.data(), tab.size() * 2, cudaMemcpyHostToDevice));
+    int rc;
+    if ((rc = upload(ahi, b.a_hi)) || (rc = upload(alo, b.a_lo)) || (rc = upload(chi, b.c_hi)) || (rc = upload(clo, b.c_lo)) ||
+        (rc = upload(tab, b.scatter)))
+        return rc;
     g.tmem[N] = b;
     out = b;
     return DCTP_OK;
@@ -288,57 +278,45 @@ int get_stack_basis(int N, StackBasis& out) {
     fill(b.lbo1);
     b.table_bytes = static_cast<uint32_t>((static_cast<size_t>(b.tile_vec) * pieces * 2 + 15) / 16 * 16);
     if (b.table_bytes > S::TABLE_MAX) return fail(DCTP_E_UNSUPPORTED, "stacked-basis kernel: offset table of side %d does not fit", N);
-    CUDA_TRY(cudaMalloc(&b.a_img, img.size() * 4));
-    CUDA_TRY(cudaMalloc(&b.c2_hi, chi.size()));
-    CUDA_TRY(cudaMalloc(&b.c2_lo, clo.size()));
-    CUDA_TRY(cudaMalloc(&b.table, tab.size() * 2));
-    CUDA_TRY(cudaMemcpy(b.a_img, img.data(), img.size() * 4, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.c2_hi, chi.data(), chi.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.c2_lo, clo.data(), clo.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.table, tab.data(), tab.size() * 2, cudaMemcpyHostToDevice));
+    int rc;
+    if ((rc = upload(img, b.a_img)) || (rc = upload(chi, b.c2_hi)) || (rc = upload(clo, b.c2_lo)) || (rc = upload(tab, b.table))) return rc;
     g.stack[N] = b;
     out = b;
     return DCTP_OK;
 }
 
 // instantiations: variant v = (KP, VEC, Np / 8) - (16,4,2) (16,2,2) (32,4,3) (32,4,4) (32,2,3) (32,2,4) (48,4,5) (48,4,6) (64,4,7) (64,4,8);
-// configuration cfg = role layout (one epilogue-1 group of 8 warps, two epilogue-2 groups of 4, producer, two issuers):
-//   cfg 4: 8 converter warps in two groups (alternate tiles), 27 warps        cfg 7: 12 converter warps (two groups of 6), 31 warps
-//   cfg 6: cfg 4 with the debug outputs compiled in (DCTP_S_TRACE cycle accounting, per-map energies, coefficient dump); the host
-//          routes launches that ask for any of them here, production launches never
-// AUTO (cfg 0): cfg 7 (56x56 4.14 against 4.06 TB/s for cfg 4, 14x14 3.55 against 3.45, 28x28 equal).
+// role layout (one epilogue-1 group of 8 warps, two epilogue-2 groups of 4, producer, two issuers), named in dctp_last_kernel():
+//   cfg7: production, 12 converter warps (two groups of 6), 31 warps
+//   cfg6: debug, 8 converter warps (two groups of 4), 27 warps, with the debug outputs compiled in (DCTP_S_TRACE cycle accounting,
+//         per-map energies, coefficient dump); the host routes launches that ask for any of them here, production launches never
+// 12 converter warps won over 8 (the retired cfg 4): 56x56 4.14 against 4.06 TB/s, 14x14 3.55 against 3.45, 28x28 equal.
 // Layouts measured and retired in round 2 (same box, 56x56 / 28x28 / 14x14 TB/s, before the instruction diet): one epilogue-2 group
 // 3.73 / 3.47 / 3.19 (two: 3.73 / 3.62 / 3.25), two epilogue-1 groups 3.78 / 3.57 / 3.12, 4 converter warps 3.59 / 3.31 / 2.89;
 // after it: 16 converter warps with one epilogue-2 group 4.08 / 3.55 / 3.38 and two epilogue-1 groups with one epilogue-2 group 4.05 / 3.66 /
 // 3.40 (cfg 7: 4.14 / 3.99 / 3.55); register rebalancing (setmaxnreg: converters 56, epilogue 1 104 registers and ONE TMEM round trip per tile) 3.36 against
 // 3.61 at 56x56; converters reading global memory directly behind an L2 bulk prefetch instead of the TMA-staged copy 3.46 against 4.07.
-constexpr int STACK_CFGS = 8, STACK_VARIANTS = 10;
+constexpr int STACK_VARIANTS = 10;
 typedef void (*StackKernel)(const ScoreTensorMaps, const StackArgs);
-template <bool TRACE, int NCONV, int NE1G = 1, int NE2G = 2>
+template <bool TRACE, int NCONV>
 StackKernel stack_kernel_of(int v) {
     switch (v) {
-        case 0: return score_stack_kernel<16, 4, NCONV, NE1G, 2, NE2G, 2, TRACE>;
-        case 1: return score_stack_kernel<16, 2, NCONV, NE1G, 2, NE2G, 2, TRACE>;
-        case 2: return score_stack_kernel<32, 4, NCONV, NE1G, 2, NE2G, 3, TRACE>;
-        case 3: return score_stack_kernel<32, 4, NCONV, NE1G, 2, NE2G, 4, TRACE>;
-        case 4: return score_stack_kernel<32, 2, NCONV, NE1G, 2, NE2G, 3, TRACE>;
-        case 5: return score_stack_kernel<32, 2, NCONV, NE1G, 2, NE2G, 4, TRACE>;
-        case 6: return score_stack_kernel<48, 4, NCONV, NE1G, 2, NE2G, 5, TRACE>;
-        case 7: return score_stack_kernel<48, 4, NCONV, NE1G, 2, NE2G, 6, TRACE>;
-        case 8: return score_stack_kernel<64, 4, NCONV, NE1G, 2, NE2G, 7, TRACE>;
-        default: return score_stack_kernel<64, 4, NCONV, NE1G, 2, NE2G, 8, TRACE>;
+        case 0: return score_stack_kernel<16, 4, NCONV, 2, TRACE>;
+        case 1: return score_stack_kernel<16, 2, NCONV, 2, TRACE>;
+        case 2: return score_stack_kernel<32, 4, NCONV, 3, TRACE>;
+        case 3: return score_stack_kernel<32, 4, NCONV, 4, TRACE>;
+        case 4: return score_stack_kernel<32, 2, NCONV, 3, TRACE>;
+        case 5: return score_stack_kernel<32, 2, NCONV, 4, TRACE>;
+        case 6: return score_stack_kernel<48, 4, NCONV, 5, TRACE>;
+        case 7: return score_stack_kernel<48, 4, NCONV, 6, TRACE>;
+        case 8: return score_stack_kernel<64, 4, NCONV, 7, TRACE>;
+        default: return score_stack_kernel<64, 4, NCONV, 8, TRACE>;
     }
 }
-bool stack_cfg_valid(int cfg) { return cfg == 4 || cfg == 6 || cfg == 7; }
-StackKernel stack_kernel_fn(int cfg, int v) {
-    switch (cfg) {
-        case 6: return stack_kernel_of<true, 8>(v);
-        case 7: return stack_kernel_of<false, 12>(v);
-        default: return stack_kernel_of<false, 8>(v);
-    }
+constexpr int STACK_NCONV = 12, STACK_NCONV_DEBUG = 8;
+StackKernel stack_kernel_fn(bool debug, int v) {
+    return debug ? stack_kernel_of<true, STACK_NCONV_DEBUG>(v) : stack_kernel_of<false, STACK_NCONV>(v);
 }
-const void* stack_kernel_ptr(int cfg, int v) { return reinterpret_cast<const void*>(stack_kernel_fn(cfg, v)); }
-int stack_threads(int cfg) { return (cfg == 7 ? 31 : 27) * 32; }
 int stack_variant(int KP, int vec, int np8) {
     if (KP == 16) return vec == 4 ? 0 : 1;
     if (KP == 32) return (vec == 4 ? 2 : 4) + (np8 == 4 ? 1 : 0);
@@ -349,26 +327,51 @@ int stack_variant(int KP, int vec, int np8) {
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-template <typename Args>
-cudaError_t launch_score_tma(void (*kern)(const ScoreTensorMaps, const Args), int grid, int block, size_t smem, cudaStream_t stream,
-                             const ScoreTensorMaps& maps, const Args& args);
-
-struct SiteDesc { const float* first; int B; int c_count; double* accum; };     // one dense activation: B * c_count maps back to back
-
-// 2-D tensor map over a dense fp32 stream viewed as [rows, 32 floats] (whole 128-byte rows only), box = `box_rows` rows
-int encode_flat_map(CUtensorMap& map, const float* first, long long total_elems, int box_rows) {
+// 2-D tensor map over fp32 rows: `rows` rows of `inner` floats, `pitch` bytes apart; box = `box_inner` floats x `box_rows` rows
+int encode_2d(CUtensorMap& map, const float* base, long long inner, long long rows, long long pitch, int box_inner, int box_rows,
+              CUtensorMapL2promotion l2) {
     std::memset(&map, 0, sizeof map);
-    const long long rows = total_elems / 32;
-    if (rows <= 0) return DCTP_OK;                           // (never dereferenced: the only tile is converted from global memory)
-    cuuint64_t gdim[2] = {32, static_cast<cuuint64_t>(rows)};
-    cuuint64_t gstr[1] = {128};
-    cuuint32_t box[2] = {32, static_cast<cuuint32_t>(box_rows)}, estr[2] = {1, 1};
+    cuuint64_t gdim[2] = {static_cast<cuuint64_t>(inner), static_cast<cuuint64_t>(rows)};
+    cuuint64_t gstr[1] = {static_cast<cuuint64_t>(pitch)};
+    cuuint32_t box[2] = {static_cast<cuuint32_t>(box_inner), static_cast<cuuint32_t>(box_rows)}, estr[2] = {1, 1};
     const CUresult r = reinterpret_cast<EncodeTiledFn>(g.encode_tiled)(
-        &map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(first), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-        CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(DCTP_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for %lld rows, box %d", (int)r, rows, box_rows);
+        &map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+        CU_TENSOR_MAP_SWIZZLE_NONE, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS)
+        return fail(DCTP_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for %lld rows of %lld floats, box %d x %d", (int)r, rows, inner,
+                    box_inner, box_rows);
     return DCTP_OK;
 }
+
+// a dense fp32 stream viewed as [rows, 32 floats] (whole 128-byte rows only), box = `box_rows` rows
+int encode_flat_map(CUtensorMap& map, const float* first, long long total_elems, int box_rows) {
+    const long long rows = total_elems / 32;
+    if (rows <= 0) {                                         // (never dereferenced: the only tile is converted from global memory)
+        std::memset(&map, 0, sizeof map);
+        return DCTP_OK;
+    }
+    return encode_2d(map, first, 32, rows, 128, 32, box_rows, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+}
+
+// Score kernels are launched with programmatic stream serialization: their prologue (shared-memory fill, basis staging,
+// TMEM allocation) may run while the preceding kernel drains; each kernel waits for that kernel's completion
+// (griddepcontrol.wait) before it touches the activation.  DCTP_PDL=0 turns it off.
+template <typename... Params, typename... Args>
+cudaError_t launch_pdl(void (*kern)(Params...), int grid, int block, size_t smem, cudaStream_t stream, const Args&... args) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(static_cast<unsigned>(grid));
+    cfg.blockDim = dim3(static_cast<unsigned>(block));
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = g.pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kern, args...);
+}
+
+struct SiteDesc { const float* first; int B; int c_count; double* accum; };     // one dense activation: B * c_count maps back to back
 
 // fills seg (tile ranges, per-site sizes); returns the launch's tile count
 int fill_segments(ScoreSegments& seg, const SiteDesc* sites, int n, int NN, int maps_per_tile) {
@@ -419,19 +422,21 @@ int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* 
         a.trace = trace_buf;
     }
     const int variant = stack_variant(KP, v4 ? 4 : 2, a.Np / 8);
-    // per-map energies, coefficients and the cycle trace live in the debug instantiation (cfg 6) only
-    const int cfg = (a.energy_out || a.dump || tracing) ? 6 : g.stack_cfg ? g.stack_cfg : 7;
-    CUDA_TRY(launch_score_tma(stack_kernel_fn(cfg, variant), grid, stack_threads(cfg), smem, stream, maps, a));
-    note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP, basis.vec, cfg);
+    // per-map energies, coefficients and the cycle trace live in the debug instantiation (cfg6) only
+    const bool debug = a.energy_out || a.dump || tracing;
+    CUDA_TRY(launch_pdl(stack_kernel_fn(debug, variant), grid, 32 * stack_warps(debug ? STACK_NCONV_DEBUG : STACK_NCONV), smem, stream,
+                        maps, a));
+    note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP, basis.vec,
+                debug ? 6 : 7);
     if (tracing) {
         long long h[64];
         CUDA_TRY(cudaMemcpy(h, trace_buf, sizeof h, cudaMemcpyDeviceToHost));
         const double nt = h[14] > 0 ? double(h[14]) : 1.0;
-        fprintf(stderr, "[dctp trace] stack N=%d cfg %d, CTA 0, %lld tiles, cycles per tile | producer: wait slot %.0f | converter: wait Bx free %.0f, "
+        fprintf(stderr, "[dctp trace] stack N=%d, CTA 0, %lld tiles, cycles per tile | producer: wait slot %.0f | converter: wait Bx free %.0f, "
                         "wait TMA %.0f, convert %.0f, fence+arrive %.0f | issuer 1: wait Bx %.0f, wait D1 free %.0f, issue %.0f | issuer 2: wait A2 %.0f, "
                         "wait D2 free %.0f, issue %.0f | epi1 (first group, per tile of the CTA): wait D1 %.0f, wait A2 free %.0f, work %.0f | "
                         "epi2: wait D2 %.0f, TMEM loads %.0f, sums+shuffles %.0f, atomics %.0f\n",
-                N, cfg, h[14], h[0] / nt, h[16] / nt, h[17] / nt, h[18] / nt, h[19] / nt, h[8] / nt, h[9] / nt, h[10] / nt, h[40] / nt,
+                N, h[14], h[0] / nt, h[16] / nt, h[17] / nt, h[18] / nt, h[19] / nt, h[8] / nt, h[9] / nt, h[10] / nt, h[40] / nt,
                 h[41] / nt, h[42] / nt, h[24] / nt, h[25] / nt, h[26] / nt, h[32] / nt, h[34] / nt, h[35] / nt, h[33] / nt);
         fprintf(stderr, "[dctp trace] CTA 0, ns since kernel entry: TMEM + barriers ready %lld, bases staged and dependency wait over %lld, tile loop %lld\n", h[52], h[53], h[51]);
         fprintf(stderr, "[dctp trace] tile loop of CTA 0: %lld SM cycles in %lld ns = %.0f MHz, %.0f cycles per tile\n", h[50], h[51],
@@ -460,10 +465,8 @@ int get_kron_basis(int N, KronBasis& out) {
                     std::memcpy(&lo[off], &ll, 2);
                 }
     KronBasis b;
-    CUDA_TRY(cudaMalloc(&b.hi, hi.size()));
-    CUDA_TRY(cudaMalloc(&b.lo, lo.size()));
-    CUDA_TRY(cudaMemcpy(b.hi, hi.data(), hi.size(), cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.lo, lo.data(), lo.size(), cudaMemcpyHostToDevice));
+    int rc;
+    if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
     g.kron[N] = b;
     out = b;
     return DCTP_OK;
@@ -497,25 +500,17 @@ int launch_kron(const SiteDesc* sites, int n, int N, float* energy_out, float* c
     a.num_tiles = fill_segments(a.seg, sites, n, NN, a.tile_maps);
     ScoreTensorMaps maps;
     for (int i = 0; i < n; ++i) {
-        if (even) {
-            std::memset(&maps.m[i], 0, sizeof(CUtensorMap));
-            cuuint64_t gdim[2] = {static_cast<cuuint64_t>(NN), static_cast<cuuint64_t>(a.seg.n_maps[i])};
-            cuuint64_t gstr[1] = {static_cast<cuuint64_t>(NN) * 4};
-            cuuint32_t box[2] = {static_cast<cuuint32_t>(a.row_floats), static_cast<cuuint32_t>(a.tile_maps)}, estr[2] = {1, 1};
-            const CUresult r = reinterpret_cast<EncodeTiledFn>(g.encode_tiled)(
-                &maps.m[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(sites[i].first), gdim, gstr, box, estr,
-                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) return fail(DCTP_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for %d maps of side %d", (int)r, a.seg.n_maps[i], N);
-        } else if ((rc = encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.box_rows))) {
-            return rc;
-        }
+        // even sides: one map per row of the box, padded to row_floats; odd sides: the flat stream
+        rc = even ? encode_2d(maps.m[i], sites[i].first, NN, a.seg.n_maps[i], 4ll * NN, a.row_floats, a.tile_maps, CU_TENSOR_MAP_L2_PROMOTION_L2_128B)
+                  : encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.box_rows);
+        if (rc) return rc;
     }
     for (int i = n; i < SCORE_MAX_SEG; ++i) maps.m[i] = maps.m[0];
     const int grid = g.sm_count < a.num_tiles ? g.sm_count : a.num_tiles;
     const size_t smem = KronSmem::TOTAL;
 #define KRON_LAUNCH(K2V)                                                                                                         \
-    CUDA_TRY(even ? launch_score_tma(score_kron_kernel<K2V, true>, grid, KRON_NT, smem, stream, maps, a)                        \
-                  : launch_score_tma(score_kron_kernel<K2V, false>, grid, KRON_NT, smem, stream, maps, a))
+    CUDA_TRY(even ? launch_pdl(score_kron_kernel<K2V, true>, grid, KRON_NT, smem, stream, maps, a)                              \
+                  : launch_pdl(score_kron_kernel<K2V, false>, grid, KRON_NT, smem, stream, maps, a))
     switch (K2) {
         case 16: KRON_LAUNCH(16); break;
         case 32: KRON_LAUNCH(32); break;
@@ -551,10 +546,8 @@ int get_large_basis(int N, LargeBasis& out) {
             const size_t at = (static_cast<size_t>(n >> 6) * b.NPR + k) * 64 + ((((n & 63) >> 3) ^ (k & 7)) << 3) + (n & 7);
             split_bf16(dct_coef(k, n, N), hi[at], lo[at]);
         }
-    CUDA_TRY(cudaMalloc(&b.hi, hi.size() * 2));
-    CUDA_TRY(cudaMalloc(&b.lo, lo.size() * 2));
-    CUDA_TRY(cudaMemcpy(b.hi, hi.data(), hi.size() * 2, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(b.lo, lo.data(), lo.size() * 2, cudaMemcpyHostToDevice));
+    int rc;
+    if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
     g.large[N] = b;
     out = b;
     return DCTP_OK;
@@ -567,45 +560,10 @@ int get_simt_basis(int N, SimtBasis& out) {
     for (int n = 0; n < N; ++n)
         for (int k = 0; k < N; ++k) t[(size_t)n * N + k] = static_cast<float>(dct_coef(k, n, N));
     SimtBasis b;
-    CUDA_TRY(cudaMalloc(&b.t, t.size() * 4));
-    CUDA_TRY(cudaMemcpy(b.t, t.data(), t.size() * 4, cudaMemcpyHostToDevice));
+    if (int rc = upload(t, b.t)) return rc;
     g.simt[N] = b;
     out = b;
     return DCTP_OK;
-}
-
-// Score kernels are launched with programmatic stream serialization: their prologue (shared-memory fill, basis staging,
-// TMEM allocation) may run while the preceding kernel drains; each kernel waits for that kernel's completion
-// (griddepcontrol.wait) before it touches the activation.  DCTP_PDL=0 turns it off.
-template <typename Args>
-cudaError_t launch_score(void (*kern)(const Args), int grid, int block, size_t smem, cudaStream_t stream, const Args& args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(static_cast<unsigned>(grid));
-    cfg.blockDim = dim3(static_cast<unsigned>(block));
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = g.pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, args);
-}
-
-template <typename Args>
-cudaError_t launch_score_tma(void (*kern)(const ScoreTensorMaps, const Args), int grid, int block, size_t smem, cudaStream_t stream,
-                             const ScoreTensorMaps& map, const Args& args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(static_cast<unsigned>(grid));
-    cfg.blockDim = dim3(static_cast<unsigned>(block));
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = g.pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kern, map, args);
 }
 
 // ------------------------------------------------------------------ init
@@ -640,10 +598,12 @@ int setup_umma_all(int (*regs)[2]) {
     int rc;
     if ((rc = setup_umma<KP, LOAD_DENSE1, false>(regs[LOAD_DENSE1][0]))) return rc;
     if ((rc = setup_umma<KP, LOAD_DENSE2, false>(regs[LOAD_DENSE2][0]))) return rc;
-    if ((rc = setup_umma<KP, LOAD_DENSE4, false>(regs[LOAD_DENSE4][0]))) return rc;
     if ((rc = setup_umma<KP, LOAD_DENSE1, true>(regs[LOAD_DENSE1][1]))) return rc;
     if ((rc = setup_umma<KP, LOAD_DENSE2, true>(regs[LOAD_DENSE2][1]))) return rc;
-    if ((rc = setup_umma<KP, LOAD_DENSE4, true>(regs[LOAD_DENSE4][1]))) return rc;
+    if constexpr (KP == 64) {                        // (KP = 128: see umma_dense_mode)
+        if ((rc = setup_umma<KP, LOAD_DENSE4, false>(regs[LOAD_DENSE4][0]))) return rc;
+        if ((rc = setup_umma<KP, LOAD_DENSE4, true>(regs[LOAD_DENSE4][1]))) return rc;
+    }
     if ((rc = setup_umma<KP, LOAD_GEN4, false>(regs[LOAD_GEN4][0]))) return rc;
     if ((rc = setup_umma<KP, LOAD_GEN2, false>(regs[LOAD_GEN2][0]))) return rc;
     return setup_umma<KP, LOAD_GEN1, false>(regs[LOAD_GEN1][0]);
@@ -673,17 +633,16 @@ int ensure_init() {
     {
         const void* fns[] = {reinterpret_cast<const void*>(score_t_kernel<64, 3, 1>), reinterpret_cast<const void*>(score_t_kernel<64, 3, 2>),
                              reinterpret_cast<const void*>(score_t_kernel<32, 6, 1>), reinterpret_cast<const void*>(score_t_kernel<32, 6, 2>),
-                             reinterpret_cast<const void*>(score_t_kernel<32, 6, 4>),
-                             reinterpret_cast<const void*>(score_t_kernel<64, 3, 1, 2>), reinterpret_cast<const void*>(score_t_kernel<64, 3, 2, 2>)};
+                             reinterpret_cast<const void*>(score_t_kernel<32, 6, 4>), reinterpret_cast<const void*>(score_t_kernel<64, 3, 1, 2>)};
         for (const void* fn : fns) {
             CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
             CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
         }
     }
     {
-        for (int cfg = 4; cfg < STACK_CFGS; ++cfg)
-            for (int v = 0; stack_cfg_valid(cfg) && v < STACK_VARIANTS; ++v) {
-                const void* fn = stack_kernel_ptr(cfg, v);
+        for (const bool debug : {false, true})
+            for (int v = 0; v < STACK_VARIANTS; ++v) {
+                const void* fn = reinterpret_cast<const void*>(stack_kernel_fn(debug, v));
                 CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(StackSmem::TOTAL)));
                 CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
             }
@@ -699,16 +658,7 @@ int ensure_init() {
         CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &g.encode_tiled, cudaEnableDefault, &qres));
         if (!g.encode_tiled) return fail(DCTP_E_CUDA, "the driver does not export cuTensorMapEncodeTiled");
     }
-    if (const char* e = std::getenv("DCTP_KRON")) g.kron_on = std::atoi(e) != 0;
-    if (const char* e = std::getenv("DCTP_STACK_CFG")) { g.stack_cfg = std::atoi(e); if (!stack_cfg_valid(g.stack_cfg)) g.stack_cfg = 0; }
-    if (const char* e = std::getenv("DCTP_STACK")) g.stack_on = std::atoi(e) != 0;
-    if (const char* e = std::getenv("DCTP_STACK_MIN_MB")) g.stack_min_bytes = static_cast<long long>(std::atoi(e)) << 20;
-    if (const char* e = std::getenv("DCTP_TP")) g.t_prod = std::atoi(e) != 0;
     if (const char* e = std::getenv("DCTP_PDL")) g.pdl = std::atoi(e) != 0;
-    if (const char* e = std::getenv("DCTP_LARGE_LO")) g.large_lo = std::atoi(e);
-    if (const char* e = std::getenv("DCTP_T_MIN_MB")) g.t_min_bytes = static_cast<long long>(std::atoi(e)) << 20;
-    if (const char* e = std::getenv("DCTP_T_SLOTS")) g.t_slots = std::atoi(e);
-    if (g.t_slots != 0) g.t_slots = 3;
     CUDA_TRY(cudaFuncSetAttribute(score_large_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LargeSmem::TOTAL));
     CUDA_TRY(cudaFuncSetAttribute(score_large_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LargeSmem::TOTAL));
     CUDA_TRY(cudaFuncSetAttribute(score_simt_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SIMT_SMALL_SMEM));
@@ -728,21 +678,19 @@ inline int pow2_floor(int v) {
 
 bool umma_shape_ok(int H, int W, long long stride_h) { return H == W && H >= 1 && H <= 128 && stride_h == W; }
 
-int pick_vec(const float* x, long long stride_b, long long stride_c, int c_begin, int N) {
+int pick_vec(const float* x, long long stride_b, long long stride_c, int N) {
     auto aligned = [&](int v) {
         return (N % v) == 0 && (reinterpret_cast<uintptr_t>(x) % (4 * v)) == 0 && (stride_b % v) == 0 && (stride_c % v) == 0;
     };
-    (void)c_begin;
     if (aligned(4)) return 4;
     if (aligned(2)) return 2;
     return 1;
 }
 
-// TMEM-operand kernel: dense tensors, N % 4 == 0, 16 <= N <= 64
-// large-map tensor-core kernel: dense square maps, 128 < N <= 320, N % 16 == 0
-// the tiled large-map kernel takes dense square maps of side 80..320 (multiples of 16); AUTO gives it everything above large_lo
+// the tiled large-map kernel takes square maps of side 80..320 (multiples of 16), and AUTO gives it all of them: measured against
+// the smem-operand kernel, [12,64,N,N]: 80 0.92 vs 0.67 TB/s (a tie in round 1, before the large kernel lost a fifth of its
+// instructions), 96 1.22 vs 0.73
 bool large_shape_supported(int H, int W, long long stride_h) { return H == W && H >= 80 && H <= 320 && (H % 16) == 0 && stride_h == W; }
-bool large_shape_ok(int H, int W, long long stride_h) { return large_shape_supported(H, W, stride_h) && H >= g.large_lo; }
 
 // up to LARGE_MAX_SEG dense activations of side N in ONE launch (energy_out / coeff_out: single-site launches only)
 int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, cudaStream_t stream) {
@@ -780,30 +728,13 @@ int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* 
     }
     // every activation as a 2-D tensor [n_maps * N rows, N floats]; a map slab is the box {64 floats, 128 rows}, out-of-range parts zero
     LargeTensorMap xmap;
-    std::memset(&xmap, 0, sizeof xmap);
-    for (int i = 0; i < n; ++i) {
-        cuuint64_t gdim[2] = {static_cast<cuuint64_t>(N), static_cast<cuuint64_t>(sites[i].B) * sites[i].c_count * N};
-        cuuint64_t gstr[1] = {static_cast<cuuint64_t>(N) * 4};
-        cuuint32_t box[2] = {64, 128}, estr[2] = {1, 1};
-        const CUresult r = reinterpret_cast<EncodeTiledFn>(g.encode_tiled)(
-            &xmap.m[i], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(sites[i].first), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(DCTP_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for site %d, side %d", (int)r, i, N);
-    }
+    for (int i = 0; i < n; ++i)
+        if ((rc = encode_2d(xmap.m[i], sites[i].first, N, static_cast<long long>(sites[i].B) * sites[i].c_count * N, 4ll * N, 64, 128,
+                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B)))
+            return rc;
     for (int i = n; i < LARGE_MAX_SEG; ++i) xmap.m[i] = xmap.m[0];
-    {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(static_cast<unsigned>(grid));
-        cfg.blockDim = dim3(LARGE_NT);
-        cfg.dynamicSmemBytes = LargeSmem::TOTAL;
-        cfg.stream = stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr;
-        cfg.numAttrs = g.pdl ? 1 : 0;
-        CUDA_TRY(cudaLaunchKernelEx(&cfg, (a.trace || a.dump) ? score_large_kernel<true> : score_large_kernel<false>, xmap, a));
-    }
+    CUDA_TRY(launch_pdl((a.trace || a.dump) ? score_large_kernel<true> : score_large_kernel<false>, grid, LARGE_NT, LargeSmem::TOTAL, stream,
+                        xmap, a));
     if (energy_out) {
         sum_parts_kernel<<<(a.n_maps + 255) / 256, 256, 0, stream>>>(a.energy_parts, a.NVC, energy_out, a.n_maps);
         CUDA_TRY(cudaFreeAsync(a.energy_parts, stream));
@@ -828,24 +759,24 @@ int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* 
 // which maps the TMEM-operand kernel takes at all (dense; side 5..64, odd sides up to 13 and only when the whole stream is a
 // multiple of four floats), and which ones AUTO gives it
 bool t_shape_supported(int N) { return N >= 5 && N <= 64 && ((N % 2) == 0 || N <= 13); }   // (odd sides: 8-byte scatter entries must fit in shared memory)
-bool t_shape_ok(int N) {
-    if (g.t_slots <= 0 || !t_shape_supported(N)) return false;
-    // measured A/B on one B200 (tools/prof_one.py, [256,C,N,N], TB/s, this kernel vs the smem-operand kernel):
-    // 56x56 3.16 vs 2.65, 64x64 3.43 vs 2.94 (3 slots); 28x28 3.28 vs 2.68, 32x32 2.93 vs 2.41 (6 slots, cp.async staging);
-    // 14x14 2.87 vs 2.18, 16x16 3.10 vs 2.58 (6 slots, two maps side by side per slot); 34..50 not better
-    return g.t_all || N >= g.t_auto_lo || N <= 32;
+// measured A/B on one B200 (tools/prof_one.py, [256,C,N,N], TB/s, this kernel vs the smem-operand kernel):
+// 56x56 3.16 vs 2.65, 64x64 3.43 vs 2.94 (3 slots); 28x28 3.28 vs 2.68, 32x32 2.93 vs 2.41 (6 slots, cp.async staging);
+// 14x14 2.87 vs 2.18, 16x16 3.10 vs 2.58 (6 slots, two maps side by side per slot); 34..50 not better
+constexpr int T_AUTO_LO = 52, T_AUTO_SMALL_HI = 32;
+bool t_shape_ok(int N) { return t_shape_supported(N) && (N >= T_AUTO_LO || N <= T_AUTO_SMALL_HI); }
+// ... and how much work a launch must carry before AUTO prefers it below T_AUTO_LO: the 6-slot variant's prologue (768 threads,
+// A' into TMEM, 96 KB of operand slots) costs a few microseconds more than the smem-operand kernel's, which decides launches of a
+// few MB (ResNet-56 [256,16,32,32] = 17 MB: 0.655 vs 0.754 ms per batch over its 55 hooks with / without this rule)
+// (sides <= 8, four maps side by side per slot, are supported but not routed: back to back on one shape this kernel shows
+//  [256,2048,7,7] at 2.09 vs 1.48 TB/s because its longer prologue hides behind the previous launch, but inside ResNet-50's
+//  step the launch takes 69 us with either kernel and the step is not faster)
+constexpr int T_AUTO_SMALL_LO = 10;
+constexpr long long T_AUTO_MIN_BYTES = 32ll << 20;
+bool t_launch_ok(int N, long long bytes) {
+    return t_shape_ok(N) && (N >= T_AUTO_LO || (N >= T_AUTO_SMALL_LO && bytes >= T_AUTO_MIN_BYTES));
 }
-// ... and how much work a launch must carry before AUTO prefers it: the 6-slot variant's prologue (768 threads, A' into
-// TMEM, 96 KB of operand slots) costs a few microseconds more than the smem-operand kernel's, which decides launches of a few MB
-// (ResNet-56 [256,16,32,32] = 17 MB: 0.655 vs 0.754 ms per batch over its 55 hooks with / without this rule)
 // odd sides: a float4 of the stream may straddle maps, the stream itself must not end inside one
 bool t_stream_ok(int N, long long n_maps) { return (N % 2) == 0 || (n_maps * N * N) % 4 == 0; }
-bool t_launch_ok(int N, long long bytes) {
-    // (sides <= 8, four maps side by side per slot, are supported but not routed: back to back on one shape this kernel shows
-    //  [256,2048,7,7] at 2.09 vs 1.48 TB/s because its longer prologue hides behind the previous launch, but inside ResNet-50's
-    //  step the launch takes 69 us with either kernel and the step is not faster)
-    return t_shape_ok(N) && (g.t_all || N >= g.t_auto_lo || (N >= 10 && bytes >= g.t_min_bytes));
-}
 
 int launch_t(const float* first, int B, int N, int c_count, double* accum, float* energy_out, float* coeff_out, cudaStream_t stream) {
     TBasis basis;
@@ -886,21 +817,21 @@ int launch_t(const float* first, int B, int N, int c_count, double* accum, float
     if (grid > need) grid = need;
     a.chan_step = static_cast<int>((static_cast<long long>(grid) * ns * a.MT) % c_count);
     const bool v2 = basis.vpe == 2;
-    if (n1max == 64 && g.t_prod && basis.tile_vec <= 13 * 128 && !v2) {   // producer warpgroups: tiles of at most 13 float4 per thread
-                                                                          // (and the 2-byte scatter table: 52x52, 56x56 fit in shared memory)
-        const size_t smem_p = TScoreSmem<64, 2>::total(ns, a.scatter_bytes);
-        if (v2) CUDA_TRY(launch_score(score_t_kernel<64, 3, 2, 2>, grid, 640, smem_p, stream, a));
-        else CUDA_TRY(launch_score(score_t_kernel<64, 3, 1, 2>, grid, 640, smem_p, stream, a));
+    // two producer warpgroups (ResNet-50 step 3.30 -> 3.15 ms) where a tile is at most 13 float4 per thread and the scatter table
+    // has one entry per float4 (52x52, 56x56: it fits in shared memory)
+    const bool producers = n1max == 64 && basis.tile_vec <= 13 * 128 && basis.vpe == 1;
+    if (producers) {
+        CUDA_TRY(launch_pdl(score_t_kernel<64, 3, 1, 2>, grid, 640, TScoreSmem<64, 2>::total(ns, a.scatter_bytes), stream, a));
     } else if (n1max == 64) {
-        if (v2) CUDA_TRY(launch_score(score_t_kernel<64, 3, 2>, grid, 384, smem, stream, a));
-        else CUDA_TRY(launch_score(score_t_kernel<64, 3, 1>, grid, 384, smem, stream, a));
+        if (v2) CUDA_TRY(launch_pdl(score_t_kernel<64, 3, 2>, grid, 384, smem, stream, a));
+        else CUDA_TRY(launch_pdl(score_t_kernel<64, 3, 1>, grid, 384, smem, stream, a));
     } else {
-        if (basis.vpe == 4) CUDA_TRY(launch_score(score_t_kernel<32, 6, 4>, grid, 768, smem, stream, a));
-        else if (v2) CUDA_TRY(launch_score(score_t_kernel<32, 6, 2>, grid, 768, smem, stream, a));
-        else CUDA_TRY(launch_score(score_t_kernel<32, 6, 1>, grid, 768, smem, stream, a));
+        if (basis.vpe == 4) CUDA_TRY(launch_pdl(score_t_kernel<32, 6, 4>, grid, 768, smem, stream, a));
+        else if (v2) CUDA_TRY(launch_pdl(score_t_kernel<32, 6, 2>, grid, 768, smem, stream, a));
+        else CUDA_TRY(launch_pdl(score_t_kernel<32, 6, 1>, grid, 768, smem, stream, a));
     }
     note_kernel("score_t_kernel<%d,%d,VPE=%d%s> (tcgen05, block-diagonal basis in TMEM)", n1max, ns, basis.vpe,
-                (n1max == 64 && g.t_prod && basis.tile_vec <= 13 * 128 && !v2) ? ",2 producer warpgroups" : "");
+                producers ? ",2 producer warpgroups" : "");
     if (tracing) {
         long long h[256];
         CUDA_TRY(cudaMemcpy(h, trace_buf, sizeof h, cudaMemcpyDeviceToHost));
@@ -922,16 +853,37 @@ int launch_t(const float* first, int B, int N, int c_count, double* accum, float
     return DCTP_OK;
 }
 
+struct Call {                                            // the arguments of one dctp_score_accum call
+    const float* x;
+    int B, H, W;
+    long long stride_b, stride_c, stride_h;
+    int c_begin, c_count;
+    double* accum;
+    float *energy_out, *coeff_out;
+    const float* first;                                  // dense_first()
+    long long maps() const { return static_cast<long long>(B) * c_count; }
+};
+
+// The first scored map when the call's maps are one contiguous, 16-byte-aligned fp32 stream (packed rows and channels, and
+// images back to back unless there is one), null otherwise.  The TMA-fed kernels read only such streams.
+const float* dense_first(const Call& c) {
+    const long long hw = static_cast<long long>(c.H) * c.W;
+    const float* first = c.x + static_cast<long long>(c.c_begin) * c.stride_c;
+    const bool dense = c.stride_h == c.W && c.stride_c == hw && (c.B == 1 || c.stride_b == c.c_count * hw) &&
+                       (reinterpret_cast<uintptr_t>(first) % 16) == 0;
+    return dense ? first : nullptr;
+}
+
 template <int KP>
-int launch_umma(const float* x, int B, int N, long long stride_b, long long stride_c, int c_begin, int c_count,
-                double* accum, float* energy_out, float* coeff_out, cudaStream_t stream, bool allow_t) {
+int launch_umma(const Call& c, cudaStream_t stream) {
+    const int N = c.H;
     UmmaBasis basis;
     int rc = get_umma_basis(N, KP, basis);
     if (rc) return rc;
     UmmaScoreArgs a;
     std::memset(&a, 0, sizeof a);
-    a.x = x; a.stride_b = stride_b; a.stride_c = stride_c; a.c_begin = c_begin; a.c_count = c_count;
-    a.n_maps = B * c_count;
+    a.x = c.x; a.stride_b = c.stride_b; a.stride_c = c.stride_c; a.c_begin = c.c_begin; a.c_count = c.c_count;
+    a.n_maps = c.B * c.c_count;
     a.N = N; a.NN = N * N;
     a.Ms = (N + 7) / 8 * 8; a.G = 128 / a.Ms; a.J = KP / a.Ms; a.MT = a.G * a.J;
     a.num_tiles = (a.n_maps + a.MT - 1) / a.MT;
@@ -945,33 +897,21 @@ int launch_umma(const float* x, int B, int N, long long stride_b, long long stri
     a.idesc1 = umma::make_idesc_bf16(128, a.N1, false, false);
     a.idesc2 = umma::make_idesc_bf16(128, a.N2, true, false);
     a.basis_hi = basis.hi; a.basis_lo = basis.lo;
-    a.accum = accum; a.energy_out = energy_out; a.dump = coeff_out; a.status = g.status;
+    a.accum = c.accum; a.energy_out = c.energy_out; a.dump = c.coeff_out; a.status = g.status;
     a.div_n.set(N); a.div_ms.set(a.Ms); a.div_j.set(a.J);
-    // dense: every scored map back to back in memory (full channel range, packed strides), 16-B aligned
-    const float* first = x + static_cast<long long>(c_begin) * stride_c;
-    const bool dense = basis.scatter != nullptr && stride_c == a.NN && (B == 1 || stride_b == static_cast<long long>(c_count) * a.NN) &&
-                       (reinterpret_cast<uintptr_t>(first) % 16) == 0;
-    if (KP == 64 && allow_t && dense && g.kron_on && N <= 8) {
-        const SiteDesc one = {first, B, c_count, accum};
-        return launch_kron(&one, 1, N, energy_out, coeff_out, stream);
-    }
-    if (KP == 64 && allow_t && dense && g.stack_on && stack_shape_supported(N) &&
-        static_cast<long long>(a.n_maps) * a.NN * 4 >= g.stack_min_bytes)
-    {
-        const SiteDesc one = {first, B, c_count, accum};
-        return launch_stack(&one, 1, N, energy_out, coeff_out, stream);
-    }
-    if (KP == 64 && allow_t && dense && t_stream_ok(N, a.n_maps) && t_launch_ok(N, static_cast<long long>(a.n_maps) * a.NN * 4))
-        return launch_t(first, B, N, c_count, accum, energy_out, coeff_out, stream);
+    // the dense load modes read the stream through a table of where each float4 of a full tile lands, which exists when a tile is a
+    // whole number of float4.  (KP = 128 serves sides 65..128, one map per tile: only even sides have a table, and its entries are
+    // never 2-byte (LOAD_DENSE4), so that instantiation is not compiled.)
+    const bool dense = c.first && basis.scatter;
     int mode;
     if (dense) {
         mode = basis.vpe == 1 ? LOAD_DENSE1 : basis.vpe == 2 ? LOAD_DENSE2 : LOAD_DENSE4;
-        a.x_dense = first; a.total_elems = static_cast<long long>(a.n_maps) * a.NN;
+        a.x_dense = c.first; a.total_elems = static_cast<long long>(a.n_maps) * a.NN;
         a.tile_vec = basis.tile_vec; a.scatter = basis.scatter;
         a.var_bytes = static_cast<uint32_t>(basis.tile_vec) * basis.vpe * 2u;
         a.div_vpm.set(1);
     } else {
-        const int vec = pick_vec(x, stride_b, stride_c, c_begin, N);
+        const int vec = pick_vec(c.x, c.stride_b, c.stride_c, N);
         mode = vec == 4 ? LOAD_GEN4 : vec == 2 ? LOAD_GEN2 : LOAD_GEN1;
         a.var_bytes = 128 * sizeof(void*);
         a.div_vpm.set(a.NN / vec);
@@ -981,23 +921,24 @@ int launch_umma(const float* x, int B, int N, long long stride_b, long long stri
     const size_t smem = UmmaScoreSmem<KP>::total(a.red_bytes, a.var_bytes);
     int grid = g.sm_count * umma_occupancy(KP, mode, pf, smem);
     if (grid > a.num_tiles) grid = a.num_tiles;
-    a.chan_step = static_cast<int>((static_cast<long long>(grid) * a.MT) % c_count);
+    a.chan_step = static_cast<int>((static_cast<long long>(grid) * a.MT) % c.c_count);
     switch (mode) {
         case LOAD_DENSE1:
-            if (pf) CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_DENSE1, true>, grid, 128, smem, stream, a));
-            else CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_DENSE1, false>, grid, 128, smem, stream, a));
+            if (pf) CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_DENSE1, true>, grid, 128, smem, stream, a));
+            else CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_DENSE1, false>, grid, 128, smem, stream, a));
             break;
         case LOAD_DENSE2:
-            if (pf) CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_DENSE2, true>, grid, 128, smem, stream, a));
-            else CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_DENSE2, false>, grid, 128, smem, stream, a));
+            if (pf) CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_DENSE2, true>, grid, 128, smem, stream, a));
+            else CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_DENSE2, false>, grid, 128, smem, stream, a));
             break;
         case LOAD_DENSE4:
-            if (pf) CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_DENSE4, true>, grid, 128, smem, stream, a));
-            else CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_DENSE4, false>, grid, 128, smem, stream, a));
+            if constexpr (KP != 64) return fail(DCTP_E_UNSUPPORTED, "no <%d, LOAD_DENSE4> instantiation (side %d)", KP, N);
+            else if (pf) CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_DENSE4, true>, grid, 128, smem, stream, a));
+            else CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_DENSE4, false>, grid, 128, smem, stream, a));
             break;
-        case LOAD_GEN4: CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_GEN4, false>, grid, 128, smem, stream, a)); break;
-        case LOAD_GEN2: CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_GEN2, false>, grid, 128, smem, stream, a)); break;
-        default: CUDA_TRY(launch_score(score_umma_kernel<KP, LOAD_GEN1, false>, grid, 128, smem, stream, a)); break;
+        case LOAD_GEN4: CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_GEN4, false>, grid, 128, smem, stream, a)); break;
+        case LOAD_GEN2: CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_GEN2, false>, grid, 128, smem, stream, a)); break;
+        default: CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_GEN1, false>, grid, 128, smem, stream, a)); break;
     }
     note_kernel("score_umma_kernel<%d,%d,%d> (tcgen05 bf16x3, operands in shared memory)", KP, mode, pf ? 1 : 0);
     ++g.launches;
@@ -1005,17 +946,17 @@ int launch_umma(const float* x, int B, int N, long long stride_b, long long stri
     return DCTP_OK;
 }
 
-int launch_simt(const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
-                int c_begin, int c_count, double* accum, float* energy_out, float* coeff_out, cudaStream_t stream) {
+int launch_simt(const Call& c, cudaStream_t stream) {
+    const int H = c.H, W = c.W;
     SimtBasis bh, bw;
     int rc = get_simt_basis(H, bh);
     if (rc) return rc;
     if ((rc = get_simt_basis(W, bw))) return rc;
     SimtScoreArgs a;
     std::memset(&a, 0, sizeof a);
-    a.x = x; a.stride_b = stride_b; a.stride_c = stride_c; a.stride_h = stride_h;
-    a.c_begin = c_begin; a.c_count = c_count; a.n_maps = B * c_count; a.H = H; a.W = W;
-    a.basis_h_t = bh.t; a.basis_w_t = bw.t; a.accum = accum; a.energy_out = energy_out; a.dump = coeff_out;
+    a.x = c.x; a.stride_b = c.stride_b; a.stride_c = c.stride_c; a.stride_h = c.stride_h;
+    a.c_begin = c.c_begin; a.c_count = c.c_count; a.n_maps = c.B * c.c_count; a.H = H; a.W = W;
+    a.basis_h_t = bh.t; a.basis_w_t = bw.t; a.accum = c.accum; a.energy_out = c.energy_out; a.dump = c.coeff_out;
     if (H <= SIMT_T && W <= SIMT_T) {
         const int G = SIMT_T / H, tiles = (a.n_maps + G - 1) / G;
         int grid = g.sm_count * 2;
@@ -1026,7 +967,7 @@ int launch_simt(const float* x, int B, int H, int W, long long stride_b, long lo
         const int Hpad = (H + SIMT_T - 1) / SIMT_T * SIMT_T;
         const size_t smem = static_cast<size_t>(Hpad + 2 * SIMT_T) * SIMT_LD * sizeof(float);
         if (smem > 200 * 1024) return fail(DCTP_E_UNSUPPORTED, "map height %d needs %zu B of shared memory", H, smem);
-        if (energy_out) CUDA_TRY(cudaMemsetAsync(energy_out, 0, sizeof(float) * a.n_maps, stream));
+        if (c.energy_out) CUDA_TRY(cudaMemsetAsync(c.energy_out, 0, sizeof(float) * a.n_maps, stream));
         const unsigned grid = static_cast<unsigned>((W + SIMT_T - 1) / SIMT_T) * static_cast<unsigned>(a.n_maps);
         score_simt_large_kernel<<<grid, 256, smem, stream>>>(a);
         note_kernel("score_simt_large_kernel (fp32 CUDA cores)");
@@ -1036,13 +977,62 @@ int launch_simt(const float* x, int B, int H, int W, long long stride_b, long lo
     return DCTP_OK;
 }
 
-int resolve_path(int path, int H, int W, long long stride_h) {
-    if (path == DCTP_PATH_AUTO) {
-        if (large_shape_ok(H, W, stride_h)) return DCTP_PATH_LARGE;
-        if (umma_shape_ok(H, W, stride_h)) return DCTP_PATH_UMMA;
-        return DCTP_PATH_SIMT;
+// ------------------------------------------------------------------ routing
+// The kernels a score call can run on.  takes() says whether a kernel takes a call; AUTO's choice and every forced
+// DCTP_PATH_* value go through it.
+enum Route { R_KRON, R_STACK, R_TMEM, R_UMMA64, R_UMMA128, R_LARGE, R_SIMT };
+
+bool takes(Route r, const Call& c) {
+    const bool square = c.H == c.W, dense = c.first != nullptr;
+    switch (r) {
+        case R_KRON: return square && c.H <= 8 && dense;
+        case R_STACK: return square && stack_shape_supported(c.H) && dense;
+        case R_TMEM: return square && t_shape_supported(c.H) && dense && t_stream_ok(c.H, c.maps());
+        case R_UMMA64: return umma_shape_ok(c.H, c.W, c.stride_h) && c.H <= 64;
+        case R_UMMA128: return umma_shape_ok(c.H, c.W, c.stride_h) && c.H > 64;
+        case R_LARGE: return large_shape_supported(c.H, c.W, c.stride_h) && dense;
+        default: return true;
     }
-    return path;
+}
+
+Route auto_route(const Call& c) {
+    if (takes(R_LARGE, c)) return R_LARGE;
+    if (takes(R_UMMA128, c)) return R_UMMA128;                  // (windows and strided batches of large maps too)
+    if (!takes(R_UMMA64, c)) return R_SIMT;
+    if (takes(R_KRON, c)) return R_KRON;
+    if (takes(R_STACK, c)) return R_STACK;
+    if (takes(R_TMEM, c) && t_launch_ok(c.H, 4 * c.maps() * c.H * c.W)) return R_TMEM;
+    return R_UMMA64;
+}
+
+// a call on one map at a 16-byte-aligned address: what AUTO and the forced paths do with dense maps of this shape
+Call dense_call(int H, int W, long long stride_h) {
+    alignas(16) static const float base[4] = {};
+    Call c = {base, 1, H, W, 0, static_cast<long long>(H) * W, stride_h, 0, 1, nullptr, nullptr, nullptr, nullptr};
+    c.first = dense_first(c);
+    return c;
+}
+
+// the kernels that score up to SCORE_MAX_SEG activations in one launch
+static_assert(SCORE_MAX_SEG == LARGE_MAX_SEG, "one multi-site batch size");
+bool multi_site(Route r) { return r == R_KRON || r == R_STACK || r == R_LARGE; }
+int launch_sites(Route r, const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, cudaStream_t s) {
+    if (r == R_KRON) return launch_kron(sites, n, N, energy_out, coeff_out, s);
+    if (r == R_STACK) return launch_stack(sites, n, N, energy_out, coeff_out, s);
+    return launch_large(sites, n, N, energy_out, coeff_out, s);
+}
+
+int launch(Route r, const Call& c, cudaStream_t s) {
+    switch (r) {
+        case R_TMEM: return launch_t(c.first, c.B, c.H, c.c_count, c.accum, c.energy_out, c.coeff_out, s);
+        case R_UMMA64: return launch_umma<64>(c, s);
+        case R_UMMA128: return launch_umma<128>(c, s);
+        case R_SIMT: return launch_simt(c, s);
+        default: {
+            const SiteDesc one = {c.first, c.B, c.c_count, c.accum};
+            return launch_sites(r, &one, 1, c.H, c.energy_out, c.coeff_out, s);
+        }
+    }
 }
 
 }  // namespace
@@ -1061,15 +1051,7 @@ int dctp_init(void) {
 int dctp_shutdown(void) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (!g.ready) return DCTP_OK;
-    for (auto& kv : g.umma) { cudaFree(kv.second.hi); cudaFree(kv.second.lo); cudaFree(kv.second.scatter); }
-    for (auto& kv : g.simt) cudaFree(kv.second.t);
-    for (auto& kv : g.large) { cudaFree(kv.second.hi); cudaFree(kv.second.lo); }
-    for (auto& kv : g.tmem) {
-        cudaFree(kv.second.a_hi); cudaFree(kv.second.a_lo); cudaFree(kv.second.c_hi); cudaFree(kv.second.c_lo); cudaFree(kv.second.scatter);
-    }
-    for (auto& kv : g.stack) { cudaFree(kv.second.a_img); cudaFree(kv.second.c2_hi); cudaFree(kv.second.c2_lo); cudaFree(kv.second.table); }
-    for (auto& kv : g.kron) { cudaFree(kv.second.hi); cudaFree(kv.second.lo); }
-    g.umma.clear(); g.simt.clear(); g.tmem.clear(); g.large.clear(); g.stack.clear(); g.kron.clear();
+    for (void* p : g.bases) cudaFree(p);
     cudaFree(g.status); cudaFree(g.hx); cudaFree(g.hacc); cudaFree(g.hout); cudaFree(g.d3_part); cudaFree(g.d3_energy);
     g = State();
     return DCTP_OK;
@@ -1083,13 +1065,17 @@ int dctp_sm_count(void) {
 long long dctp_launch_count(void) { return g.launches; }
 const char* dctp_last_kernel(void) { return g.last_kernel; }
 
-int dctp_path_for(int H, int W, long long stride_h) { return resolve_path(DCTP_PATH_AUTO, H, W, stride_h); }
+int dctp_path_for(int H, int W, long long stride_h) {
+    const Route r = auto_route(dense_call(H, W, stride_h));
+    return r == R_LARGE ? DCTP_PATH_LARGE : r == R_SIMT ? DCTP_PATH_SIMT : DCTP_PATH_UMMA;
+}
 
 int dctp_occupancy(int kp, int mode) {
     std::lock_guard<std::mutex> lk(g_mu);
     int rc = ensure_init();
     if (rc) return rc;
     if ((kp != 64 && kp != 128) || mode < 0 || mode > 5) return fail(DCTP_E_INVALID, "dctp_occupancy(%d, %d)", kp, mode);
+    if (kp == 128 && mode == LOAD_DENSE4) return fail(DCTP_E_UNSUPPORTED, "dctp_occupancy: no <128, LOAD_DENSE4> instantiation");
     const size_t smem = kp == 64 ? UmmaScoreSmem<64>::total(2048, 3136) : UmmaScoreSmem<128>::total(2560, 3200);
     return umma_occupancy(kp, mode, mode <= LOAD_DENSE4, smem);
 }
@@ -1099,36 +1085,23 @@ int dctp_prepare(int H, int W) {
     int rc = ensure_init();
     if (rc) return rc;
     if (H < 1 || W < 1) return fail(DCTP_E_INVALID, "dctp_prepare: H=%d W=%d", H, W);
-    if (umma_shape_ok(H, W, W)) {
-        if (H <= 8) {
-            KronBasis kb;
-            int rc2 = get_kron_basis(H, kb);
-            if (rc2) return rc2;
-        }
-        if (stack_shape_supported(H)) {
-            StackBasis sb;
-            int rc2 = get_stack_basis(H, sb);
-            if (rc2) return rc2;
-        }
-        if (t_shape_ok(H)) {
-            TBasis tb;
-            int rc2 = get_t_basis(H, tb);
-            if (rc2) return rc2;
-        }
-        if (large_shape_ok(H, W, W)) {
-            LargeBasis lb;
-            if ((rc = get_large_basis(H, lb))) return rc;
-        }
-        UmmaBasis b;
-        return get_umma_basis(H, H <= 64 ? 64 : 128, b);
+    // the bases of the kernels dense maps of this shape can run on (the TMEM-operand kernel: the sides AUTO may give it)
+    const Call c = dense_call(H, W, W);
+    LargeBasis lb;
+    if (takes(R_LARGE, c) && (rc = get_large_basis(H, lb))) return rc;
+    if (!takes(R_UMMA64, c) && !takes(R_UMMA128, c)) {
+        SimtBasis b;
+        if ((rc = get_simt_basis(H, b))) return rc;
+        return get_simt_basis(W, b);
     }
-    if (large_shape_ok(H, W, W)) {
-        LargeBasis lb;
-        if ((rc = get_large_basis(H, lb))) return rc;
-    }
-    SimtBasis b;
-    if ((rc = get_simt_basis(H, b))) return rc;
-    return get_simt_basis(W, b);
+    KronBasis kb;
+    StackBasis sb;
+    TBasis tb;
+    UmmaBasis ub;
+    if (takes(R_KRON, c) && (rc = get_kron_basis(H, kb))) return rc;
+    if (takes(R_STACK, c) && (rc = get_stack_basis(H, sb))) return rc;
+    if (t_shape_ok(H) && (rc = get_t_basis(H, tb))) return rc;
+    return get_umma_basis(H, H <= 64 ? 64 : 128, ub);
 }
 
 int dctp_score_accum(const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
@@ -1144,61 +1117,26 @@ int dctp_score_accum(const float* x, int B, int H, int W, long long stride_b, lo
     if (B == 0 || c_count == 0) return DCTP_OK;                     // empty batch / empty window: nothing to add
     if (!x || !accum) return fail(DCTP_E_INVALID, "dctp_score_accum: null pointer");
     if (static_cast<long long>(B) * c_count > (1ll << 30)) return fail(DCTP_E_INVALID, "too many maps in one call");
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    const int p = resolve_path(path, H, W, stride_h);
-    switch (p) {
-        case DCTP_PATH_UMMA:
-            if (!umma_shape_ok(H, W, stride_h))
-                return fail(DCTP_E_UNSUPPORTED, "UMMA path takes contiguous square maps of side <= 128 (got %dx%d, stride_h %lld)", H, W,
-                            stride_h);
-            return H <= 64 ? launch_umma<64>(x, B, H, stride_b, stride_c, c_begin, c_count, accum, energy_out, coeff_out, s, path == DCTP_PATH_AUTO)
-                           : launch_umma<128>(x, B, H, stride_b, stride_c, c_begin, c_count, accum, energy_out, coeff_out, s, false);
-        case DCTP_PATH_TMEM: {
-            const float* first = x + static_cast<long long>(c_begin) * stride_c;
-            const bool dense = stride_h == W && stride_c == static_cast<long long>(H) * W &&
-                               (B == 1 || stride_b == static_cast<long long>(c_count) * H * W) && (reinterpret_cast<uintptr_t>(first) % 16) == 0;
-            if (H != W || !t_shape_supported(H) || !dense || !t_stream_ok(H, static_cast<long long>(B) * c_count))
-                return fail(DCTP_E_UNSUPPORTED, "TMEM-operand path takes dense 16-B aligned square maps of side 5..64 (odd sides: up to 13, and a whole "
-                                                "number of float4 in the call) (got %dx%d)", H, W);
-            return launch_t(first, B, H, c_count, accum, energy_out, coeff_out, s);
-        }
-        case DCTP_PATH_KRON: {
-            const float* first = x + static_cast<long long>(c_begin) * stride_c;
-            const bool dense = stride_h == W && stride_c == static_cast<long long>(H) * W &&
-                               (B == 1 || stride_b == static_cast<long long>(c_count) * H * W) && (reinterpret_cast<uintptr_t>(first) % 16) == 0;
-            if (H != W || H > 8 || !dense)
-                return fail(DCTP_E_UNSUPPORTED, "Kronecker path takes dense 16-B aligned square maps of side <= 8 (got %dx%d)", H, W);
-            const SiteDesc one = {first, B, c_count, accum};
-            return launch_kron(&one, 1, H, energy_out, coeff_out, s);
-        }
-        case DCTP_PATH_STACK: {
-            const float* first = x + static_cast<long long>(c_begin) * stride_c;
-            const bool dense = stride_h == W && stride_c == static_cast<long long>(H) * W &&
-                               (B == 1 || stride_b == static_cast<long long>(c_count) * H * W) && (reinterpret_cast<uintptr_t>(first) % 16) == 0;
-            if (H != W || !stack_shape_supported(H) || !dense)
-                return fail(DCTP_E_UNSUPPORTED, "stacked-basis path takes dense 16-B aligned square maps of even side 10..64 (above 32: multiples of 4) (got %dx%d)", H, W);
-            const SiteDesc one = {first, B, c_count, accum};
-            return launch_stack(&one, 1, H, energy_out, coeff_out, s);
-        }
-        case DCTP_PATH_LARGE: {
-            const float* first = x + static_cast<long long>(c_begin) * stride_c;
-            const bool dense = stride_c == static_cast<long long>(H) * W && (B == 1 || stride_b == static_cast<long long>(c_count) * H * W) &&
-                               (reinterpret_cast<uintptr_t>(first) % 16) == 0;
-            if (!(path == DCTP_PATH_AUTO ? large_shape_ok(H, W, stride_h) : large_shape_supported(H, W, stride_h)) || !dense) {
-                if (path == DCTP_PATH_AUTO && umma_shape_ok(H, W, stride_h))   // windows / strided batches: the smem-operand kernel ...
-                    return launch_umma<128>(x, B, H, stride_b, stride_c, c_begin, c_count, accum, energy_out, coeff_out, s, false);
-                if (path == DCTP_PATH_AUTO)              // ... or, above its range, CUDA cores
-                    return launch_simt(x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, s);
-                return fail(DCTP_E_UNSUPPORTED, "large-map path takes dense 16-B aligned square maps, side 80..320 multiple of 16 (got %dx%d)", H, W);
-            }
-            const SiteDesc one = {first, B, c_count, accum};
-            return launch_large(&one, 1, H, energy_out, coeff_out, s);
-        }
-        case DCTP_PATH_SIMT:
-            return launch_simt(x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, s);
-        default:
-            return fail(DCTP_E_INVALID, "unknown path %d", path);
+    Call c = {x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, nullptr};
+    c.first = dense_first(c);
+    Route r = R_SIMT;
+    const char* needs = "";
+    switch (path) {
+        case DCTP_PATH_AUTO: r = auto_route(c); break;
+        case DCTP_PATH_UMMA: r = H <= 64 ? R_UMMA64 : R_UMMA128; needs = "UMMA path takes contiguous square maps of side <= 128"; break;
+        case DCTP_PATH_TMEM:
+            r = R_TMEM;
+            needs = "TMEM-operand path takes dense 16-B aligned square maps of side 5..64 (odd sides: up to 13, and a whole number of float4 in the call)";
+            break;
+        case DCTP_PATH_KRON: r = R_KRON; needs = "Kronecker path takes dense 16-B aligned square maps of side <= 8"; break;
+        case DCTP_PATH_STACK:
+            r = R_STACK;
+            needs = "stacked-basis path takes dense 16-B aligned square maps of even side 10..64 (above 32: multiples of 4)";
+            break;
+        case DCTP_PATH_LARGE: r = R_LARGE; needs = "large-map path takes dense 16-B aligned square maps, side 80..320 multiple of 16"; break;
     }
+    if (!takes(r, c)) return fail(DCTP_E_UNSUPPORTED, "%s (got %dx%d, stride_h %lld)", needs, H, W, stride_h);
+    return launch(r, c, static_cast<cudaStream_t>(stream));
 }
 
 int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, void* stream) {
@@ -1214,22 +1152,27 @@ int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, vo
             if (static_cast<long long>(sites[i].B) * sites[i].c_count > (1ll << 30)) return fail(DCTP_E_INVALID, "too many maps in site %d", i);
         }
         cudaStream_t s = static_cast<cudaStream_t>(stream);
-        const bool kron = H == W && H <= 8 && g.kron_on, stack = H == W && g.stack_on && stack_shape_supported(H);
-        const bool large = !kron && !stack && large_shape_ok(H, W, W);
-        // one launch per SCORE_MAX_SEG sites; shapes the multi-site kernels do not take, and sites that are not 16-byte aligned,
-        // go through the single-site entry below
+        // sites AUTO gives to a multi-site kernel: one launch per SCORE_MAX_SEG of them; the others go through the single-site
+        // entry below
         SiteDesc batch[SCORE_MAX_SEG];
         int nb = 0;
+        Route batched = R_SIMT;
         for (int i = 0; i < n_sites; ++i) {
-            if (sites[i].B == 0 || sites[i].c_count == 0) continue;
-            if (!(kron || stack || large) || (reinterpret_cast<uintptr_t>(sites[i].x) % 16) != 0) { single.push_back(i); continue; }
-            batch[nb++] = SiteDesc{sites[i].x, sites[i].B, sites[i].c_count, sites[i].accum};
-            if (nb == SCORE_MAX_SEG || i == n_sites - 1) {
-                if ((rc = kron ? launch_kron(batch, nb, H, nullptr, nullptr, s) : stack ? launch_stack(batch, nb, H, nullptr, nullptr, s) : launch_large(batch, nb, H, nullptr, nullptr, s))) return rc;
+            const dctp_site& site = sites[i];
+            if (site.B == 0 || site.c_count == 0) continue;
+            Call c = {site.x, site.B, H, W, static_cast<long long>(site.c_count) * H * W, static_cast<long long>(H) * W, W, 0, site.c_count,
+                      site.accum, nullptr, nullptr, nullptr};
+            c.first = dense_first(c);
+            const Route r = auto_route(c);
+            if (!multi_site(r)) { single.push_back(i); continue; }
+            batched = r;                                     // (the same for every dense site of the shape)
+            batch[nb++] = SiteDesc{c.first, site.B, site.c_count, site.accum};
+            if (nb == SCORE_MAX_SEG) {
+                if ((rc = launch_sites(r, batch, nb, H, nullptr, nullptr, s))) return rc;
                 nb = 0;
             }
         }
-        if (nb > 0 && (rc = kron ? launch_kron(batch, nb, H, nullptr, nullptr, s) : stack ? launch_stack(batch, nb, H, nullptr, nullptr, s) : launch_large(batch, nb, H, nullptr, nullptr, s))) return rc;
+        if (nb > 0 && (rc = launch_sites(batched, batch, nb, H, nullptr, nullptr, s))) return rc;
     }
     for (int i : single) {
         const int rc = dctp_score_accum(sites[i].x, sites[i].B, H, W, static_cast<long long>(sites[i].c_count) * H * W, static_cast<long long>(H) * W, W, 0,

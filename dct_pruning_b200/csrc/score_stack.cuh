@@ -93,19 +93,25 @@ struct StackSmem {
 };
 
 
+// Role groups: converters in NCG groups (group g converts the CTA's tiles g, g + NCG, ...), NE1G epilogue-1 groups and NE2G
+// epilogue-2 groups (group g takes the CTA's tiles g, g + NE1G / NE2G, ...).
+constexpr int STACK_NCG = 2, STACK_NE1G = 1, STACK_NE2G = 2;
+// warps of a CTA with NCONV converter warps: converters, epilogue 1 (8 per group), epilogue 2 (4 per group), producer, two issuers
+constexpr int stack_warps(int nconv) { return nconv + 8 * STACK_NE1G + 4 * STACK_NE2G + 3; }
+
 // KP: contraction length per map (N rounded up to 16); VEC: granularity of a row in the fp32 stream (4: N % 4 == 0, 2: N even)
-// NCONV: converter warps (8 or 12) in NCG groups (group g converts the CTA's tiles g, g + NCG, ...); NE1G / NE2G: epilogue-1 / epilogue-2
-// groups (1 or 2; group g takes the CTA's tiles g, g + 2, ...).
+// NCONV: converter warps (8 or 12).
 // Every warp polls the mbarriers it depends on itself.  (Measured and dropped: one polling warp per role releasing its siblings
 // through a named barrier - the polls cost issue slots, the sleep behind mbarrier.try_wait being woken by any barrier event of
 // the CTA, but the extra hop costs more: 56x56 3.17 against 3.49 TB/s.)
-// NP8: Np / 8 as a compile-time constant (0: read it from the arguments) - epilogue 1's column loops lose their branches.
+// NP8: Np / 8 as a compile-time constant - epilogue 1's column loops lose their branches.
 // TRACE: the debug instantiation - the cycle accounting of DCTP_S_TRACE, the per-map energies (energy_out) and the coefficient dump
 // (coeff_out); the production instantiations carry none of that code (the host routes launches that ask for any of it here).
-template <int KP, int VEC, int NCONV, int NE1G, int NCG, int NE2G = 1, int NP8 = 0, bool TRACE = false>
-__global__ void __launch_bounds__((NCONV + 8 * NE1G + 4 * NE2G + 3) * 32, 1) score_stack_kernel(const __grid_constant__ ScoreTensorMaps tmaps, const __grid_constant__ StackArgs a) {
+template <int KP, int VEC, int NCONV, int NP8, bool TRACE>
+__global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel(const __grid_constant__ ScoreTensorMaps tmaps, const __grid_constant__ StackArgs a) {
     using S = StackSmem;
     using namespace umma;
+    constexpr int NCG = STACK_NCG, NE1G = STACK_NE1G, NE2G = STACK_NE2G;
     constexpr int J = KP <= 32 ? 64 / KP : 1;
     constexpr int K1S = J * KP / 16, K2S = KP / 16;
     constexpr int G = KP == 16 ? 8 : KP == 32 ? 4 : 2, T2 = G / 2;
@@ -433,7 +439,7 @@ __global__ void __launch_bounds__((NCONV + 8 * NE1G + 4 * NE2G + 3) * 32, 1) sco
         // ================================================================ epilogue 1: D1 -> y = za + zb -> bf16 hi/lo -> A2
         const uint32_t q = warp & 3u, s = ((warp - W_E1) >> 2) & 1u, eg = (warp - W_E1) >> 3;
         const uint32_t lane_q = (q * 32u) << 16, lane_s = (q * 32u + s * 16u) << 16;
-        const int np8 = NP8 ? NP8 : (a.Np >> 3);
+        constexpr int np8 = NP8;
         tr_me = tr_on && warp == W_E1 && lane == 0;
         auto convert16 = [&](const uint32_t (&za)[8], const uint32_t (&zb)[8], uint32_t dst_hi, uint32_t dst_lo) {
             uint32_t h[4], l[4];
@@ -618,7 +624,7 @@ __global__ void __launch_bounds__((NCONV + 8 * NE1G + 4 * NE2G + 3) * 32, 1) sco
                 }
             } else {
                 // per-map energies asked for: the shares of a map are summed in a fixed order (bit-reproducible fp32 energy)
-                float* red_w = red + (NE2G == 2 ? eg2 : (n & 1u)) * 32;      // (one group: alternate; two: each its own)
+                float* red_w = red + eg2 * 32;                             // (each epilogue-2 group its own)
                 if (r == 0)
 #pragma unroll
                     for (int t = 0; t < T2; ++t) red_w[q * 8 + 2 * t + s] = e[t];

@@ -150,7 +150,8 @@ int dctp_score_host(const float* x_host, int B, int C, int H, int W, int c_begin
  * the number of kernel launches issued by this library since dctp_init(), SM count of the device. */
 int dctp_path_for(int H, int W, long long stride_h);
 /* resident CTAs per SM of the tensor-core kernel instantiation (kp in {64,128}; load mode 0..5: dense
- * 8/4/2-byte scatter, generic 128/64/32-bit loads) at a typical table size */
+ * 8/4/2-byte scatter, generic 128/64/32-bit loads) at a typical table size.  DCTP_E_UNSUPPORTED for kp 128
+ * with mode 2: no side that kernel serves has 2-byte scatter entries, so that instantiation is not built. */
 int dctp_occupancy(int kp, int mode);
 long long dctp_launch_count(void);
 /* Name of the kernel instantiation the most recent dctp_score_accum call launched (AUTO's choice made visible: bench.py labels
