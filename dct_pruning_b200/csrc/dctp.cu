@@ -85,9 +85,6 @@ struct State {
     // scratch of dctp_score_host (grow-only)
     float* hx = nullptr; size_t hx_bytes = 0;
     double* hacc = nullptr; float* hout = nullptr; size_t hc = 0;
-    // scratch of dctp_score_op's DCT3 (grow-only): per-channel sums, per-(image, channel) energies
-    double* d3_part = nullptr; size_t d3_part_n = 0;
-    float* d3_energy = nullptr; size_t d3_energy_n = 0;
 } g;
 
 void note_kernel(const char* fmt, ...) {
@@ -1052,7 +1049,7 @@ int dctp_shutdown(void) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (!g.ready) return DCTP_OK;
     for (void* p : g.bases) cudaFree(p);
-    cudaFree(g.status); cudaFree(g.hx); cudaFree(g.hacc); cudaFree(g.hout); cudaFree(g.d3_part); cudaFree(g.d3_energy);
+    cudaFree(g.status); cudaFree(g.hx); cudaFree(g.hacc); cudaFree(g.hout);
     g = State();
     return DCTP_OK;
 }
@@ -1183,6 +1180,21 @@ int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, vo
 }
 
 // ------------------------------------------------------------------ alternative scoring ops (SURVEY §8f-3)
+// DCTP_OP_DCT3 with caller-owned scratch: per-channel sums part [c_count], and per-(image, channel) energies [B * c_count] when
+// values_out is wanted
+static int dct3_energy(const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h, int c_begin,
+                       int c_count, double* accum, float* values_out, double* part, float* energy, cudaStream_t s) {
+    CUDA_TRY(cudaMemsetAsync(part, 0, sizeof(double) * c_count, s));
+    int rc = dctp_score_accum(x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, part, energy, nullptr, DCTP_PATH_AUTO, s);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (values_out) dct3_reduce_kernel<<<B, 256, 0, s>>>(energy, c_count, values_out, accum);
+    else sum_to_one_kernel<<<1, 256, 0, s>>>(part, c_count, accum);
+    ++g.launches;
+    CUDA_TRY(cudaGetLastError());
+    return DCTP_OK;
+}
+
 int dctp_score_op(int op, const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
                   int c_begin, int c_count, double* accum, float* values_out, void* stream) {
     if (op == DCTP_OP_DCT2)
@@ -1234,36 +1246,22 @@ int dctp_score_op(int op, const float* x, int B, int H, int W, long long stride_
     if (B < 0 || c_count < 0) return fail(DCTP_E_INVALID, "dctp_score_op: B=%d c_count=%d", B, c_count);
     if (B == 0 || c_count == 0) return DCTP_OK;
     if (!accum) return fail(DCTP_E_INVALID, "dctp_score_op: null pointer");
-    double* part = nullptr;
-    float* energy = nullptr;
     {
         std::lock_guard<std::mutex> lk(g_mu);
         int rc = ensure_init();
         if (rc) return rc;
-        if (static_cast<size_t>(c_count) > g.d3_part_n) {
-            CUDA_TRY(cudaStreamSynchronize(s));                             // the old scratch may still be in use on this stream
-            cudaFree(g.d3_part); g.d3_part = nullptr; g.d3_part_n = 0;
-            CUDA_TRY(cudaMalloc(&g.d3_part, sizeof(double) * c_count));
-            g.d3_part_n = c_count;
-        }
-        const size_t ne = static_cast<size_t>(B) * c_count;
-        if (values_out && ne > g.d3_energy_n) {
-            CUDA_TRY(cudaStreamSynchronize(s));
-            cudaFree(g.d3_energy); g.d3_energy = nullptr; g.d3_energy_n = 0;
-            CUDA_TRY(cudaMalloc(&g.d3_energy, sizeof(float) * ne));
-            g.d3_energy_n = ne;
-        }
-        part = g.d3_part;
-        energy = values_out ? g.d3_energy : nullptr;
-        CUDA_TRY(cudaMemsetAsync(part, 0, sizeof(double) * c_count, s));
     }
-    int rc = dctp_score_accum(x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, part, energy, nullptr, DCTP_PATH_AUTO, stream);
+    // the scratch is allocated and freed on the caller's stream: calls on different streams never share it, and a call captured
+    // into a graph allocates inside the graph
+    const size_t part_bytes = sizeof(double) * ((c_count + 1) & ~1);   // the energies start 16-byte aligned
+    void* scratch = nullptr;
+    CUDA_TRY(cudaMallocAsync(&scratch, part_bytes + (values_out ? sizeof(float) * B * c_count : 0), s));
+    double* part = static_cast<double*>(scratch);
+    float* energy = values_out ? reinterpret_cast<float*>(static_cast<char*>(scratch) + part_bytes) : nullptr;
+    const int rc = dct3_energy(x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, values_out, part, energy, s);
+    const cudaError_t freed = cudaFreeAsync(scratch, s);
     if (rc) return rc;
-    std::lock_guard<std::mutex> lk(g_mu);
-    if (values_out) dct3_reduce_kernel<<<B, 256, 0, s>>>(energy, c_count, values_out, accum);
-    else sum_to_one_kernel<<<1, 256, 0, s>>>(part, c_count, accum);
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(freed);
     return DCTP_OK;
 }
 

@@ -28,7 +28,7 @@ constexpr int RANK_EPT = 8;            // elements of a vector per lane (registe
 constexpr int RANK_MAX_SWEEPS = 30;    // LAPACK's xGESVJ bound; fp32 maps converge in 5-9
 constexpr int RANK_MAX_LEN = 256;      // longest vector: 32 lanes x 8 elements
 constexpr float RANK_NEGLIGIBLE = 1.4e-20f;   // (1e-3 * eps_fp32)^2, on squared norms
-constexpr int RANK_SMEM_MAX = 200 * 1024;   // a map (n vectors, odd leading dimension) has to fit: side <= 224
+constexpr int RANK_SMEM_MAX = 200 * 1024;   // a map (n vectors, odd leading dimension) has to fit: side <= 225, 256 x 198
 
 struct RankArgs {
     const float* x;

@@ -105,7 +105,9 @@ int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, vo
  *   DCTP_OP_DCT3     utils/common.py:269  dct_3d(output[i,:,:,:]) -> cnt_score: ONE value per image, accum[0] += sum_b energy of the
  *                    3-D coefficient cube over channels [c_begin, c_begin + c_count) (accum has ONE entry for this op)
  * values_out  optional fp32: per-(image, channel) value [B * c_count] for DCT2 / RANK / RANK_SQ, per-image energy [B] for DCT3.
- * RANK / RANK_SQ hold a map in shared memory: longer side <= 256 and side <= 224 for square maps (DCTP_E_UNSUPPORTED beyond). */
+ * RANK / RANK_SQ hold a map in shared memory: longer side m <= 256 and (n * (m | 1) + n + 1) * 4 bytes <= 200 KiB, n the shorter
+ * side, which is side <= 225 for square maps and shorter side <= 198 at a longer side of 256 (DCTP_E_UNSUPPORTED beyond).
+ * Every call may run on its own stream: DCT3 allocates its scratch on the caller's stream (stream-ordered, graph-capturable). */
 #define DCTP_OP_DCT2     0
 #define DCTP_OP_RANK     1
 #define DCTP_OP_RANK_SQ  2

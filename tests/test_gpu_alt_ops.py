@@ -12,6 +12,9 @@ import numpy as np
 import pytest
 import torch
 
+from dct_pruning_b200 import _lib
+from oracle import alt_ops_port as ao
+
 pytestmark = pytest.mark.gpu
 
 
@@ -133,6 +136,70 @@ def test_dct3_energy_matches_3d_transform(lib, cuda_device, shape):
     st = ScoreState()
     ao.hook_dct3(st)(None, None, x)
     np.testing.assert_allclose(float(accum[0]) / shape[0], float(st.feature_result[0]), rtol=1e-4)
+
+
+def test_dct3_calls_on_two_streams_keep_their_own_scratch(lib, cuda_device):
+    """A long dct3 call on one stream and a short one on a second stream, issued back to back with no synchronisation: both
+    equal float64.  The 24x20 maps take the CUDA-core kernel, which leaves room on the SMs for the short call to run while
+    the long one is still accumulating; with scratch shared between calls, the short call's memset and sums land in the
+    long call's partial sums.  Both routes: per-channel sums (no per-image values) and per-image energies."""
+    from dct_pruning_b200.ops import score_op
+    g = torch.Generator().manual_seed(11)
+    big = torch.rand(128, 816, 24, 20, generator=g)                  # 200 MB
+    small = torch.rand(2, 4, 24, 20, generator=g)
+    want_big = big.double().square().sum((1, 2, 3)).numpy()            # Parseval: the orthonormal 3-D DCT keeps the sum of squares
+    want_small = ao.dct3_energy64(small.numpy())
+    xb, xs = big.to(cuda_device), small.to(cuda_device)
+    s1, s2 = torch.cuda.Stream(), torch.cuda.Stream()
+    for want_values in (False, True):
+        acc1 = torch.zeros(1, dtype=torch.float64, device=cuda_device)
+        acc2 = torch.zeros(1, dtype=torch.float64, device=cuda_device)
+        torch.cuda.synchronize()
+        with torch.cuda.stream(s1):
+            _, v1 = score_op(xb, 'dct3', accum=acc1, want_values=want_values, check=False)
+        with torch.cuda.stream(s2):
+            _, v2 = score_op(xs, 'dct3', accum=acc2, want_values=want_values, check=False)
+        torch.cuda.synchronize()
+        _lib.check(lib.dctp_check(None))
+        np.testing.assert_allclose(float(acc1[0]), want_big.sum(), rtol=1e-4, err_msg='long call, values=%s' % want_values)
+        np.testing.assert_allclose(float(acc2[0]), want_small.sum(), rtol=1e-4, err_msg='short call, values=%s' % want_values)
+        if want_values:
+            np.testing.assert_allclose(v1.cpu().numpy(), want_big, rtol=1e-4)
+            np.testing.assert_allclose(v2.cpu().numpy(), want_small, rtol=1e-4)
+
+
+def test_dct3_captured_in_a_cuda_graph(lib, cuda_device):
+    """Both dct3 routes captured into one CUDA graph (the scratch is allocated and freed inside it) and replayed with two
+    different inputs: each replay equals float64."""
+    g = torch.Generator().manual_seed(12)
+    x = torch.rand(4, 16, 14, 14, generator=g).to(cuda_device)
+    acc_sum = torch.zeros(1, dtype=torch.float64, device=cuda_device)
+    acc_val = torch.zeros(1, dtype=torch.float64, device=cuda_device)
+    vals = torch.zeros(4, dtype=torch.float32, device=cuda_device)
+
+    def both():
+        for acc, out in ((acc_sum, None), (acc_val, vals)):
+            _lib.check(lib.dctp_score_op(_lib.OP_DCT3, _lib.ptr(x), 4, 14, 14, x.stride(0), x.stride(1), x.stride(2), 0, 16,
+                                         _lib.ptr(acc), _lib.ptr(out), _lib.current_stream()))
+
+    both()                                                           # bases uploaded and kernels loaded outside the capture
+    torch.cuda.synchronize()
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        both()
+    for seed in (1, 2):
+        new = torch.relu(torch.randn(4, 16, 14, 14, generator=torch.Generator().manual_seed(seed)))
+        x.copy_(new)
+        acc_sum.zero_()
+        acc_val.zero_()
+        vals.fill_(float('nan'))
+        graph.replay()
+        torch.cuda.synchronize()
+        _lib.check(lib.dctp_check(None))
+        want = ao.dct3_energy64(new.numpy())
+        np.testing.assert_allclose(vals.cpu().numpy(), want, rtol=1e-4)
+        np.testing.assert_allclose(float(acc_sum[0]), want.sum(), rtol=1e-4)
+        np.testing.assert_allclose(float(acc_val[0]), want.sum(), rtol=1e-4)
 
 
 @pytest.mark.parametrize('op', ['rank', 'rank_sq', 'dct3'])
