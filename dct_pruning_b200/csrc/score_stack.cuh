@@ -525,6 +525,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         const uint32_t s = lane >> 4, r = lane & 15u;
         const uint32_t my_set = J == 4 ? q : J == 2 ? (q >> 1) : 0u;
         const uint32_t my_v = J == 4 ? r : J == 2 ? 16u * (q & 1u) + r : 16u * q + r;
+        const uint32_t my_v0 = my_v - r;                                  // the warp's share of a map: basis rows [my_v0, my_v0 + 16)
         uint32_t n = eg2;
         int sg = 0, chan_sg = -1;
         uint32_t chan0 = 0, chan_step = 0;
@@ -619,7 +620,13 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                     if (m0 + ml < seg_maps) {
                         uint32_t ch = chan0 + ml;
                         while (ch >= C) ch -= C;
-                        atomicAdd(accum + ch, static_cast<double>(mine));
+                        // With J > 1 a non-finite map in the tile (rare: see map_energy64) makes every share of the maps of its lanes
+                        // non-finite: the share of rows from 0 then carries the map's whole fp64 energy (NaN for that map itself), the
+                        // others 0.  (With J = 1 the maps of a tile never meet in one contraction.)
+                        double share = mine;
+                        if (J > 1 && !isfinite(mine))
+                            share = my_v0 == 0 ? detail::map_energy64(a.seg.x[sg] + static_cast<long long>(m0 + ml) * a.NN, a.N) : 0.0;
+                        atomicAdd(accum + ch, share);
                     }
                 }
             } else {
@@ -639,7 +646,12 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                     if (m < seg_maps) {
                         uint32_t ch = chan0 + et;
                         while (ch >= C) ch -= C;
-                        atomicAdd(accum + ch, static_cast<double>(en));
+                        double e = en;
+                        if (!isfinite(en)) {                       // a non-finite map in the tile (rare: see map_energy64)
+                            e = detail::map_energy64(a.seg.x[sg] + static_cast<long long>(m) * a.NN, a.N);
+                            en = static_cast<float>(e);
+                        }
+                        atomicAdd(accum + ch, e);
                         a.energy_out[m] = en;
                     }
                 }

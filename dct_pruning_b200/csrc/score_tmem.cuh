@@ -471,7 +471,12 @@ __global__ void __launch_bounds__(128 * (NSLOT + NPROD), 1) score_t_kernel(const
             for (uint32_t o = 16; o > 0; o >>= 1)
                 if (o < tpm) s += __shfl_xor_sync(0xffffffffu, s, o);
             if ((int)red_t < maps_here && red_sub == 0) {
-                atomicAdd(a.accum + chan, (double)s);
+                double e = s;
+                if (!isfinite(s)) {                                // a non-finite map in the tile (rare: see map_energy64)
+                    e = detail::map_energy64(a.x_dense + static_cast<long long>(map0 + (int)red_t) * a.NN, a.N);
+                    s = static_cast<float>(e);
+                }
+                atomicAdd(a.accum + chan, e);
                 if (a.energy_out) a.energy_out[map0 + (int)red_t] = s;
             }
             chan += a.chan_step;                                   // (map0 + red_t) mod c_count, without the division

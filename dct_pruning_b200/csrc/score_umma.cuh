@@ -252,6 +252,23 @@ __device__ __forceinline__ void issue_ts_pass_n(int ks, uint32_t d, uint32_t a_c
     }
 }
 
+// The fp64 energy of one map, recomputed from global memory.  The tensor-core kernels call it only when the fp32 energy they
+// computed is not finite; a finite map gives a finite value unless its fp32 energy overflows, so clean inputs never get here.
+// Kernels that put several maps into one MMA keep them apart with zero blocks in an operand, and 0 * NaN and 0 * Inf are NaN:
+// a non-finite map turns the energies of the other maps of its tile non-finite too.  This tells the two apart: NaN if the
+// N x N map at x (rows N floats apart) holds a NaN or an Inf - it is the culprit -, otherwise its sum of squares (Parseval: the
+// orthonormal DCT keeps it), exactly 0 for a dead map.
+__device__ __forceinline__ double map_energy64(const float* x, int N) {
+    double s = 0.0;
+#pragma unroll 1
+    for (int i = 0; i < N * N; ++i) {
+        const double e = x[i];
+        if (!isfinite(e)) return __longlong_as_double(0x7FF8000000000000ll);
+        s = fma(e, e, s);
+    }
+    return s;
+}
+
 }  // namespace detail
 
 template <int KP>
@@ -601,7 +618,15 @@ __global__ void __launch_bounds__(128, KP == 64 ? 4 : 1) score_umma_kernel(const
             for (uint32_t o = 16; o > 0; o >>= 1)
                 if (o < tpm) s += __shfl_xor_sync(0xffffffffu, s, o);
             if (live && red_sub == 0) {
-                atomicAdd(a.accum + chan, (double)s);
+                double e = s;
+                if (!isfinite(s)) {                                // a non-finite map in the tile (rare: see map_energy64)
+                    const int m = map0 + (int)red_t, b = m / a.c_count;
+                    const float* xm = DENSE ? a.x_dense + static_cast<long long>(m) * a.NN
+                                            : a.x + b * a.stride_b + static_cast<long long>(a.c_begin + m - b * a.c_count) * a.stride_c;
+                    e = detail::map_energy64(xm, a.N);
+                    s = static_cast<float>(e);
+                }
+                atomicAdd(a.accum + chan, e);
                 if (a.energy_out) a.energy_out[map0 + (int)red_t] = s;
             }
             chan += a.chan_step;                                   // (map0 + red_t) mod c_count, without the division

@@ -72,7 +72,19 @@ int dctp_prepare(int H, int W);
  * accum       fp64 [c_count], caller-zeroed before the first batch, accumulated across calls
  * energy_out  optional fp32 [B * c_count]: per-(image, channel) energies, image-major (may be NULL)
  * coeff_out   optional fp32 [B * c_count * H * W]: the DCT coefficients themselves (debug / parity; NULL in production)
- * path        DCTP_PATH_* */
+ * path        DCTP_PATH_*
+ *
+ * Non-finite input.  Call a map non-finite if one of its elements is NaN or +-Inf.  As in the reference, which scores every
+ * (image, channel) slice on its own, a non-finite map changes only its own channel:
+ *   1. a channel with a non-finite map gets a non-finite accum entry, and the map a non-finite energy_out entry (NaN or Inf);
+ *   2. every other channel and map gets the value it would get without that map; a dead map (all +0.0 or all -0.0) scores
+ *      exactly 0, also in the same tile as a non-finite map;
+ *   3. DCTP_OP_DCT3: values_out[b] is non-finite exactly for the images with a non-finite map inside the window;
+ *   4. the call sets no status word for it: dctp_check returns DCTP_OK, also when every map is non-finite.
+ * The tensor-core kernels that put several maps into one MMA test every contribution to accum / energy_out for finiteness and
+ * recompute a non-finite one in fp64 from the map in global memory.  A finite map whose fp32 energy overflows (elements of about
+ * 1e18 and more) is outside these rules: depending on the kernel its channel gets Inf or an fp64 value.  coeff_out of a map that
+ * shares a tile with a non-finite map is not specified: it is a debug dump. */
 int dctp_score_accum(const float* x, int B, int H, int W,
                      long long stride_b, long long stride_c, long long stride_h,
                      int c_begin, int c_count,

@@ -14,8 +14,8 @@ mod 16 for the unaligned fallbacks):
   energy_out, coeff_out (fp32)   guards -0.0, compared bitwise; the live region starts as NaN, so every element must be written.
 
 Oracle: float64 sums of squares (Parseval) per map and per channel, scipy's dctn for the coefficients of small cases, exactly 0
-for dead maps (all +0.0 or all -0.0).  NaN never sits inside the caller's tensors (a non-finite map may legitimately reach other
-maps of its tile through the zero blocks of the tensor-core kernels' bases).
+for dead maps (all +0.0 or all -0.0).  NaN never sits inside the caller's tensors here; what a non-finite map does to its own and
+to the other channels is pinned by test_gpu_nonfinite.py.
 
 The module records which kernel instantiation every score launch ran (dctp_last_kernel); its last test checks that the cases
 reached each one in REQUIRED.
