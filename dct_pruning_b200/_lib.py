@@ -16,6 +16,14 @@ OPS = {'dct2': OP_DCT2, 'rank': OP_RANK, 'rank_sq': OP_RANK_SQ, 'dct3': OP_DCT3}
 
 OK, E_INVALID, E_CUDA, E_UNSUPPORTED, E_DEVICE = 0, -1, -2, -3, -4
 
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2
+
+
+def dtype_code(dtype):
+    """DCTP_DTYPE_* of a torch dtype the score entries read (fp32, bf16, fp16), None for any other."""
+    import torch
+    return {torch.float32: DTYPE_F32, torch.bfloat16: DTYPE_BF16, torch.float16: DTYPE_F16}.get(dtype)
+
 _c = ctypes
 _SIGNATURES = {
     'dctp_version': (_c.c_int, []),
@@ -28,7 +36,13 @@ _SIGNATURES = {
                                     _c.c_int, _c.c_int,
                                     _c.c_void_p, _c.c_void_p, _c.c_void_p,
                                     _c.c_int, _c.c_void_p]),
+    'dctp_score_accum_ex': (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_int,
+                                       _c.c_longlong, _c.c_longlong, _c.c_longlong,
+                                       _c.c_int, _c.c_int,
+                                       _c.c_void_p, _c.c_void_p, _c.c_void_p,
+                                       _c.c_int, _c.c_void_p]),
     'dctp_score_accum_multi': (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p]),
+    'dctp_score_accum_multi_ex': (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p]),
     'dctp_score_op': (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_int, _c.c_int, _c.c_int,
                                  _c.c_longlong, _c.c_longlong, _c.c_longlong,
                                  _c.c_int, _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p]),
@@ -50,7 +64,7 @@ EXPORTS = tuple(_SIGNATURES)
 
 
 class Site(_c.Structure):
-    """dctp_site of include/dctp.h: one dense activation of a multi-site launch."""
+    """dctp_site of include/dctp.h: one dense activation of a multi-site launch (x: of the call's dtype)."""
     _fields_ = [('x', _c.c_void_p), ('accum', _c.c_void_p), ('B', _c.c_int), ('c_count', _c.c_int)]
 
 

@@ -52,6 +52,10 @@ def build_parser():
                    help="per-slice reduction: dct2 (utils/common.py:267, the default) or one of the lines the reference keeps commented out "
                         "beside it: rank (HRank's matrix_rank, :268), rank_sq (the same through the unchanged cnt_score), dct3 (:269)")
     p.add_argument('--input_side', type=int, default=None, help='override the input resolution (e.g. 288 for DUTS crops)')
+    p.add_argument('--amp', type=str, default='off', choices=('off', 'bf16', 'fp16'),
+                   help='run the forward under torch.autocast in bf16 or fp16 (faster on a B200).  The scores then come from the '
+                        'reduced-precision forward\'s activations and differ from the fp32 forward\'s (the reference\'s); files keep '
+                        'their names and format.  Default: off (fp32 forward)')
     return p
 
 

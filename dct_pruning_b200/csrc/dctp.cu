@@ -20,6 +20,7 @@
 #include "topk.cuh"
 #include "gather.cuh"
 #include "score_alt.cuh"
+#include "widen.cuh"
 
 namespace {
 
@@ -295,25 +296,30 @@ int get_stack_basis(int N, StackBasis& out) {
 // 3.61 at 56x56; converters reading global memory directly behind an L2 bulk prefetch instead of the TMA-staged copy 3.46 against 4.07.
 constexpr int STACK_VARIANTS = 10;
 typedef void (*StackKernel)(const ScoreTensorMaps, const StackArgs);
-template <bool TRACE, int NCONV>
+template <bool TRACE, int NCONV, int IN>
 StackKernel stack_kernel_of(int v) {
     switch (v) {
-        case 0: return score_stack_kernel<16, 4, NCONV, 2, TRACE>;
-        case 1: return score_stack_kernel<16, 2, NCONV, 2, TRACE>;
-        case 2: return score_stack_kernel<32, 4, NCONV, 3, TRACE>;
-        case 3: return score_stack_kernel<32, 4, NCONV, 4, TRACE>;
-        case 4: return score_stack_kernel<32, 2, NCONV, 3, TRACE>;
-        case 5: return score_stack_kernel<32, 2, NCONV, 4, TRACE>;
-        case 6: return score_stack_kernel<48, 4, NCONV, 5, TRACE>;
-        case 7: return score_stack_kernel<48, 4, NCONV, 6, TRACE>;
-        case 8: return score_stack_kernel<64, 4, NCONV, 7, TRACE>;
-        default: return score_stack_kernel<64, 4, NCONV, 8, TRACE>;
+        case 0: return score_stack_kernel<16, 4, NCONV, 2, TRACE, IN>;
+        case 1: return score_stack_kernel<16, 2, NCONV, 2, TRACE, IN>;
+        case 2: return score_stack_kernel<32, 4, NCONV, 3, TRACE, IN>;
+        case 3: return score_stack_kernel<32, 4, NCONV, 4, TRACE, IN>;
+        case 4: return score_stack_kernel<32, 2, NCONV, 3, TRACE, IN>;
+        case 5: return score_stack_kernel<32, 2, NCONV, 4, TRACE, IN>;
+        case 6: return score_stack_kernel<48, 4, NCONV, 5, TRACE, IN>;
+        case 7: return score_stack_kernel<48, 4, NCONV, 6, TRACE, IN>;
+        case 8: return score_stack_kernel<64, 4, NCONV, 7, TRACE, IN>;
+        default: return score_stack_kernel<64, 4, NCONV, 8, TRACE, IN>;
     }
 }
 constexpr int STACK_NCONV = 12, STACK_NCONV_DEBUG = 8;
-StackKernel stack_kernel_fn(bool debug, int v) {
-    return debug ? stack_kernel_of<true, STACK_NCONV_DEBUG>(v) : stack_kernel_of<false, STACK_NCONV>(v);
+template <int IN>
+StackKernel stack_kernel_in(bool debug, int v) {
+    return debug ? stack_kernel_of<true, STACK_NCONV_DEBUG, IN>(v) : stack_kernel_of<false, STACK_NCONV, IN>(v);
 }
+StackKernel stack_kernel_fn(bool debug, int v, int in) {
+    return in == IN_BF16 ? stack_kernel_in<IN_BF16>(debug, v) : in == IN_F16 ? stack_kernel_in<IN_F16>(debug, v) : stack_kernel_in<IN_F32>(debug, v);
+}
+const char* in_name(int in) { return in == IN_BF16 ? "bf16" : in == IN_F16 ? "f16" : "f32"; }
 int stack_variant(int KP, int vec, int np8) {
     if (KP == 16) return vec == 4 ? 0 : 1;
     if (KP == 32) return (vec == 4 ? 2 : 4) + (np8 == 4 ? 1 : 0);
@@ -324,30 +330,32 @@ int stack_variant(int KP, int vec, int np8) {
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// 2-D tensor map over fp32 rows: `rows` rows of `inner` floats, `pitch` bytes apart; box = `box_inner` floats x `box_rows` rows
-int encode_2d(CUtensorMap& map, const float* base, long long inner, long long rows, long long pitch, int box_inner, int box_rows,
-              CUtensorMapL2promotion l2) {
+// 2-D tensor map: `rows` rows of `inner` elements (fp32 unless `in` says otherwise), `pitch` bytes apart; box = `box_inner`
+// elements x `box_rows` rows
+int encode_2d(CUtensorMap& map, const void* base, long long inner, long long rows, long long pitch, int box_inner, int box_rows,
+              CUtensorMapL2promotion l2, int in = IN_F32) {
     std::memset(&map, 0, sizeof map);
     cuuint64_t gdim[2] = {static_cast<cuuint64_t>(inner), static_cast<cuuint64_t>(rows)};
     cuuint64_t gstr[1] = {static_cast<cuuint64_t>(pitch)};
     cuuint32_t box[2] = {static_cast<cuuint32_t>(box_inner), static_cast<cuuint32_t>(box_rows)}, estr[2] = {1, 1};
     const CUresult r = reinterpret_cast<EncodeTiledFn>(g.encode_tiled)(
-        &map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+        &map, in == IN_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : in == IN_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
+        const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
         CU_TENSOR_MAP_SWIZZLE_NONE, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS)
-        return fail(DCTP_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for %lld rows of %lld floats, box %d x %d", (int)r, rows, inner,
-                    box_inner, box_rows);
+        return fail(DCTP_E_CUDA, "cuTensorMapEncodeTiled failed (%d) for %lld rows of %lld %s elements, box %d x %d", (int)r, rows, inner,
+                    in_name(in), box_inner, box_rows);
     return DCTP_OK;
 }
 
-// a dense fp32 stream viewed as [rows, 32 floats] (whole 128-byte rows only), box = `box_rows` rows
-int encode_flat_map(CUtensorMap& map, const float* first, long long total_elems, int box_rows) {
+// a dense stream viewed as [rows, 32 elements] (whole rows only: 128 bytes of fp32, 64 of 16-bit input), box = `box_rows` rows
+int encode_flat_map(CUtensorMap& map, const void* first, long long total_elems, int box_rows, int in = IN_F32) {
     const long long rows = total_elems / 32;
     if (rows <= 0) {                                         // (never dereferenced: the only tile is converted from global memory)
         std::memset(&map, 0, sizeof map);
         return DCTP_OK;
     }
-    return encode_2d(map, first, 32, rows, 128, 32, box_rows, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    return encode_2d(map, first, 32, rows, 32 * in_bytes(in), 32, box_rows, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, in);
 }
 
 // Score kernels are launched with programmatic stream serialization: their prologue (shared-memory fill, basis staging,
@@ -368,7 +376,7 @@ cudaError_t launch_pdl(void (*kern)(Params...), int grid, int block, size_t smem
     return cudaLaunchKernelEx(&cfg, kern, args...);
 }
 
-struct SiteDesc { const float* first; int B; int c_count; double* accum; };     // one dense activation: B * c_count maps back to back
+struct SiteDesc { const void* first; int B; int c_count; double* accum; };      // one dense activation: B * c_count maps back to back
 
 // fills seg (tile ranges, per-site sizes); returns the launch's tile count
 int fill_segments(ScoreSegments& seg, const SiteDesc* sites, int n, int NN, int maps_per_tile) {
@@ -388,7 +396,7 @@ int fill_segments(ScoreSegments& seg, const SiteDesc* sites, int n, int NN, int 
 }
 
 // up to SCORE_MAX_SEG dense activations of side N in ONE launch (energy_out / coeff_out: single-site launches only)
-int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, cudaStream_t stream) {
+int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, int in, cudaStream_t stream) {
     StackBasis basis;
     int rc = get_stack_basis(N, basis);
     if (rc) return rc;
@@ -406,7 +414,7 @@ int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* 
     a.energy_out = n == 1 ? energy_out : nullptr; a.dump = n == 1 ? coeff_out : nullptr; a.status = g.status;
     ScoreTensorMaps maps;
     for (int i = 0; i < n; ++i)
-        if ((rc = encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.tile_rows))) return rc;
+        if ((rc = encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.tile_rows, in))) return rc;
     for (int i = n; i < SCORE_MAX_SEG; ++i) maps.m[i] = maps.m[0];
     int grid = g.sm_count < a.num_tiles ? g.sm_count : a.num_tiles;
     const size_t smem = StackSmem::TOTAL;
@@ -421,10 +429,14 @@ int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* 
     const int variant = stack_variant(KP, v4 ? 4 : 2, a.Np / 8);
     // per-map energies, coefficients and the cycle trace live in the debug instantiation (cfg6) only
     const bool debug = a.energy_out || a.dump || tracing;
-    CUDA_TRY(launch_pdl(stack_kernel_fn(debug, variant), grid, 32 * stack_warps(debug ? STACK_NCONV_DEBUG : STACK_NCONV), smem, stream,
+    CUDA_TRY(launch_pdl(stack_kernel_fn(debug, variant, in), grid, 32 * stack_warps(debug ? STACK_NCONV_DEBUG : STACK_NCONV), smem, stream,
                         maps, a));
-    note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP, basis.vec,
-                debug ? 6 : 7);
+    if (in == IN_F32)
+        note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP, basis.vec,
+                    debug ? 6 : 7);
+    else
+        note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d,IN=%s> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP,
+                    basis.vec, debug ? 6 : 7, in_name(in));
     if (tracing) {
         long long h[64];
         CUDA_TRY(cudaMemcpy(h, trace_buf, sizeof h, cudaMemcpyDeviceToHost));
@@ -469,53 +481,75 @@ int get_kron_basis(int N, KronBasis& out) {
     return DCTP_OK;
 }
 
-int launch_kron(const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, cudaStream_t stream) {
+typedef void (*KronKernel)(const ScoreTensorMaps, const KronArgs);
+// the instantiations a (K2, layout, input type) runs on; 16-bit maps take the row layout at sides 4 and 8 only (K2 16 and 64), so
+// 16-bit row-layout kernels of K2 32 and 48 are not built (kron_kernel_built)
+bool kron_kernel_built(int K2, bool even, int in) { return !even || in == IN_F32 || K2 == 16 || K2 == 64; }
+template <int IN>
+KronKernel kron_kernel_in(int K2, bool even) {
+    switch (K2) {
+        case 16: return even ? score_kron_kernel<16, true, IN> : score_kron_kernel<16, false, IN>;
+        case 32:
+            if constexpr (IN == IN_F32)
+                if (even) return score_kron_kernel<32, true, IN>;
+            return score_kron_kernel<32, false, IN>;
+        case 48:
+            if constexpr (IN == IN_F32)
+                if (even) return score_kron_kernel<48, true, IN>;
+            return score_kron_kernel<48, false, IN>;
+        default: return even ? score_kron_kernel<64, true, IN> : score_kron_kernel<64, false, IN>;
+    }
+}
+KronKernel kron_kernel_fn(int K2, bool even, int in) {
+    return in == IN_BF16 ? kron_kernel_in<IN_BF16>(K2, even) : in == IN_F16 ? kron_kernel_in<IN_F16>(K2, even) : kron_kernel_in<IN_F32>(K2, even);
+}
+
+int launch_kron(const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, int in, cudaStream_t stream) {
     KronBasis basis;
     int rc = get_kron_basis(N, basis);
     if (rc) return rc;
     KronArgs a;
     std::memset(&a, 0, sizeof a);
-    const int NN = N * N, K2 = (NN + 15) / 16 * 16;
-    const bool even = (N % 2) == 0;
+    const int NN = N * N, K2 = (NN + 15) / 16 * 16, eb = in_bytes(in);
+    // the row layout needs a row pitch of whole 16-byte units: every even side in fp32, sides 4 and 8 in 16-bit
+    const bool even = (N % 2) == 0 && (NN * eb) % 16 == 0;
     a.N = N; a.NN = NN;
     a.idesc = umma::make_idesc_bf16(128, K2, false, false);
     a.k_hi = basis.hi; a.k_lo = basis.lo;
     a.energy_out = n == 1 ? energy_out : nullptr; a.dump = n == 1 ? coeff_out : nullptr; a.status = g.status;
     if (even) {
         a.sub_tiles = N == 8 ? 1 : 2;
-        a.row_floats = NN + (((NN / 4) % 2) == 0 ? 4 : 0);            // an odd number of 16-byte units per row: conflict-free 128-bit reads
+        const int unit = 16 / eb;                                       // elements per 16-byte unit
+        a.row_elems = NN + (((NN / unit) % 2) == 0 ? unit : 0);         // an odd number of 16-byte units per row: conflict-free 128-bit reads
         a.tile_maps = 128 * a.sub_tiles;
         a.box_rows = a.tile_maps;
-        a.tile_bytes = static_cast<uint32_t>(a.tile_maps) * a.row_floats * 4u;
+        a.tile_bytes = static_cast<uint32_t>(a.tile_maps) * a.row_elems * eb;
     } else {
-        a.sub_tiles = N == 7 ? 1 : N == 5 ? 2 : 4;
-        a.row_floats = NN;
+        // (16-bit 6x6 and 2x2 maps take this layout too; one sub-tile of 6x6 is already 144 rows, and a box holds at most 256)
+        a.sub_tiles = N == 7 || N == 6 ? 1 : N == 5 || N == 2 ? 2 : 4;
+        a.row_elems = NN;
         a.tile_maps = 128 * a.sub_tiles;
         a.box_rows = a.tile_maps * NN / 32;
-        a.tile_bytes = static_cast<uint32_t>(a.box_rows) * 128u;
+        a.tile_bytes = static_cast<uint32_t>(a.box_rows) * 32u * eb;
     }
     a.num_tiles = fill_segments(a.seg, sites, n, NN, a.tile_maps);
     ScoreTensorMaps maps;
     for (int i = 0; i < n; ++i) {
-        // even sides: one map per row of the box, padded to row_floats; odd sides: the flat stream
-        rc = even ? encode_2d(maps.m[i], sites[i].first, NN, a.seg.n_maps[i], 4ll * NN, a.row_floats, a.tile_maps, CU_TENSOR_MAP_L2_PROMOTION_L2_128B)
-                  : encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.box_rows);
+        // even sides: one map per row of the box, padded to row_elems; odd sides: the flat stream
+        rc = even ? encode_2d(maps.m[i], sites[i].first, NN, a.seg.n_maps[i], static_cast<long long>(eb) * NN, a.row_elems, a.tile_maps,
+                              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, in)
+                  : encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.box_rows, in);
         if (rc) return rc;
     }
     for (int i = n; i < SCORE_MAX_SEG; ++i) maps.m[i] = maps.m[0];
     const int grid = g.sm_count < a.num_tiles ? g.sm_count : a.num_tiles;
     const size_t smem = KronSmem::TOTAL;
-#define KRON_LAUNCH(K2V)                                                                                                         \
-    CUDA_TRY(even ? launch_pdl(score_kron_kernel<K2V, true>, grid, KRON_NT, smem, stream, maps, a)                              \
-                  : launch_pdl(score_kron_kernel<K2V, false>, grid, KRON_NT, smem, stream, maps, a))
-    switch (K2) {
-        case 16: KRON_LAUNCH(16); break;
-        case 32: KRON_LAUNCH(32); break;
-        case 48: KRON_LAUNCH(48); break;
-        default: KRON_LAUNCH(64); break;
-    }
-#undef KRON_LAUNCH
-    note_kernel("score_kron_kernel<K2=%d,%s> (tcgen05, single-stage Kronecker, TMA tile ring, warp specialised)", K2, even ? "even" : "odd");
+    CUDA_TRY(launch_pdl(kron_kernel_fn(K2, even, in), grid, KRON_NT, smem, stream, maps, a));
+    if (in == IN_F32)
+        note_kernel("score_kron_kernel<K2=%d,%s> (tcgen05, single-stage Kronecker, TMA tile ring, warp specialised)", K2, even ? "even" : "odd");
+    else
+        note_kernel("score_kron_kernel<K2=%d,%s,IN=%s> (tcgen05, single-stage Kronecker, TMA tile ring, warp specialised)", K2,
+                    even ? "even" : "odd", in_name(in));
     g.launches += 1;
     CUDA_TRY(cudaGetLastError());
     return DCTP_OK;
@@ -637,19 +671,20 @@ int ensure_init() {
         }
     }
     {
-        for (const bool debug : {false, true})
-            for (int v = 0; v < STACK_VARIANTS; ++v) {
-                const void* fn = reinterpret_cast<const void*>(stack_kernel_fn(debug, v));
-                CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(StackSmem::TOTAL)));
-                CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-            }
-        const void* kfns[] = {reinterpret_cast<const void*>(score_kron_kernel<16, true>), reinterpret_cast<const void*>(score_kron_kernel<16, false>),
-                              reinterpret_cast<const void*>(score_kron_kernel<32, true>), reinterpret_cast<const void*>(score_kron_kernel<32, false>),
-                              reinterpret_cast<const void*>(score_kron_kernel<48, true>), reinterpret_cast<const void*>(score_kron_kernel<48, false>),
-                              reinterpret_cast<const void*>(score_kron_kernel<64, true>), reinterpret_cast<const void*>(score_kron_kernel<64, false>)};
-        for (const void* fn : kfns) {
-            CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(KronSmem::TOTAL)));
-            CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+        for (const int in : {IN_F32, IN_BF16, IN_F16}) {
+            for (const bool debug : {false, true})
+                for (int v = 0; v < STACK_VARIANTS; ++v) {
+                    const void* fn = reinterpret_cast<const void*>(stack_kernel_fn(debug, v, in));
+                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(StackSmem::TOTAL)));
+                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+                }
+            for (const int k2 : {16, 32, 48, 64})
+                for (const bool even : {true, false}) {
+                    if (!kron_kernel_built(k2, even, in)) continue;
+                    const void* fn = reinterpret_cast<const void*>(kron_kernel_fn(k2, even, in));
+                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(KronSmem::TOTAL)));
+                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+                }
         }
         cudaDriverEntryPointQueryResult qres;
         CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &g.encode_tiled, cudaEnableDefault, &qres));
@@ -850,22 +885,24 @@ int launch_t(const float* first, int B, int N, int c_count, double* accum, float
     return DCTP_OK;
 }
 
-struct Call {                                            // the arguments of one dctp_score_accum call
-    const float* x;
+struct Call {                                            // the arguments of one dctp_score_accum_ex call
+    const void* x;
     int B, H, W;
     long long stride_b, stride_c, stride_h;
     int c_begin, c_count;
     double* accum;
     float *energy_out, *coeff_out;
-    const float* first;                                  // dense_first()
+    const void* first;                                   // dense_first()
+    int in;                                              // element type of x (IN_*: DCTP_DTYPE_*)
     long long maps() const { return static_cast<long long>(B) * c_count; }
+    const float* xf() const { return static_cast<const float*>(x); }          // (fp32 calls only)
 };
 
-// The first scored map when the call's maps are one contiguous, 16-byte-aligned fp32 stream (packed rows and channels, and
+// The first scored map when the call's maps are one contiguous, 16-byte-aligned stream (packed rows and channels, and
 // images back to back unless there is one), null otherwise.  The TMA-fed kernels read only such streams.
-const float* dense_first(const Call& c) {
+const void* dense_first(const Call& c) {
     const long long hw = static_cast<long long>(c.H) * c.W;
-    const float* first = c.x + static_cast<long long>(c.c_begin) * c.stride_c;
+    const void* first = static_cast<const char*>(c.x) + static_cast<long long>(c.c_begin) * c.stride_c * in_bytes(c.in);
     const bool dense = c.stride_h == c.W && c.stride_c == hw && (c.B == 1 || c.stride_b == c.c_count * hw) &&
                        (reinterpret_cast<uintptr_t>(first) % 16) == 0;
     return dense ? first : nullptr;
@@ -879,7 +916,7 @@ int launch_umma(const Call& c, cudaStream_t stream) {
     if (rc) return rc;
     UmmaScoreArgs a;
     std::memset(&a, 0, sizeof a);
-    a.x = c.x; a.stride_b = c.stride_b; a.stride_c = c.stride_c; a.c_begin = c.c_begin; a.c_count = c.c_count;
+    a.x = c.xf(); a.stride_b = c.stride_b; a.stride_c = c.stride_c; a.c_begin = c.c_begin; a.c_count = c.c_count;
     a.n_maps = c.B * c.c_count;
     a.N = N; a.NN = N * N;
     a.Ms = (N + 7) / 8 * 8; a.G = 128 / a.Ms; a.J = KP / a.Ms; a.MT = a.G * a.J;
@@ -903,12 +940,12 @@ int launch_umma(const Call& c, cudaStream_t stream) {
     int mode;
     if (dense) {
         mode = basis.vpe == 1 ? LOAD_DENSE1 : basis.vpe == 2 ? LOAD_DENSE2 : LOAD_DENSE4;
-        a.x_dense = c.first; a.total_elems = static_cast<long long>(a.n_maps) * a.NN;
+        a.x_dense = static_cast<const float*>(c.first); a.total_elems = static_cast<long long>(a.n_maps) * a.NN;
         a.tile_vec = basis.tile_vec; a.scatter = basis.scatter;
         a.var_bytes = static_cast<uint32_t>(basis.tile_vec) * basis.vpe * 2u;
         a.div_vpm.set(1);
     } else {
-        const int vec = pick_vec(c.x, c.stride_b, c.stride_c, N);
+        const int vec = pick_vec(c.xf(), c.stride_b, c.stride_c, N);
         mode = vec == 4 ? LOAD_GEN4 : vec == 2 ? LOAD_GEN2 : LOAD_GEN1;
         a.var_bytes = 128 * sizeof(void*);
         a.div_vpm.set(a.NN / vec);
@@ -951,7 +988,7 @@ int launch_simt(const Call& c, cudaStream_t stream) {
     if ((rc = get_simt_basis(W, bw))) return rc;
     SimtScoreArgs a;
     std::memset(&a, 0, sizeof a);
-    a.x = c.x; a.stride_b = c.stride_b; a.stride_c = c.stride_c; a.stride_h = c.stride_h;
+    a.x = c.xf(); a.stride_b = c.stride_b; a.stride_c = c.stride_c; a.stride_h = c.stride_h;
     a.c_begin = c.c_begin; a.c_count = c.c_count; a.n_maps = c.B * c.c_count; a.H = H; a.W = W;
     a.basis_h_t = bh.t; a.basis_w_t = bw.t; a.accum = c.accum; a.energy_out = c.energy_out; a.dump = c.coeff_out;
     if (H <= SIMT_T && W <= SIMT_T) {
@@ -1005,7 +1042,7 @@ Route auto_route(const Call& c) {
 // a call on one map at a 16-byte-aligned address: what AUTO and the forced paths do with dense maps of this shape
 Call dense_call(int H, int W, long long stride_h) {
     alignas(16) static const float base[4] = {};
-    Call c = {base, 1, H, W, 0, static_cast<long long>(H) * W, stride_h, 0, 1, nullptr, nullptr, nullptr, nullptr};
+    Call c = {base, 1, H, W, 0, static_cast<long long>(H) * W, stride_h, 0, 1, nullptr, nullptr, nullptr, nullptr, IN_F32};
     c.first = dense_first(c);
     return c;
 }
@@ -1013,21 +1050,23 @@ Call dense_call(int H, int W, long long stride_h) {
 // the kernels that score up to SCORE_MAX_SEG activations in one launch
 static_assert(SCORE_MAX_SEG == LARGE_MAX_SEG, "one multi-site batch size");
 bool multi_site(Route r) { return r == R_KRON || r == R_STACK || r == R_LARGE; }
-int launch_sites(Route r, const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, cudaStream_t s) {
-    if (r == R_KRON) return launch_kron(sites, n, N, energy_out, coeff_out, s);
-    if (r == R_STACK) return launch_stack(sites, n, N, energy_out, coeff_out, s);
+// the kernels that read 16-bit input themselves; every other route scores a widened fp32 copy of the window (score_accum)
+bool reads_16bit(Route r) { return r == R_KRON || r == R_STACK; }
+int launch_sites(Route r, const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, int in, cudaStream_t s) {
+    if (r == R_KRON) return launch_kron(sites, n, N, energy_out, coeff_out, in, s);
+    if (r == R_STACK) return launch_stack(sites, n, N, energy_out, coeff_out, in, s);
     return launch_large(sites, n, N, energy_out, coeff_out, s);
 }
 
 int launch(Route r, const Call& c, cudaStream_t s) {
     switch (r) {
-        case R_TMEM: return launch_t(c.first, c.B, c.H, c.c_count, c.accum, c.energy_out, c.coeff_out, s);
+        case R_TMEM: return launch_t(static_cast<const float*>(c.first), c.B, c.H, c.c_count, c.accum, c.energy_out, c.coeff_out, s);
         case R_UMMA64: return launch_umma<64>(c, s);
         case R_UMMA128: return launch_umma<128>(c, s);
         case R_SIMT: return launch_simt(c, s);
         default: {
             const SiteDesc one = {c.first, c.B, c.c_count, c.accum};
-            return launch_sites(r, &one, 1, c.H, c.energy_out, c.coeff_out, s);
+            return launch_sites(r, &one, 1, c.H, c.energy_out, c.coeff_out, c.in, s);
         }
     }
 }
@@ -1101,20 +1140,24 @@ int dctp_prepare(int H, int W) {
     return get_umma_basis(H, H <= 64 ? 64 : 128, ub);
 }
 
-int dctp_score_accum(const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
-                     int c_begin, int c_count, double* accum, float* energy_out, float* coeff_out, int path,
-                     void* stream) {
-    std::lock_guard<std::mutex> lk(g_mu);
+}  // extern "C"
+
+namespace {
+
+// one score call; the caller holds g_mu
+int score_accum(const void* x, int dtype, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h, int c_begin,
+                int c_count, double* accum, float* energy_out, float* coeff_out, int path, cudaStream_t s) {
     int rc = ensure_init();
     if (rc) return rc;
     if (B < 0 || H < 1 || W < 1 || c_begin < 0 || c_count < 0 || stride_h < W)
         return fail(DCTP_E_INVALID, "dctp_score_accum: B=%d H=%d W=%d c_begin=%d c_count=%d stride_h=%lld", B, H, W, c_begin,
                     c_count, stride_h);
     if (path < DCTP_PATH_AUTO || path > DCTP_PATH_KRON) return fail(DCTP_E_INVALID, "unknown path %d", path);
+    if (dtype != DCTP_DTYPE_F32 && dtype != DCTP_DTYPE_BF16 && dtype != DCTP_DTYPE_F16) return fail(DCTP_E_INVALID, "unknown dtype %d", dtype);
     if (B == 0 || c_count == 0) return DCTP_OK;                     // empty batch / empty window: nothing to add
     if (!x || !accum) return fail(DCTP_E_INVALID, "dctp_score_accum: null pointer");
     if (static_cast<long long>(B) * c_count > (1ll << 30)) return fail(DCTP_E_INVALID, "too many maps in one call");
-    Call c = {x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, nullptr};
+    Call c = {x, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, nullptr, dtype};
     c.first = dense_first(c);
     Route r = R_SIMT;
     const char* needs = "";
@@ -1133,24 +1176,67 @@ int dctp_score_accum(const float* x, int B, int H, int W, long long stride_b, lo
         case DCTP_PATH_LARGE: r = R_LARGE; needs = "large-map path takes dense 16-B aligned square maps, side 80..320 multiple of 16"; break;
     }
     if (!takes(r, c)) return fail(DCTP_E_UNSUPPORTED, "%s (got %dx%d, stride_h %lld)", needs, H, W, stride_h);
-    return launch(r, c, static_cast<cudaStream_t>(stream));
+    if (dtype == DCTP_DTYPE_F32 || reads_16bit(r)) return launch(r, c, s);
+    // 16-bit input on a kernel that reads fp32 only: the scored window is widened into a dense fp32 copy, allocated and freed on the
+    // caller's stream (calls on different streams never share it; a call captured into a graph allocates inside the graph), and scored
+    // as the fp32 entry scores that copy with the same path
+    const long long rows = c.maps() * H;
+    void* buf = nullptr;
+    CUDA_TRY(cudaMallocAsync(&buf, sizeof(float) * rows * W, s));
+    WidenArgs wa = {static_cast<const uint16_t*>(x), stride_b, stride_c, stride_h, c_begin, c_count, H, W, rows, static_cast<float*>(buf)};
+    long long blocks = (rows + 7) / 8;
+    if (blocks > 16ll * g.sm_count) blocks = 16ll * g.sm_count;
+    if (dtype == DCTP_DTYPE_BF16) widen_window_kernel<IN_BF16><<<static_cast<unsigned>(blocks), 256, 0, s>>>(wa);
+    else widen_window_kernel<IN_F16><<<static_cast<unsigned>(blocks), 256, 0, s>>>(wa);
+    ++g.launches;
+    const cudaError_t launched = cudaGetLastError();
+    rc = launched != cudaSuccess ? fail(DCTP_E_CUDA, "widen_window_kernel: %s", cudaGetErrorString(launched)) : DCTP_OK;
+    if (!rc) {
+        Call w = {buf, B, H, W, static_cast<long long>(c_count) * H * W, static_cast<long long>(H) * W, W, 0, c_count, accum, energy_out, coeff_out,
+                  nullptr, IN_F32};
+        w.first = dense_first(w);
+        rc = launch(path == DCTP_PATH_AUTO ? auto_route(w) : r, w, s);
+    }
+    const cudaError_t freed = cudaFreeAsync(buf, s);
+    if (rc) return rc;
+    CUDA_TRY(freed);
+    return DCTP_OK;
 }
 
-int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, void* stream) {
+}  // namespace
+
+extern "C" {
+
+int dctp_score_accum_ex(const void* x, int dtype, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
+                        int c_begin, int c_count, double* accum, float* energy_out, float* coeff_out, int path, void* stream) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    return score_accum(x, dtype, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, path,
+                       static_cast<cudaStream_t>(stream));
+}
+
+int dctp_score_accum(const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
+                     int c_begin, int c_count, double* accum, float* energy_out, float* coeff_out, int path,
+                     void* stream) {
+    return dctp_score_accum_ex(x, DCTP_DTYPE_F32, B, H, W, stride_b, stride_c, stride_h, c_begin, c_count, accum, energy_out, coeff_out, path,
+                               stream);
+}
+
+int dctp_score_accum_multi_ex(const dctp_site* sites, int n_sites, int H, int W, int dtype, void* stream) {
     std::vector<int> single;                                 // sites left to the single-site entry
     {
         std::lock_guard<std::mutex> lk(g_mu);
         int rc = ensure_init();
         if (rc) return rc;
         if (n_sites < 0 || H < 1 || W < 1 || (n_sites > 0 && !sites)) return fail(DCTP_E_INVALID, "dctp_score_accum_multi: n_sites=%d H=%d W=%d", n_sites, H, W);
+        if (dtype != DCTP_DTYPE_F32 && dtype != DCTP_DTYPE_BF16 && dtype != DCTP_DTYPE_F16) return fail(DCTP_E_INVALID, "unknown dtype %d", dtype);
         for (int i = 0; i < n_sites; ++i) {
             if (sites[i].B < 0 || sites[i].c_count < 0 || ((sites[i].B > 0 && sites[i].c_count > 0) && (!sites[i].x || !sites[i].accum)))
                 return fail(DCTP_E_INVALID, "dctp_score_accum_multi: site %d: B=%d c_count=%d or a null pointer", i, sites[i].B, sites[i].c_count);
             if (static_cast<long long>(sites[i].B) * sites[i].c_count > (1ll << 30)) return fail(DCTP_E_INVALID, "too many maps in site %d", i);
         }
         cudaStream_t s = static_cast<cudaStream_t>(stream);
-        // sites AUTO gives to a multi-site kernel: one launch per SCORE_MAX_SEG of them; the others go through the single-site
-        // entry below
+        // sites AUTO gives to a multi-site kernel that reads their dtype: one launch per SCORE_MAX_SEG of them; the others go through
+        // the single-site entry below
         SiteDesc batch[SCORE_MAX_SEG];
         int nb = 0;
         Route batched = R_SIMT;
@@ -1158,25 +1244,30 @@ int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, vo
             const dctp_site& site = sites[i];
             if (site.B == 0 || site.c_count == 0) continue;
             Call c = {site.x, site.B, H, W, static_cast<long long>(site.c_count) * H * W, static_cast<long long>(H) * W, W, 0, site.c_count,
-                      site.accum, nullptr, nullptr, nullptr};
+                      site.accum, nullptr, nullptr, nullptr, dtype};
             c.first = dense_first(c);
             const Route r = auto_route(c);
-            if (!multi_site(r)) { single.push_back(i); continue; }
+            if (!multi_site(r) || (dtype != DCTP_DTYPE_F32 && !reads_16bit(r))) { single.push_back(i); continue; }
             batched = r;                                     // (the same for every dense site of the shape)
             batch[nb++] = SiteDesc{c.first, site.B, site.c_count, site.accum};
             if (nb == SCORE_MAX_SEG) {
-                if ((rc = launch_sites(r, batch, nb, H, nullptr, nullptr, s))) return rc;
+                if ((rc = launch_sites(r, batch, nb, H, nullptr, nullptr, dtype, s))) return rc;
                 nb = 0;
             }
         }
-        if (nb > 0 && (rc = launch_sites(batched, batch, nb, H, nullptr, nullptr, s))) return rc;
+        if (nb > 0 && (rc = launch_sites(batched, batch, nb, H, nullptr, nullptr, dtype, s))) return rc;
     }
     for (int i : single) {
-        const int rc = dctp_score_accum(sites[i].x, sites[i].B, H, W, static_cast<long long>(sites[i].c_count) * H * W, static_cast<long long>(H) * W, W, 0,
-                                        sites[i].c_count, sites[i].accum, nullptr, nullptr, DCTP_PATH_AUTO, stream);
+        const int rc = dctp_score_accum_ex(sites[i].x, dtype, sites[i].B, H, W, static_cast<long long>(sites[i].c_count) * H * W,
+                                           static_cast<long long>(H) * W, W, 0, sites[i].c_count, sites[i].accum, nullptr, nullptr, DCTP_PATH_AUTO,
+                                           stream);
         if (rc) return rc;
     }
     return DCTP_OK;
+}
+
+int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, void* stream) {
+    return dctp_score_accum_multi_ex(sites, n_sites, H, W, DCTP_DTYPE_F32, stream);
 }
 
 // ------------------------------------------------------------------ alternative scoring ops (SURVEY §8f-3)

@@ -20,6 +20,9 @@
 // EVEN sides: 2-D tensor map over [n_maps, N^2] whose box is a few floats wider than a row (the excess is out of bounds and
 // arrives as zeros), so that a thread's 128-bit reads of its own row are free of bank conflicts.  ODD sides: rows are not
 // 16-byte multiples; the stream is viewed as [rows, 32 floats] (as in score_stack.cuh) and read with 32-bit loads (odd stride).
+// 16-bit input (IN, score_stack.cuh): the row layout (EVEN) needs a row pitch of whole 16-byte units, which 16-bit maps have at sides
+// 4 and 8 only (box width padded to an odd number of 16-byte units); every other side uses the flat [rows, 32 elements] view.  bf16
+// maps are their own hi part: A_lo is not written and the MMA issuer runs the hi*hi and hi*lo passes only; fp16 is split as fp32.
 #pragma once
 #include <cuda.h>
 #include "score_stack.cuh"
@@ -30,7 +33,7 @@ struct KronArgs {
     ScoreSegments seg;              // the activations of the launch (score_stack.cuh)
     int N, NN;
     int sub_tiles;                  // 128-map sub-tiles per TMA tile (1, 2 or 4)
-    int row_floats;                 // shared-memory stride of a map's row in floats (EVEN: box width, ODD: NN)
+    int row_elems;                  // shared-memory stride of a map's row in elements (EVEN: box width, ODD: NN)
     int tile_maps, num_tiles;
     uint32_t tile_bytes;            // bytes one TMA tile lands
     int box_rows;                   // second box dimension (EVEN: maps per tile, ODD: 128-byte rows per tile)
@@ -52,7 +55,7 @@ struct KronSmem {
 
 constexpr int KRON_NT = 576, KRON_W_PROD = 16, KRON_W_MMA = 17;
 
-template <int K2, bool EVEN>
+template <int K2, bool EVEN, int IN = IN_F32>
 __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_constant__ ScoreTensorMaps tmaps, const __grid_constant__ KronArgs a) {
     using S = KronSmem;
     using namespace umma;
@@ -141,11 +144,13 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
                     tc_fence_after_sync();
                     const uint32_t ahi = tmem + TM_A + sl * 64, alo = ahi + K2 / 2, d = tmem + TM_D + sl * 64;
 #pragma unroll
-                    for (int pass = 0; pass < 3; ++pass)
+                    for (int pass = 0; pass < 3; ++pass) {
+                        if (IN == IN_BF16 && pass == 1) continue;                // bf16 input: A_lo = 0
 #pragma unroll
                         for (int ks = 0; ks < KS; ++ks)
                             mma_bf16_ts(d, (pass == 1 ? alo : ahi) + 8 * ks, desc_with_lo(desc, (pass == 2 ? lo_lo : lo_hi) + ks * STEP), a.idesc,
                                         (pass | ks) != 0);
+                    }
                     mma_commit(d_full + sl);
                     mma_commit(a_free + sl);
                 }
@@ -170,15 +175,80 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
                 const uint32_t sl = j & 3u;
                 if (j >= 4) KRON_WAIT(a_free + sl, ((j >> 2) - 1u) & 1u);
                 tc_fence_after_sync();
+                const uint32_t ahi = tmem + TM_A + sl * 64 + lane_bits, alo = ahi + K2 / 2;
+                if constexpr (IN == IN_BF16) {
+                    // the map's raw bf16 pairs are A_hi as they are
+                    uint32_t p[K2 / 2];
+                    const long long m0 = static_cast<long long>(tile - a.seg.tile0[sg]) * a.tile_maps + st * 128 + gt;
+                    if (from_global) {
+                        const long long e0 = m0 * a.NN, total = a.seg.total_elems[sg];
+                        const uint16_t* xs = static_cast<const uint16_t*>(a.seg.x[sg]);
+#pragma unroll
+                        for (int i = 0; i < K2 / 2; ++i) {
+                            const uint32_t x0 = (2 * i < a.NN && e0 + 2 * i < total) ? xs[e0 + 2 * i] : 0u;
+                            const uint32_t x1 = (2 * i + 1 < a.NN && e0 + 2 * i + 1 < total) ? xs[e0 + 2 * i + 1] : 0u;
+                            p[i] = x0 | (x1 << 16);
+                        }
+                    } else if constexpr (EVEN) {
+                        const uint4* row = reinterpret_cast<const uint4*>(stg + s * S::STG_STRIDE) + static_cast<uint32_t>(st * 128 + gt) * (a.row_elems >> 3);
+#pragma unroll
+                        for (int i = 0; i < K2 / 8; ++i) {
+                            const uint4 q4 = 8 * i < a.NN ? row[i] : make_uint4(0u, 0u, 0u, 0u);
+                            p[4 * i] = q4.x; p[4 * i + 1] = q4.y; p[4 * i + 2] = q4.z; p[4 * i + 3] = q4.w;
+                        }
+                    } else {
+                        const uint16_t* row = reinterpret_cast<const uint16_t*>(stg + s * S::STG_STRIDE) + static_cast<uint32_t>(st * 128 + gt) * a.NN;
+#pragma unroll
+                        for (int i = 0; i < K2 / 2; ++i)
+                            p[i] = (2 * i < a.NN ? static_cast<uint32_t>(row[2 * i]) : 0u) | ((2 * i + 1 < a.NN ? static_cast<uint32_t>(row[2 * i + 1]) : 0u) << 16);
+                    }
+#pragma unroll
+                    for (int c = 0; c < K2 / 2; c += 16) {
+                        uint32_t h[16];
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) h[i] = c + i < K2 / 2 ? p[c + i] : 0u;
+                        if (c + 16 <= K2 / 2) tmem_st16(ahi + c, h);
+                        else tmem_st8(ahi + c, h);
+                    }
+                    tmem_st_wait();
+                    tc_fence_before_sync();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(a_full + sl);
+                    continue;
+                }
                 float v[K2];
-                if (from_global) {
+                if constexpr (IN == IN_F16) {                            // widened in registers, split as fp32
+                    if (from_global) {
+                        const long long e0 = (static_cast<long long>(tile - a.seg.tile0[sg]) * a.tile_maps + st * 128 + gt) * a.NN;
+                        const long long total = a.seg.total_elems[sg];
+                        const uint16_t* xs = static_cast<const uint16_t*>(a.seg.x[sg]);
+#pragma unroll
+                        for (int i = 0; i < K2; ++i) v[i] = (i < a.NN && e0 + i < total) ? in16_to_float<IN_F16>(xs, e0 + i) : 0.f;
+                    } else if constexpr (EVEN) {
+                        const uint4* row = reinterpret_cast<const uint4*>(stg + s * S::STG_STRIDE) + static_cast<uint32_t>(st * 128 + gt) * (a.row_elems >> 3);
+#pragma unroll
+                        for (int i = 0; i < K2 / 8; ++i) {
+                            const uint4 q4 = 8 * i < a.NN ? row[i] : make_uint4(0u, 0u, 0u, 0u);
+                            const uint32_t w[4] = {q4.x, q4.y, q4.z, q4.w};
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) {
+                                const float2 f = f16x2_to_float2(w[k]);
+                                v[8 * i + 2 * k] = f.x; v[8 * i + 2 * k + 1] = f.y;
+                            }
+                        }
+                    } else {
+                        const uint16_t* row = reinterpret_cast<const uint16_t*>(stg + s * S::STG_STRIDE) + static_cast<uint32_t>(st * 128 + gt) * a.NN;
+#pragma unroll
+                        for (int i = 0; i < K2; ++i) v[i] = i < a.NN ? in16_to_float<IN_F16>(row, i) : 0.f;
+                    }
+                } else if (from_global) {
                     const long long e0 = (static_cast<long long>(tile - a.seg.tile0[sg]) * a.tile_maps + st * 128 + gt) * a.NN;
                     const long long total = a.seg.total_elems[sg];
-                    const float* xs = a.seg.x[sg];
+                    const float* xs = static_cast<const float*>(a.seg.x[sg]);
 #pragma unroll
                     for (int i = 0; i < K2; ++i) v[i] = (i < a.NN && e0 + i < total) ? xs[e0 + i] : 0.f;
                 } else if constexpr (EVEN) {
-                    const float4* row = reinterpret_cast<const float4*>(stg + s * S::STG_STRIDE) + static_cast<uint32_t>(st * 128 + gt) * (a.row_floats >> 2);
+                    const float4* row = reinterpret_cast<const float4*>(stg + s * S::STG_STRIDE) + static_cast<uint32_t>(st * 128 + gt) * (a.row_elems >> 2);
 #pragma unroll
                     for (int i = 0; i < K2 / 4; ++i) {
                         const float4 q4 = 4 * i < a.NN ? row[i] : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -189,7 +259,6 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
 #pragma unroll
                     for (int i = 0; i < K2; ++i) v[i] = i < a.NN ? row[i] : 0.f;
                 }
-                const uint32_t ahi = tmem + TM_A + sl * 64 + lane_bits, alo = ahi + K2 / 2;
 #pragma unroll
                 for (int c = 0; c < K2 / 2; c += 16) {                   // 16 packed columns (32 contraction values) per store
                     uint32_t h[16], l[16];

@@ -36,11 +36,55 @@
 //   issuers     2 warps (one thread each): stage 1 and stage 2 have their own issuing thread, so that neither the waits nor
 //               the ~25 cycles it takes to issue an MMA of one stage hold up the other
 // TMEM (512 columns): A 32 | D1 2 x 128 | A2 2 x 64 | D2 NB2 x 64 (NB2 = 1: 480 columns in use).
+//
+// 16-bit input (IN = IN_BF16 / IN_F16, an autocast forward's activations): the tensor map views the stream as [rows, 32 elements]
+// (64-byte rows: tile_rows and the tail rule stay those of fp32 - a tile of 2 x 22 x 22 or 8 x 18 x 18 maps is not a whole number of
+// 128-byte rows of 16-bit elements), and a converter thread reads 4 elements (8 bytes) per table entry, so the offset table and the
+// Bx layout are the fp32 ones.  A bf16 value is its own bf16 hi part: the converters store it into Bx_hi unchanged and stage 1 issues
+// the Bx_hi pass only (the Bx_lo pass would add exact zeros).  fp16 (11 significant bits) splits exactly into a bf16 hi / lo pair: it
+// is widened in registers and runs the fp32 split.
 #pragma once
 #include <cuda.h>
+#include <cuda_fp16.h>
+#include <type_traits>
 #include "score_umma.cuh"
 
 namespace dctp {
+
+// element type of the activation a score kernel reads (the values of DCTP_DTYPE_* in include/dctp.h)
+constexpr int IN_F32 = 0, IN_BF16 = 1, IN_F16 = 2;
+__host__ __device__ constexpr int in_bytes(int in) { return in == IN_F32 ? 4 : 2; }
+
+// element i of a 16-bit stream as fp32 (exact)
+template <int IN>
+__device__ __forceinline__ float in16_to_float(const uint16_t* x, long long i) {
+    if constexpr (IN == IN_BF16) return __uint_as_float(static_cast<uint32_t>(x[i]) << 16);
+    else return __half2float(__ushort_as_half(x[i]));
+}
+// two packed fp16 values (the first in the low half) as fp32
+__device__ __forceinline__ float2 f16x2_to_float2(uint32_t p) {
+    __half2 h;
+    memcpy(&h, &p, 4);
+    return __half22float2(h);
+}
+
+// detail::map_energy64 of map m of a dense stream of element type IN (x: the stream's first element)
+template <int IN>
+__device__ __forceinline__ double map_energy64_in(const void* x, long long m, int NN, int N) {
+    if constexpr (IN == IN_F32) {
+        return detail::map_energy64(static_cast<const float*>(x) + m * NN, N);
+    } else {
+        const uint16_t* p = static_cast<const uint16_t*>(x) + m * NN;
+        double s = 0.0;
+#pragma unroll 1
+        for (int i = 0; i < N * N; ++i) {
+            const double e = in16_to_float<IN>(p, i);
+            if (!isfinite(e)) return __longlong_as_double(0x7FF8000000000000ll);
+            s = fma(e, e, s);
+        }
+        return s;
+    }
+}
 
 constexpr int SCORE_MAX_SEG = 16;   // activations (hook sites of the same map side) one launch can score
 
@@ -51,7 +95,7 @@ struct ScoreSegments {
     int tile0[SCORE_MAX_SEG + 1];
     int n_maps[SCORE_MAX_SEG], c_count[SCORE_MAX_SEG];
     long long total_elems[SCORE_MAX_SEG];                // n_maps * NN
-    const float* x[SCORE_MAX_SEG];                       // first scored element, 16-B aligned
+    const void* x[SCORE_MAX_SEG];                        // first scored element (of the kernel's IN type), 16-B aligned
     double* accum[SCORE_MAX_SEG];                        // fp64 [c_count] of the site
 };
 struct ScoreTensorMaps { CUtensorMap m[SCORE_MAX_SEG]; };
@@ -107,7 +151,8 @@ constexpr int stack_warps(int nconv) { return nconv + 8 * STACK_NE1G + 4 * STACK
 // NP8: Np / 8 as a compile-time constant - epilogue 1's column loops lose their branches.
 // TRACE: the debug instantiation - the cycle accounting of DCTP_S_TRACE, the per-map energies (energy_out) and the coefficient dump
 // (coeff_out); the production instantiations carry none of that code (the host routes launches that ask for any of it here).
-template <int KP, int VEC, int NCONV, int NP8, bool TRACE>
+// IN: element type of the activation (IN_F32, IN_BF16, IN_F16; see the head of this file).
+template <int KP, int VEC, int NCONV, int NP8, bool TRACE, int IN = IN_F32>
 __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel(const __grid_constant__ ScoreTensorMaps tmaps, const __grid_constant__ StackArgs a) {
     using S = StackSmem;
     using namespace umma;
@@ -235,7 +280,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         a.trace[53] = tr_g0 - tr_entry;                                   // TMEM + barriers + bases staged + the preceding kernel complete
     }
     const int first = blockIdx.x, stride = gridDim.x;
-    const uint32_t tile_bytes = static_cast<uint32_t>(a.tile_rows) * 128u;
+    const uint32_t tile_bytes = static_cast<uint32_t>(a.tile_rows) * (32u * in_bytes(IN));      // rows of 32 elements
     bool dead = false;
     // segment of a tile: the roles walk the tiles in increasing order, so each keeps a cursor.  A segment whose stream does not
     // end on a 128-byte row has its last tile converted straight from global memory (that row is not in the tensor map).
@@ -275,6 +320,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         __syncwarp();
     } else if (warp == W_MMA) {
         // ================================================================ MMA issuer, stage 1: D1 = A * Bx^T (Bx_hi, then Bx_lo)
+        constexpr int P1 = IN == IN_BF16 ? 1 : 2;                          // bf16 input: X_lo = 0, the Bx_lo pass is not issued
         if (elect_one()) {
             tr_me = tr_on;
             const uint64_t desc = make_smem_desc(0, a.lbo1, 128, SWIZZLE_NONE);
@@ -291,7 +337,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                 const uint32_t lo_hi = static_cast<uint32_t>(desc) + (smem_u32(bx + bb * 2 * S::BX_HALF) >> 4);
                 const uint32_t lo_lo = lo_hi + (S::BX_HALF >> 4);
 #pragma unroll
-                for (int pass = 0; pass < 2; ++pass)
+                for (int pass = 0; pass < P1; ++pass)
 #pragma unroll
                     for (int ks = 0; ks < K1S; ++ks)
                         mma_bf16_ts(d1, tmem + TM_A + 8 * ks, desc_with_lo(desc, (pass ? lo_lo : lo_hi) + ks * STEP1), a.idesc1,
@@ -382,26 +428,45 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                     *reinterpret_cast<uint32_t*>(lo + o1) = l1;
                 }
             };
+            // 16-bit input, 4 elements (8 bytes) per table entry: bf16 goes into Bx_hi as it is, fp16 is widened and split as fp32
+            auto emit16 = [&](uint32_t o, const uint2 r) {
+                if constexpr (IN == IN_BF16) {
+                    if constexpr (VEC == 4) {
+                        *reinterpret_cast<uint2*>(hi + o) = r;
+                    } else {
+                        *reinterpret_cast<uint32_t*>(hi + (o & 0xFFFFu)) = r.x;
+                        *reinterpret_cast<uint32_t*>(hi + (o >> 16)) = r.y;
+                    }
+                } else {
+                    const float2 p = f16x2_to_float2(r.x), q = f16x2_to_float2(r.y);
+                    emit(o, make_float4(p.x, p.y, q.x, q.y));
+                }
+            };
+            using Vec = std::conditional_t<IN == IN_F32, float4, uint2>;
+            auto put = [&](uint32_t o, const Vec& v) {
+                if constexpr (IN == IN_F32) emit(o, v);
+                else emit16(o, v);
+            };
             auto entry = [&](int f) {
                 return VEC == 4 ? static_cast<uint32_t>(reinterpret_cast<const uint16_t*>(tab)[f]) : reinterpret_cast<const uint32_t*>(tab)[f];
             };
             if (!tail) {
-                const float4* src = reinterpret_cast<const float4*>(stg + s * S::STG_STRIDE);
+                const Vec* src = reinterpret_cast<const Vec*>(stg + s * S::STG_STRIDE);
                 // CB vectors (and their table entries) are loaded before the first store: the stores go to shared memory
                 // too, so the compiler cannot hoist a later iteration's loads above them by itself
                 // (full rounds run without predicates in one basic block, so that the compiler interleaves the three vectors)
                 constexpr int CB = 3;
                 int f0 = ctid;
                 for (; f0 + (int)NCT * (CB - 1) < a.tile_vec - (a.tile_vec % (int)NCT) ; f0 += NCT * CB) {
-                    float4 v[CB];
+                    Vec v[CB];
                     uint32_t o[CB];
 #pragma unroll
                     for (int i = 0; i < CB; ++i) { v[i] = src[f0 + (int)NCT * i]; o[i] = entry(f0 + (int)NCT * i); }
 #pragma unroll
-                    for (int i = 0; i < CB; ++i) emit(o[i], v[i]);
+                    for (int i = 0; i < CB; ++i) put(o[i], v[i]);
                 }
                 {
-                    float4 v[CB];
+                    Vec v[CB];
                     uint32_t o[CB];
 #pragma unroll
                     for (int i = 0; i < CB; ++i) {
@@ -410,7 +475,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                     }
 #pragma unroll
                     for (int i = 0; i < CB; ++i)
-                        if (f0 + (int)NCT * i < a.tile_vec) emit(o[i], v[i]);
+                        if (f0 + (int)NCT * i < a.tile_vec) put(o[i], v[i]);
                 }
                 TR_ADD(tr2);
                 __syncwarp();
@@ -418,15 +483,26 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                 ++it;
             } else {                                                      // the stream's last, partial 128-byte row is not in the tensor map
                 const long long e0 = static_cast<long long>(tile - a.seg.tile0[sg]) * a.tile_elems, total = a.seg.total_elems[sg];
-                const float* xs = a.seg.x[sg];
-                for (int f = ctid; f < a.tile_vec; f += NCT) {
-                    const long long e = e0 + 4ll * f;
-                    float4 v;
-                    v.x = e + 0 < total ? xs[e + 0] : 0.f;
-                    v.y = e + 1 < total ? xs[e + 1] : 0.f;
-                    v.z = e + 2 < total ? xs[e + 2] : 0.f;
-                    v.w = e + 3 < total ? xs[e + 3] : 0.f;
-                    emit(entry(f), v);
+                if constexpr (IN == IN_F32) {
+                    const float* xs = static_cast<const float*>(a.seg.x[sg]);
+                    for (int f = ctid; f < a.tile_vec; f += NCT) {
+                        const long long e = e0 + 4ll * f;
+                        float4 v;
+                        v.x = e + 0 < total ? xs[e + 0] : 0.f;
+                        v.y = e + 1 < total ? xs[e + 1] : 0.f;
+                        v.z = e + 2 < total ? xs[e + 2] : 0.f;
+                        v.w = e + 3 < total ? xs[e + 3] : 0.f;
+                        emit(entry(f), v);
+                    }
+                } else {
+                    const uint16_t* xs = static_cast<const uint16_t*>(a.seg.x[sg]);
+                    for (int f = ctid; f < a.tile_vec; f += NCT) {
+                        const long long e = e0 + 4ll * f;
+                        uint32_t p[4];
+#pragma unroll
+                        for (int k = 0; k < 4; ++k) p[k] = e + k < total ? xs[e + k] : 0u;        // (0x0000 is +0 in bf16 and fp16)
+                        emit16(entry(f), make_uint2(p[0] | (p[1] << 16), p[2] | (p[3] << 16)));
+                    }
                 }
             }
             fence_async_smem();
@@ -625,7 +701,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                         // others 0.  (With J = 1 the maps of a tile never meet in one contraction.)
                         double share = mine;
                         if (J > 1 && !isfinite(mine))
-                            share = my_v0 == 0 ? detail::map_energy64(a.seg.x[sg] + static_cast<long long>(m0 + ml) * a.NN, a.N) : 0.0;
+                            share = my_v0 == 0 ? map_energy64_in<IN>(a.seg.x[sg], static_cast<long long>(m0 + ml), a.NN, a.N) : 0.0;
                         atomicAdd(accum + ch, share);
                     }
                 }
@@ -648,7 +724,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                         while (ch >= C) ch -= C;
                         double e = en;
                         if (!isfinite(en)) {                       // a non-finite map in the tile (rare: see map_energy64)
-                            e = detail::map_energy64(a.seg.x[sg] + static_cast<long long>(m) * a.NN, a.N);
+                            e = map_energy64_in<IN>(a.seg.x[sg], static_cast<long long>(m), a.NN, a.N);
                             en = static_cast<float>(e);
                         }
                         atomicAdd(accum + ch, e);

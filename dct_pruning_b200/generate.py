@@ -92,10 +92,17 @@ def device_batches(host_batches, device):
         yield bufs[slot]
 
 
-def inference(net, loader, limit, device, rank=0, world=1):
+# --amp: the forward's autocast dtype.  The hooks then score the reduced-precision activations the forward produced (bf16 / fp16
+# maps are read by the library as they are); those scores are not the reference's, whose forward runs in fp32.
+AMP_DTYPES = {'off': None, 'bf16': torch.bfloat16, 'fp16': torch.float16}
+
+
+def inference(net, loader, limit, device, rank=0, world=1, amp='off'):
     """eval + no_grad forward over the first `limit` batches (common.py:312-320); under
-    world > 1 each rank forwards its contiguous slice of every batch."""
+    world > 1 each rank forwards its contiguous slice of every batch.  amp: 'off', or 'bf16' / 'fp16' to run the
+    forward under torch.autocast with that dtype."""
     net.eval()
+    amp_dtype = AMP_DTYPES[amp]
 
     def shards():
         for batch_idx, sample in enumerate(loader):
@@ -109,7 +116,7 @@ def inference(net, loader, limit, device, rank=0, world=1):
                 yield x
 
     n = 0
-    with torch.no_grad():
+    with torch.no_grad(), torch.autocast(torch.device(device).type, dtype=amp_dtype, enabled=amp_dtype is not None):
         if torch.device(device).type == 'cuda':
             for x in device_batches(shards(), device):
                 n += x.shape[0]
@@ -141,7 +148,7 @@ def score_session(net, args, loader=None, path='auto', op=None):
         side0 = getattr(args, 'input_side', None) or side0
         session.plan_layout(torch.zeros(1, 3, side0, side0, device=device))
     with session:
-        inference(net, loader, args.limit, device, rank=rank, world=world)
+        inference(net, loader, args.limit, device, rank=rank, world=world, amp=getattr(args, 'amp', None) or 'off')
     return session
 
 

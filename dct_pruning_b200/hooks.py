@@ -8,8 +8,9 @@ Replaces the three hook functions and their module-global accumulators in
     get_feature_hook_u2net_input  :296-309   'I'  all channels of input[0]
     feature_result / total        :258-259   ->   one flat fp64 device accumulator per session
 
-Each hook call is one asynchronous `dctp_score_accum` launch on the current torch stream:
-the activation is read once where cuDNN left it (NCHW fp32, any batch/channel stride), no
+Each hook call is one asynchronous `dctp_score_accum(_ex)` launch on the current torch stream:
+the activation is read once where cuDNN left it (NCHW fp32, or bf16 / fp16 under torch.autocast,
+any batch/channel stride), no
 coefficient tensor or per-slice value ever reaches host memory, and nothing synchronises
 until `finalize()`.  The reference runs one forward sweep per site; registering all sites
 together gives the same numbers on fixed inputs with one forward per batch.
@@ -71,17 +72,18 @@ class ScoreSession:
         self.handles = []
         self.lib = _lib.load()
         self._score_accum = self.lib.dctp_score_accum
+        self._score_accum_ex = self.lib.dctp_score_accum_ex     # 16-bit activations (dtype after the pointer)
         self._score_op = self.lib.dctp_score_op
         self._plans = [None] * len(self.sites)
         self._planned = False                 # plan_layout() ran: slots exist for every site, in site order
         self.defer_bytes = self.DEFER_BYTES if defer_bytes is None else int(defer_bytes)
-        self._pending = {}                    # (H, W, device index, stream) -> [(tensor kept alive, address of its first scored map,
+        self._pending = {}                    # (H, W, device index, stream, dtype) -> [(tensor kept alive, address of its first scored map,
         self._held = 0                        #                                   B, c_count, accumulator address)]; bytes held
-        self._score_multi = self.lib.dctp_score_accum_multi
+        self._score_multi = self.lib.dctp_score_accum_multi_ex
         self.launches = 0
         # The forward pass of the CIFAR nets is bound by the host (~20 us per module call), so what a hook costs the host is what it costs
         # end to end.  After a site's first firing everything that depends only on the activation's geometry is remembered here:
-        # (shape, strides, device index, map bytes, byte offset of the first scored map, B, c_count, accumulator address, H, W)
+        # (shape, strides, device index, map bytes, byte offset of the first scored map, B, c_count, accumulator address, H, W, dtype)
         self._fast = [None] * len(self.sites)
         self._site_buf = bytearray(_SITE.size * self.MAX_PENDING)
         self._site_arr = (ctypes_char_array(self.MAX_PENDING)).from_buffer(self._site_buf)
@@ -125,12 +127,12 @@ class ScoreSession:
     # ------------------------------------------------------------------ one hook firing
     def score(self, idx, t):
         fast = self._fast[idx]
-        if (fast is not None and t.shape == fast[0] and t.stride() == fast[1] and t.dtype is torch.float32 and t.is_cuda
+        if (fast is not None and t.shape == fast[0] and t.stride() == fast[1] and t.dtype is fast[10] and t.is_cuda
                 and fast[3] < self.defer_bytes):
             first = t.data_ptr() + fast[4]
             if first % 16 == 0 and t.device.index == fast[2]:
                 B = fast[5]
-                key = (fast[8], fast[9], fast[2], _raw_stream(fast[2]))
+                key = (fast[8], fast[9], fast[2], _raw_stream(fast[2]), fast[11])
                 group = self._pending.get(key)
                 if group is None:
                     group = self._pending[key] = []
@@ -147,8 +149,10 @@ class ScoreSession:
                                % (self.sites[idx].module, t.device))
         if t.dim() != 4:
             raise ValueError('site %r: expected an NCHW activation, got shape %s' % (self.sites[idx].module, tuple(t.shape)))
-        if t.dtype != torch.float32:
-            t = t.float()                     # the reference scores in fp32 (common.py:233,289)
+        dtype = _lib.dtype_code(t.dtype)
+        if dtype is None or (dtype != _lib.DTYPE_F32 and self.op != 'dct2'):
+            t = t.float()                     # the reference scores in fp32 (common.py:233,289); the DCT energy reads 16-bit maps itself
+            dtype = _lib.DTYPE_F32
         sb, sc, sh, sw = t.stride()
         B, C, H, W = t.shape
         if sw != 1 or sh < W:
@@ -176,13 +180,15 @@ class ScoreSession:
             self.launches += 1
             return
         dense = sh == W and sc == H * W and (B == 1 or (c_count == C and sb == C * H * W))
-        if (self.defer_bytes and dense and H == W and self.path == _lib.PATH_AUTO and 4 * B * c_count * H * W < self.defer_bytes
-                and (t.data_ptr() + 4 * c_begin * sc) % 16 == 0):
-            key = (H, W, t.device.index, stream)
+        es = t.element_size()
+        if (self.defer_bytes and dense and H == W and self.path == _lib.PATH_AUTO and es * B * c_count * H * W < self.defer_bytes
+                and (t.data_ptr() + es * c_begin * sc) % 16 == 0):
+            key = (H, W, t.device.index, stream, dtype)
             group = self._pending.setdefault(key, [])
-            group.append((t, t.data_ptr() + 4 * c_begin * sc, B, c_count, plan[3]))
-            self._held += 4 * B * c_count * H * W
-            self._fast[idx] = (t.shape, t.stride(), t.device.index, 4 * B * c_count * H * W, 4 * c_begin * sc, B, c_count, plan[3], H, W)
+            group.append((t, t.data_ptr() + es * c_begin * sc, B, c_count, plan[3]))
+            self._held += es * B * c_count * H * W
+            self._fast[idx] = (t.shape, t.stride(), t.device.index, es * B * c_count * H * W, es * c_begin * sc, B, c_count, plan[3], H, W,
+                               t.dtype, dtype)
             if len(group) >= self.MAX_PENDING:
                 self.flush(key)
             elif self._held > self.HELD_BYTES:
@@ -191,11 +197,12 @@ class ScoreSession:
             return
         # launch on the activation's own device and on that device's current stream (the hook may fire while another
         # device is current); the library refuses a device other than the one it was initialised on
+        args = (B, H, W, sb, sc, sh, plan[1], plan[2], plan[3], None, None, self.path, stream)
         if t.device.index != torch.cuda.current_device():
             with torch.cuda.device(t.device):
-                code = self._score_accum(t.data_ptr(), B, H, W, sb, sc, sh, plan[1], plan[2], plan[3], None, None, self.path, stream)
+                code = self._score_accum(t.data_ptr(), *args) if dtype == _lib.DTYPE_F32 else self._score_accum_ex(t.data_ptr(), dtype, *args)
         else:
-            code = self._score_accum(t.data_ptr(), B, H, W, sb, sc, sh, plan[1], plan[2], plan[3], None, None, self.path, stream)
+            code = self._score_accum(t.data_ptr(), *args) if dtype == _lib.DTYPE_F32 else self._score_accum_ex(t.data_ptr(), dtype, *args)
         if code:
             _lib.check(code)
         self.images[idx] += B
@@ -208,8 +215,8 @@ class ScoreSession:
             pending = self._pending.pop(k, None)
             if not pending:
                 continue
-            H, W, dev_index, stream = k
-            buf, off, map_bytes = self._site_buf, 0, 4 * H * W
+            H, W, dev_index, stream, dtype = k
+            buf, off, map_bytes = self._site_buf, 0, (4 if dtype == _lib.DTYPE_F32 else 2) * H * W
             for _, x_ptr, B, c_count, acc_ptr in pending:             # dctp_site records packed in place (ctypes field stores are slow)
                 _SITE.pack_into(buf, off, x_ptr, acc_ptr, B, c_count)
                 off += _SITE.size
@@ -217,9 +224,9 @@ class ScoreSession:
             sites = self._site_arr
             if dev_index != torch.cuda.current_device():
                 with torch.cuda.device(dev_index):
-                    code = self._score_multi(sites, len(pending), H, W, stream)
+                    code = self._score_multi(sites, len(pending), H, W, dtype, stream)
             else:
-                code = self._score_multi(sites, len(pending), H, W, stream)
+                code = self._score_multi(sites, len(pending), H, W, dtype, stream)
             if code:
                 _lib.check(code)
             self.launches += 1

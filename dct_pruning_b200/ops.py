@@ -8,12 +8,14 @@ def dct_energy(x, c_begin=0, c_count=None, path='auto', accum=None, want_energy=
     """Per-channel sum over the batch of the orthonormal 2-D DCT-II energy of x[b, c] (what
     get_feature_hook computes before its running mean, /root/reference/utils/common.py:262-274).
 
-    x: CUDA fp32 [B, C, H, W], innermost stride 1.  Returns (accum fp64 [c_count],
-    energies fp32 [B, c_count] or None, coefficients fp32 [B, c_count, H, W] or None)."""
+    x: CUDA fp32, bf16 or fp16 [B, C, H, W] (16-bit: an autocast forward's activations; the energies are those of the values x
+    holds, computed as for fp32).  Returns (accum fp64 [c_count], energies fp32 [B, c_count] or None, coefficients fp32
+    [B, c_count, H, W] or None)."""
     if not x.is_cuda:
         raise RuntimeError('dct_energy runs on CUDA only; there is no CPU fallback')
-    if x.dtype != torch.float32 or x.dim() != 4:
-        raise ValueError('expected an fp32 NCHW tensor')
+    dtype = _lib.dtype_code(x.dtype)
+    if dtype is None or x.dim() != 4:
+        raise ValueError('expected an fp32, bf16 or fp16 NCHW tensor')
     if x.stride(3) != 1 or x.stride(2) < x.shape[3]:
         x = x.contiguous()
     lib = _lib.load()
@@ -28,8 +30,8 @@ def dct_energy(x, c_begin=0, c_count=None, path='auto', accum=None, want_energy=
         energy = torch.empty(B, c_count, dtype=torch.float32, device=x.device) if want_energy else None
         coeff = torch.empty(B, c_count, H, W, dtype=torch.float32, device=x.device) if want_coeff else None
         code = _lib.PATHS[path] if isinstance(path, str) else int(path)
-        _lib.check(lib.dctp_score_accum(_lib.ptr(x), B, H, W, x.stride(0), x.stride(1), x.stride(2), c_begin, c_count,
-                                        _lib.ptr(accum), _lib.ptr(energy), _lib.ptr(coeff), code, _lib.current_stream()))
+        _lib.check(lib.dctp_score_accum_ex(_lib.ptr(x), dtype, B, H, W, x.stride(0), x.stride(1), x.stride(2), c_begin, c_count,
+                                           _lib.ptr(accum), _lib.ptr(energy), _lib.ptr(coeff), code, _lib.current_stream()))
         if check:
             _lib.check(lib.dctp_check(_lib.current_stream()))
     return accum, energy, coeff

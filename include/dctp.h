@@ -91,6 +91,25 @@ int dctp_score_accum(const float* x, int B, int H, int W,
                      double* accum, float* energy_out, float* coeff_out,
                      int path, void* stream);
 
+/* Element type of an activation (dctp_score_accum_ex, dctp_score_accum_multi_ex). */
+#define DCTP_DTYPE_F32   0
+#define DCTP_DTYPE_BF16  1        /* the activations of a forward pass under torch.autocast(dtype=torch.bfloat16) */
+#define DCTP_DTYPE_F16   2        /* ... under torch.autocast(dtype=torch.float16) */
+
+/* dctp_score_accum for an activation x of element type `dtype` (DCTP_DTYPE_*; anything else: DCTP_E_INVALID).  Every shape, layout
+ * and path dctp_score_accum takes is taken, with the same results for the values x holds: the energies are those of the maps widened
+ * to fp32 (exactly), and the non-finite rules above hold unchanged.  accum, energy_out and coeff_out are fp64 / fp32 as there.
+ * dctp_score_accum(...) is dctp_score_accum_ex(x, DCTP_DTYPE_F32, ...).
+ * 16-bit maps that DCTP_PATH_KRON or DCTP_PATH_STACK take (AUTO's choice or forced) are read by those kernels directly: 2 bytes per
+ * element.  Every other 16-bit call widens its scored window into a dense fp32 copy, allocated and freed on `stream`
+ * (stream-ordered, graph-capturable: call dctp_prepare first, as for fp32), and scores that copy as dctp_score_accum would with the
+ * same path: one extra launch, and 2 + 4 + 4 bytes of traffic per element. */
+int dctp_score_accum_ex(const void* x, int dtype, int B, int H, int W,
+                        long long stride_b, long long stride_c, long long stride_h,
+                        int c_begin, int c_count,
+                        double* accum, float* energy_out, float* coeff_out,
+                        int path, void* stream);
+
 /* Several hook sites in ONE launch.  The forward pass of the CIFAR nets and of U^2-Netp's small stages fires tens of hooks on
  * activations of a few MB; scored one by one they are bound by the host's launch rate (~12 us per hook), not by the GPU.  The host
  * side may therefore hold on to a run of activations of the same map size and hand them over together
@@ -100,12 +119,15 @@ int dctp_score_accum(const float* x, int B, int H, int W,
  * kernels take (square; side <= 8, even side 10..64 - above 32 a multiple of 4 -, or side 80..320 a multiple of 16) are scored 16 sites per launch;
  * any other shape falls back to one launch per site.  Results are identical to n_sites dctp_score_accum calls. */
 typedef struct dctp_site {
-    const float* x;
+    const void* x;                /* first scored element, of the call's dtype (fp32 for dctp_score_accum_multi) */
     double* accum;
     int B;
     int c_count;
 } dctp_site;
 int dctp_score_accum_multi(const dctp_site* sites, int n_sites, int H, int W, void* stream);
+/* The same for sites of element type `dtype` (DCTP_DTYPE_*).  16-bit sites of the shapes the Kronecker and stacked-basis kernels take
+ * are scored 16 per launch as above; 16-bit sites of any other shape go through dctp_score_accum_ex one by one. */
+int dctp_score_accum_multi_ex(const dctp_site* sites, int n_sites, int H, int W, int dtype, void* stream);
 
 /* Alternative per-slice scoring ops behind the same accumulate / finalise / top-k plumbing: the two lines the reference keeps
  * commented out beside the DCT in get_feature_hook and compares against in chart*.py.
@@ -169,7 +191,8 @@ int dctp_path_for(int H, int W, long long stride_h);
 int dctp_occupancy(int kp, int mode);
 long long dctp_launch_count(void);
 /* Name of the kernel instantiation the most recent dctp_score_accum call launched (AUTO's choice made visible: bench.py labels
- * its per-kernel table with it instead of re-deriving the dispatch).  Static storage, valid until the next score call. */
+ * its per-kernel table with it instead of re-deriving the dispatch; 16-bit instantiations carry ",IN=bf16" / ",IN=f16").  Static
+ * storage, valid until the next score call. */
 const char* dctp_last_kernel(void);
 int dctp_sm_count(void);
 
