@@ -105,7 +105,7 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
     auto seg_of = [&](int tile, int& sg) {
         while (tile >= a.seg.tile0[sg + 1]) ++sg;
     };
-    auto is_tail = [&](int tile, int sg) {               // (ODD) a stream that does not end on a 128-byte row: last tile from global memory
+    auto is_tail = [&](int tile, int sg) {               // (ODD) a stream that does not end on a 32-element row: last tile from global memory
         return !EVEN && tile == a.seg.tile0[sg + 1] - 1 && (a.seg.total_elems[sg] & 31) != 0;
     };
 #define KRON_WAIT(bar, par)                          \

@@ -282,8 +282,8 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
     const int first = blockIdx.x, stride = gridDim.x;
     const uint32_t tile_bytes = static_cast<uint32_t>(a.tile_rows) * (32u * in_bytes(IN));      // rows of 32 elements
     bool dead = false;
-    // segment of a tile: the roles walk the tiles in increasing order, so each keeps a cursor.  A segment whose stream does not
-    // end on a 128-byte row has its last tile converted straight from global memory (that row is not in the tensor map).
+    // segment of a tile: the roles walk the tiles in increasing order, so each keeps a cursor.  A segment whose stream does not end
+    // on a 32-element row (128 bytes in fp32, 64 in 16-bit) has its last tile converted from global memory (that row is not in the tensor map).
     auto seg_of = [&](int tile, int& sg) {
         while (tile >= a.seg.tile0[sg + 1]) ++sg;
     };
@@ -481,7 +481,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                 __syncwarp();
                 if (lane == 0) mbar_arrive(stg_free + s);
                 ++it;
-            } else {                                                      // the stream's last, partial 128-byte row is not in the tensor map
+            } else {                                                      // the stream's last, partial 32-element row is not in the tensor map
                 const long long e0 = static_cast<long long>(tile - a.seg.tile0[sg]) * a.tile_elems, total = a.seg.total_elems[sg];
                 if constexpr (IN == IN_F32) {
                     const float* xs = static_cast<const float*>(a.seg.x[sg]);

@@ -18,7 +18,8 @@ for dead maps (all +0.0 or all -0.0).  NaN never sits inside the caller's tensor
 to the other channels is pinned by test_gpu_nonfinite.py.
 
 The module records which kernel instantiation every score launch ran (dctp_last_kernel); its last test checks that the cases
-reached each one in REQUIRED.
+reached each one in REQUIRED.  bf16 / fp16 input (dctp_score_accum_ex, dctp_score_accum_multi_ex) is held to the same rules by
+test_gpu_half_bounds.py, through the helpers here (Arena, maps, score, geometry, map_counts take a dtype).
 """
 import math
 
@@ -34,7 +35,8 @@ pytestmark = pytest.mark.gpu
 COEFF_TOL = 2e-5                     # coefficients vs scipy, relative to the largest coefficient (as in test_gpu_kernels.py)
 GUARD = 256 << 10                    # bytes on each side of every view, at the least
 NEG0 = 'neg0'                        # edge value: -0.0, written and compared as a bit pattern
-_INT = {torch.float32: (torch.int32, -2 ** 31), torch.float64: (torch.int64, -2 ** 63)}
+_INT = {torch.float32: (torch.int32, -2 ** 31), torch.float64: (torch.int64, -2 ** 63), torch.bfloat16: (torch.int16, -2 ** 15),
+        torch.float16: (torch.int16, -2 ** 15)}
 
 LARGE_SIDES = list(range(80, 321, 16))
 AUTO_ELSEWHERE = [9, 11, 13, 34, 50, 54, 62, 72, 100, 130]     # sides AUTO sends to neither the Kronecker nor the stacked-basis kernel
@@ -93,11 +95,11 @@ def note(lib):
     return name
 
 
-def maps(B, C, H, W, seed):
-    """relu(N(0, 1)) maps on the device.  Channels c % 7 == 1 are all +0.0 and c % 7 == 4 all -0.0 in every image (dead
-    channels); image 1 of channel 2 is a dead map of a live channel."""
+def maps(B, C, H, W, seed, dtype=torch.float32):
+    """relu(N(0, 1)) maps on the device, rounded to `dtype`.  Channels c % 7 == 1 are all +0.0 and c % 7 == 4 all -0.0 in every
+    image (dead channels); image 1 of channel 2 is a dead map of a live channel."""
     g = torch.Generator(device='cuda').manual_seed(seed)
-    x = torch.relu(torch.randn(B, C, H, W, generator=g, device='cuda'))
+    x = torch.relu(torch.randn(B, C, H, W, generator=g, device='cuda')).to(dtype)
     x[:, 1::7] = 0.0
     x[:, 4::7] = -0.0
     if B > 1 and C > 2:
@@ -111,31 +113,51 @@ def rel_err(got, want):
     return float(((got.double() - want).abs() / want.abs().clamp_min(1e-30)).max())
 
 
+SHARES = 8                           # fp64 adds one map makes into its channel's accumulator, at the most (score kernels: 1 to 5)
+
+
+def acc_err(acc, want, maps_per_channel):
+    """rel_err of acc - 0.5 against `want`, for accumulators that started at 0.5, less the rounding that start costs: the sum is
+    held at 0.5 and above, so each of the SHARES * maps_per_channel fp64 adds (and the subtraction of 0.5) may round by half an
+    ulp of the final value.  (That is 5.6e-17 absolute: more than ENERGY_TOL of a channel whose only live map is a value near 1e-6.)"""
+    if acc.numel() == 0:
+        return 0.0
+    got = acc.double()
+    ulp = torch.nextafter(got, torch.full_like(got, math.inf)) - got
+    diff = ((got - 0.5 - want).abs() - (SHARES * maps_per_channel + 1) * 0.5 * ulp).clamp_min(0)
+    return float((diff / want.abs().clamp_min(1e-30)).max())
+
+
 def score(lib, path, B, C, H, W, *, c_begin=0, c_count=None, batch_step=1, row=None, x_off=0, acc_off=0, debug=False, seed=0,
-          tol=ENERGY_TOL, what=''):
-    """dctp_score_accum on x[::batch_step, c_begin:c_begin + c_count, :, :W] of a NaN arena [B * batch_step, C, H, row], into guarded
-    outputs (energy_out and coeff_out when `debug`); checks every output and guard."""
+          tol=ENERGY_TOL, what='', dtype=torch.float32, out=None):
+    """dctp_score_accum (dctp_score_accum_ex for bf16 / fp16 `dtype`) on x[::batch_step, c_begin:c_begin + c_count, :, :W] of a NaN
+    arena [B * batch_step, C, H, row], into guarded outputs (energy_out and coeff_out when `debug`); checks every output and guard.
+    Returns the kernel that ran; `out` (a dict), when given, receives the scored maps and the live views of the outputs (src, acc,
+    en, co; None where not asked for)."""
     row = row or W
     cc = C - c_begin if c_count is None else c_count
     n = B * cc
     full = (B * batch_step, C, H, row)
     guard = max(GUARD, 4 * H * row * 4)
-    xa = Arena([math.prod(full)], torch.float32, [x_off], guard=guard)
+    xa = Arena([math.prod(full)], dtype, [x_off], guard=guard)
     x = xa.live.view(full)[::batch_step, :, :, :W]
-    src = maps(B, cc, H, W, seed)
+    src = maps(B, cc, H, W, seed, dtype)
     acc = Arena([cc], torch.float64, [acc_off], edge=NEG0, live=0.5)
     en = Arena([n], torch.float32, [4 * (seed % 2)], edge=NEG0, live=float('nan')) if debug else None
     co = Arena([n * H * W], torch.float32, [64], edge=NEG0, live=float('nan'), guard=guard) if debug else None
     _lib.check(lib.dctp_prepare(H, W))                       # (bases are uploaded synchronously on first use of a size)
     stream = _lib.current_stream()
     x[:, c_begin:c_begin + cc].copy_(src)                   # the launch below must wait for this copy
-    rc = lib.dctp_score_accum(_lib.ptr(x), B, H, W, x.stride(0), x.stride(1), x.stride(2), c_begin, cc, _lib.ptr(acc.live),
-                              _lib.ptr(en.live) if en else None, _lib.ptr(co.live) if co else None, _lib.PATHS[path], stream)
+    args = (B, H, W, x.stride(0), x.stride(1), x.stride(2), c_begin, cc, _lib.ptr(acc.live), _lib.ptr(en.live) if en else None,
+            _lib.ptr(co.live) if co else None, _lib.PATHS[path], stream)
+    code = _lib.dtype_code(dtype)
+    rc = lib.dctp_score_accum(_lib.ptr(x), *args) if code == _lib.DTYPE_F32 else lib.dctp_score_accum_ex(_lib.ptr(x), code, *args)
     _lib.check(rc)
     _lib.check(lib.dctp_check(stream))
     name = note(lib)
-    label = '%s %dx%dx%dx%d (window %d+%d, batch step %d, row %d, offset %d) %s: %s%s' % (
-        path, B, C, H, W, c_begin, cc, batch_step, row, x_off, what, name, ' [energy_out, coeff_out]' if debug else '')
+    label = '%s %s %dx%dx%dx%d (window %d+%d, batch step %d, row %d, offset %d) %s: %s%s' % (
+        path, str(dtype).split('.')[-1], B, C, H, W, c_begin, cc, batch_step, row, x_off, what, name,
+        ' [energy_out, coeff_out]' if debug else '')
 
     want = (src.double() ** 2).sum((2, 3))                  # [B, cc]
     chan = want.sum(0)
@@ -143,8 +165,10 @@ def score(lib, path, B, C, H, W, *, c_begin=0, c_count=None, batch_step=1, row=N
     assert acc.guards_intact(), 'accum guard written: ' + label
     assert not bool(torch.isnan(acc.live).any()), 'NaN in accum: ' + label
     assert bool((acc.live[~live] == 0.5).all()), 'a dead channel changed (it must read exactly 0.5): ' + label
-    err = rel_err(acc.live[live] - 0.5, chan[live])
+    err = acc_err(acc.live[live], chan[live], B)
     assert err < tol, (err, label)
+    if out is not None:
+        out.update(src=src, acc=acc.live, en=en.live if en else None, co=co.live if co else None)
     if not debug:
         return name
     e = en.live.view(B, cc)
@@ -158,7 +182,7 @@ def score(lib, path, B, C, H, W, *, c_begin=0, c_count=None, batch_step=1, row=N
     assert not bool(torch.isnan(co.live).any()), 'coeff_out not written everywhere: ' + label
     if n * H * W <= 1 << 18:
         from scipy.fft import dctn
-        z = dctn(src.cpu().numpy().astype(np.float64), type=2, norm='ortho', axes=(-2, -1))
+        z = dctn(src.double().cpu().numpy(), type=2, norm='ortho', axes=(-2, -1))
         got = co.live.view(B, cc, H, W).cpu().numpy()
         assert np.abs(got - z).max() <= COEFF_TOL * np.abs(z).max(), label
     return name
@@ -173,9 +197,9 @@ def takes(path, n):
 PATH_SIDES = [(p, n) for p in ('auto', 'kron', 'stack', 'tmem', 'umma', 'large', 'simt') for n in SIDES if takes(p, n)]
 
 
-def geometry(lib, path, N):
+def geometry(lib, path, N, dtype=torch.float32):
     """(maps per tile, tiles at which every CTA loops over its ring of stages more than twice) of the kernel that `path` runs on
-    N x N maps; (maps per CTA tile, None) for the CUDA-core kernels, which have no ring."""
+    N x N maps of `dtype`; (maps per CTA tile, None) for the CUDA-core kernels, which have no ring."""
     sm = lib.dctp_sm_count()
     kern = path
     if path == 'auto':
@@ -183,7 +207,9 @@ def geometry(lib, path, N):
                 'tmem' if 52 <= N <= 64 else 'umma' if N <= 128 else 'simt')
     ms = -(-N // 8) * 8
     if kern == 'kron':                                       # 128-map sub-tiles, 1, 2 or 4 per TMA tile; a ring of 3
-        return 128 * ((1 if N == 8 else 2) if N % 2 == 0 else (1 if N == 7 else 2 if N == 5 else 4)), sm * 7
+        if N % 2 == 0 and (N * N * dtype.itemsize) % 16 == 0:  # row layout: every even side in fp32, sides 4 and 8 in 16-bit
+            return 128 * (1 if N == 8 else 2), sm * 7
+        return 128 * (1 if N in (6, 7) else 2 if N in (2, 5) else 4), sm * 7
     if kern == 'stack':                                      # G * J maps per tile; a ring of 3
         kp = -(-N // 16) * 16
         return (32 if kp == 16 else 8 if kp == 32 else 2), sm * 7
@@ -211,8 +237,8 @@ def map_counts(path, N, mt, wrap):
     cases = {'one map': first(1, lambda n: n == 1)}
     if mt > 1:
         cases['one tile'] = first(mt, lambda n: n == mt)
-        cases['ragged last tile, stream ends on a 128-byte row'] = first(mt + 1, lambda n: n % mt and (n * NN) % 32 == 0)
-        cases['ragged last tile, stream ends inside a 128-byte row'] = first(mt + 1, lambda n: n % mt and (n * NN) % 32)
+        cases['ragged last tile, stream ends on a 32-element row'] = first(mt + 1, lambda n: n % mt and (n * NN) % 32 == 0)
+        cases['ragged last tile, stream ends inside a 32-element row'] = first(mt + 1, lambda n: n % mt and (n * NN) % 32)
     else:
         cases['several maps'] = 5
     if wrap:
@@ -222,7 +248,7 @@ def map_counts(path, N, mt, wrap):
 
 @pytest.mark.parametrize('path,n', PATH_SIDES)
 def test_score_stays_inside_its_buffers(lib, cuda_device, path, n):
-    """Each kernel path on each side: one map, one tile, ragged last tiles (the stream ending on a 128-byte row and inside one), and
+    """Each kernel path on each side: one map, one tile, ragged last tiles (the stream ending on a 32-element row and inside one), and
     enough tiles that every CTA's mbarrier phases wrap - with per-map energies and coefficients (the debug instantiations) and
     without (the production ones)."""
     mt, wrap = geometry(lib, path, n)
@@ -320,13 +346,15 @@ def test_multi_site_entry(lib, cuda_device, side, n_sites):
     assert launches == want_launches, (launches, want_launches, name)
     assert acc.guards_intact(), 'accumulator guard written'
     energy = [torch.zeros(c, dtype=torch.float64, device='cuda') for _, c, _ in plan]
+    images = [0] * n_sites                      # maps each channel of an accumulator receives
     for i in live:
         energy[slot[i]] += (src[i].double() ** 2).sum((2, 3)).sum(0)
+        images[slot[i]] += plan[i][0]
     for j, e in enumerate(energy):
         got = acc.views[j]
         assert not bool(torch.isnan(got).any()), ('NaN in the accumulator of site', j, name)
         assert bool((got[e == 0] == 0.5).all()), ('a dead channel (or an unused accumulator) changed', j, name)
-        assert rel_err(got[e > 0] - 0.5, e[e > 0]) < ENERGY_TOL, (j, name)
+        assert acc_err(got[e > 0], e[e > 0], images[j]) < ENERGY_TOL, (j, name)
 
     ref = [torch.full((c,), 0.5, dtype=torch.float64, device='cuda') for _, c, _ in plan]
     for i in live:

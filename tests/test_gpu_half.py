@@ -4,6 +4,8 @@ dctp_score_accum_multi_ex.
 The stacked-basis (even sides 10..64) and Kronecker (sides <= 8) kernels read 16-bit maps themselves; their per-map energies are
 held to the float64 energy of the widened maps at the bar tests/test_gpu_kernels.py applies to those kernels in fp32.  Every other
 shape and path widens the scored window to fp32 and runs the fp32 kernels: bit-identical to the fp32 entry on that copy.
+The guard-band and non-finite rules of test_gpu_bounds.py and test_gpu_nonfinite.py are applied to 16-bit input in
+test_gpu_half_bounds.py.
 """
 import ctypes
 import struct

@@ -18,7 +18,9 @@ float64 value otherwise).  What this module pins, for dctp_score_accum, dctp_sco
 Culprits sit at the first and the last map of the stream (a ragged last tile), at maps P - 1 and P for P = 2 .. 128 (the first
 or last map of a tile for every kernel's maps per tile) and at a few seeded random maps; at (0, 0), (N-1, N-1), (0, N-1) and
 the middle of their map; in distinct channels, at most one in eight.  The oracle is float64 on the host with the culprits left
-out, and for small cases the finite / non-finite pattern of the op-for-op port of the reference hook.
+out, and for small cases the finite / non-finite pattern of the op-for-op port of the reference hook.  test_gpu_half_bounds.py runs
+the same matrix on bf16 and fp16 maps (dctp_score_accum_ex, dctp_score_accum_multi_ex) through the helpers here, with the bit
+patterns of those types (KINDS16).
 """
 import numpy as np
 import pytest
@@ -31,9 +33,13 @@ from test_gpu_kernels import ENERGY_TOL, STACK_SIDES, TMEM_SIDES
 
 pytestmark = pytest.mark.gpu
 
-# culprit kinds: float32 bit patterns; 'all_nan' fills the whole map
+# culprit kinds: float32 bit patterns; 'all_nan' fills the whole map; 'flt_max' is the largest finite value of the type
 KINDS = {'nan': 0x7fc00000, 'neg_nan': 0xffc00000, 'snan': 0x7f800001, 'inf': 0x7f800000, 'neg_inf': 0xff800000,
          'all_nan': 0x7fc00000, 'flt_max': 0x7f7fffff}
+KINDS16 = {torch.bfloat16: {'nan': 0x7fc0, 'neg_nan': 0xffc0, 'snan': 0x7f81, 'inf': 0x7f80, 'neg_inf': 0xff80, 'all_nan': 0x7fc0,
+                            'flt_max': 0x7f7f},
+           torch.float16: {'nan': 0x7e00, 'neg_nan': 0xfe00, 'snan': 0x7c01, 'inf': 0x7c00, 'neg_inf': 0xfc00, 'all_nan': 0x7e00,
+                           'flt_max': 0x7bff}}
 TILE_EDGES = (2, 4, 8, 16, 32, 64, 128)
 
 AUTO_SIDES = sorted(set(range(1, 9)) | set(STACK_SIDES) | {9, 11, 13, 34, 50, 54, 62, 72, 80, 96, 144, 160, 288, 320, 100, 130})
@@ -53,19 +59,22 @@ def family(path, N):
     return FAMILY[path]
 
 
-def bits(kind):
-    return int(np.array([KINDS[kind]], np.uint32).view(np.int32)[0])
+def bits(kind, dtype=torch.float32):
+    """The bit pattern of culprit `kind` in `dtype` (float32, bfloat16 or float16) as a signed integer of its width."""
+    if dtype == torch.float32:
+        return int(np.array([KINDS[kind]], np.uint32).view(np.int32)[0])
+    return int(np.array([KINDS16[dtype][kind]], np.uint16).view(np.int16)[0])
 
 
 def plant(x, b, c, kind, pos):
     """Culprit `kind` into map x[b, c] at position `pos` (0: (0, 0), 1: (H-1, W-1), 2: (0, W-1), 3: the middle)."""
     H, W = x.shape[2:]
-    xi = x.view(torch.int32)
+    xi = x.view(torch.int32 if x.element_size() == 4 else torch.int16)
     if kind == 'all_nan':
-        xi[b, c] = bits(kind)
+        xi[b, c] = bits(kind, x.dtype)
     else:
         i, j = ((0, 0), (H - 1, W - 1), (0, W - 1), (H // 2, W // 2))[pos]
-        xi[b, c, i, j] = bits(kind)
+        xi[b, c, i, j] = bits(kind, x.dtype)
 
 
 def culprit_maps(B, cc, seed):
@@ -83,13 +92,15 @@ def culprit_maps(B, cc, seed):
 
 
 def launch(lib, path, x, cb, cc, debug):
-    """dctp_score_accum of x[:, cb:cb + cc] into a zeroed accumulator (and energy_out set to -1 when `debug`)."""
+    """dctp_score_accum (dctp_score_accum_ex for 16-bit x) of x[:, cb:cb + cc] into a zeroed accumulator (and energy_out set to -1
+    when `debug`)."""
     B, _, H, W = x.shape
     acc = torch.zeros(cc, dtype=torch.float64, device='cuda')
     en = torch.full((B, cc), -1.0, device='cuda') if debug else None
     stream = _lib.current_stream()
-    _lib.check(lib.dctp_score_accum(_lib.ptr(x), B, H, W, x.stride(0), x.stride(1), x.stride(2), cb, cc, _lib.ptr(acc),
-                                    _lib.ptr(en), None, _lib.PATHS[path], stream))
+    args = (B, H, W, x.stride(0), x.stride(1), x.stride(2), cb, cc, _lib.ptr(acc), _lib.ptr(en), None, _lib.PATHS[path], stream)
+    code = _lib.dtype_code(x.dtype)
+    _lib.check(lib.dctp_score_accum(_lib.ptr(x), *args) if code == _lib.DTYPE_F32 else lib.dctp_score_accum_ex(_lib.ptr(x), code, *args))
     _lib.check(lib.dctp_check(stream))
     return acc.cpu().numpy(), (en.cpu().numpy() if debug else None), lib.dctp_last_kernel().decode()
 
@@ -98,13 +109,20 @@ def rel(got, want):
     return np.abs(got - want) / np.maximum(np.abs(want), 1e-30)
 
 
-def check(acc, en, want, bad, kind, tol, label):
-    """Rules 1 and 2.  want: float64 [B, cc] energies of the maps as scored; bad: [B, cc] culprit mask."""
+def culprit_ok(got, want, kind, may_overflow):
+    """Rule 1: non-finite; the largest finite value: within ENERGY_TOL of float64, or non-finite where its energy may overflow."""
+    if kind != 'flt_max':
+        return not np.isfinite(got)
+    return rel(got, want) < ENERGY_TOL if np.isfinite(got) else may_overflow
+
+
+def check(acc, en, want, bad, kind, tol, label, may_overflow=True):
+    """Rules 1 and 2.  want: float64 [B, cc] energies of the maps as scored; bad: [B, cc] culprit mask; may_overflow: False where
+    the square of the largest finite value of the input type is far from the fp32 range (fp16), so that culprit must stay finite."""
     bad_ch = bad.any(0)
     chan = want.sum(0)
     for c in np.flatnonzero(bad_ch):
-        assert not np.isfinite(acc[c]) or (kind == 'flt_max' and rel(acc[c], chan[c]) < ENERGY_TOL), \
-            'culprit channel %d scored %r: %s' % (c, acc[c], label)
+        assert culprit_ok(acc[c], chan[c], kind, may_overflow), 'culprit channel %d scored %r: %s' % (c, acc[c], label)
     ok = ~bad_ch
     assert np.isfinite(acc[ok]).all(), 'non-finite score in clean channels %s: %s' % (np.flatnonzero(ok & ~np.isfinite(acc)), label)
     dead = ok & (chan == 0)
@@ -116,8 +134,7 @@ def check(acc, en, want, bad, kind, tol, label):
         return
     for b, c in zip(*np.nonzero(bad)):
         e = float(en[b, c])
-        assert not np.isfinite(e) or (kind == 'flt_max' and rel(e, want[b, c]) < ENERGY_TOL), \
-            'culprit map (%d, %d) energy %r: %s' % (b, c, e, label)
+        assert culprit_ok(e, want[b, c], kind, may_overflow), 'culprit map (%d, %d) energy %r: %s' % (b, c, e, label)
     assert np.isfinite(en[~bad]).all(), 'non-finite energy_out of a clean map: %s' % label
     dead = ~bad & (want == 0)
     assert (en[dead] == 0).all(), 'dead maps must score exactly 0: %s' % label
@@ -134,8 +151,10 @@ def port_pattern(window):
 
 
 def culprits_everywhere(lib, path, x, cb, cc, kernel, seed, what, tol=ENERGY_TOL, port_check=False):
-    """Every culprit kind at the culprit maps of the window x[:, cb:cb + cc], with and without energy_out."""
+    """Every culprit kind at the culprit maps of the window x[:, cb:cb + cc] (fp32, bf16 or fp16), with and without energy_out.
+    Returns the kernels that ran."""
     B = x.shape[0]
+    names = set()
     win = x[:, cb:cb + cc]
     clean = win.clone()
     picks = culprit_maps(B, cc, seed)
@@ -146,23 +165,27 @@ def culprits_everywhere(lib, path, x, cb, cc, kernel, seed, what, tol=ENERGY_TOL
         for i, m in enumerate(picks):
             plant(win, m // cc, m % cc, kind, i % 4)
         host = win.cpu()
-        want = port.energy_parseval64(host.numpy())
+        want = port.energy_parseval64(host.double().numpy())
         for debug in (True, False):
             acc, en, name = launch(lib, path, x, cb, cc, debug)
-            label = '%s %s, culprit %s at maps %s%s: %s' % (path, what, kind, picks, ' [energy_out]' if debug else '', name)
+            names.add(name.split(' (')[0])
+            label = '%s %s %s, culprit %s at maps %s%s: %s' % (path, str(x.dtype).split('.')[-1], what, kind, picks,
+                                                              ' [energy_out]' if debug else '', name)
             assert name.startswith(kernel), label
-            check(acc, en, want, bad, kind, tol, label)
+            check(acc, en, want, bad, kind, tol, label, may_overflow=x.dtype != torch.float16)
             if port_check and kind != 'flt_max' and not debug:
-                np.testing.assert_array_equal(np.isfinite(acc), port_pattern(host), err_msg=label)
+                np.testing.assert_array_equal(np.isfinite(acc), port_pattern(host.float()), err_msg=label)
         win.copy_(clean)
+    return names
 
 
-def dense_shape(lib, path, N):
-    """(B, C) of a dense call on N x N maps: a ragged last tile, and a whole number of float4 where the TMEM-operand kernel needs
-    it.  Maps of 72 x 72 and more: 32 maps (the kernels there take one map, or one 128-row slab of one, per work item)."""
+def dense_shape(lib, path, N, dtype=torch.float32):
+    """(B, C) of a dense call on N x N maps of `dtype`: a ragged last tile, and a whole number of float4 where the TMEM-operand
+    kernel needs it.  Maps of 72 x 72 and more: 32 maps (the kernels there take one map, or one 128-row slab of one, per work
+    item)."""
     if N >= 72:
         return 2, 16
-    mt, _ = geometry(lib, path, N)
+    mt, _ = geometry(lib, path, N, dtype)
     tmem = path == 'tmem' or (path == 'auto' and family('auto', N) == 'score_t_kernel')
     for B, C in ((3, 139), (3, 140), (3, 141), (2, 139), (2, 140)):
         if (mt == 1 or (B * C) % mt) and not (tmem and N % 2 and (B * C * N * N) % 4):
@@ -201,17 +224,18 @@ def test_simt_non_square_and_cropped(lib, cuda_device):
 
 
 # ------------------------------------------------------------------------------------------------------ the multi-site entry
-@pytest.mark.parametrize('k', [0, 7, 15])
-@pytest.mark.parametrize('side', [7, 14, 28, 56, 160])
-def test_multi_site_culprit_stays_in_its_site(lib, cuda_device, side, k):
-    """dctp_score_accum_multi over 16 dense sites with a culprit in site k: every other site matches float64 and a clean call
-    per site (tiles and work items never span two sites)."""
+def multi_site_culprit(lib, side, k, kinds, dtype=torch.float32):
+    """dctp_score_accum_multi (_ex for 16-bit `dtype`) over 16 dense sites with a culprit of each of `kinds` in site k: the culprit
+    follows the rules of check() and every other site matches float64 and a clean call per site.  Returns the kernel that ran."""
     n_sites = 16
+    code = _lib.dtype_code(dtype)
     shapes = [(1 + i % 3, (9, 16, 11)[i % 3]) for i in range(n_sites)]
-    xs = [maps(B, c, side, side, seed=100 * side + i) for i, (B, c) in enumerate(shapes)]
+    xs = [maps(B, c, side, side, seed=100 * side + i, dtype=dtype) for i, (B, c) in enumerate(shapes)]
     Bk, ck = shapes[k]
     bc = (Bk - 1, ck - 1 - k % 3)
-    for kind in ('nan', 'neg_inf'):
+    clean = xs[k].clone()
+    for kind in kinds:
+        xs[k].copy_(clean)
         plant(xs[k], bc[0], bc[1], kind, k % 4)
         accs = [torch.zeros(c, dtype=torch.float64, device='cuda') for _, c in shapes]
         sites = (_lib.Site * n_sites)()
@@ -220,23 +244,36 @@ def test_multi_site_culprit_stays_in_its_site(lib, cuda_device, side, k):
             sites[i].x, sites[i].accum = xs[i].data_ptr(), accs[i].data_ptr()
         stream = _lib.current_stream()
         _lib.check(lib.dctp_prepare(side, side))
-        _lib.check(lib.dctp_score_accum_multi(sites, n_sites, side, side, stream))
+        if code == _lib.DTYPE_F32:
+            _lib.check(lib.dctp_score_accum_multi(sites, n_sites, side, side, stream))
+        else:
+            _lib.check(lib.dctp_score_accum_multi_ex(sites, n_sites, side, side, code, stream))
         _lib.check(lib.dctp_check(stream))
         name = lib.dctp_last_kernel().decode()
         assert name.startswith(family('auto', side)), name
         for i, (B, c) in enumerate(shapes):
-            want = port.energy_parseval64(xs[i].cpu().numpy())
+            want = port.energy_parseval64(xs[i].double().cpu().numpy())
             bad = np.zeros((B, c), bool)
             if i == k:
                 bad[bc] = True
-            check(accs[i].cpu().numpy(), None, want, bad, kind, ENERGY_TOL, 'site %d of 16, side %d, culprit %s in site %d: %s'
-                  % (i, side, kind, k, name))
+            check(accs[i].cpu().numpy(), None, want, bad, kind, ENERGY_TOL, 'site %d of 16, side %d, %s culprit %s in site %d: %s'
+                  % (i, side, str(dtype).split('.')[-1], kind, k, name), may_overflow=dtype != torch.float16)
             if i != k:
                 ref = torch.zeros(c, dtype=torch.float64, device='cuda')
-                _lib.check(lib.dctp_score_accum(xs[i].data_ptr(), B, side, side, c * side * side, side * side, side, 0, c,
-                                                _lib.ptr(ref), None, None, _lib.PATH_AUTO, stream))
+                args = (B, side, side, c * side * side, side * side, side, 0, c, _lib.ptr(ref), None, None, _lib.PATH_AUTO, stream)
+                _lib.check(lib.dctp_score_accum(xs[i].data_ptr(), *args) if code == _lib.DTYPE_F32
+                           else lib.dctp_score_accum_ex(xs[i].data_ptr(), code, *args))
                 np.testing.assert_allclose(accs[i].cpu().numpy(), ref.cpu().numpy(), rtol=1e-12, err_msg='site %d' % i)
         _lib.check(lib.dctp_check(stream))
+    return name
+
+
+@pytest.mark.parametrize('k', [0, 7, 15])
+@pytest.mark.parametrize('side', [7, 14, 28, 56, 160])
+def test_multi_site_culprit_stays_in_its_site(lib, cuda_device, side, k):
+    """dctp_score_accum_multi over 16 dense sites with a culprit in site k: every other site matches float64 and a clean call
+    per site (tiles and work items never span two sites)."""
+    multi_site_culprit(lib, side, k, ('nan', 'neg_inf'))
 
 
 # ---------------------------------------------------------------------------------------------------------------- density
