@@ -97,6 +97,10 @@ void note_kernel(const char* fmt, ...) {
 
 // ------------------------------------------------------------------ cosine bases
 inline double dct_coef(int k, int n, int N) {          // orthonormal DCT-II: C_N[k][n]
+    // cos(pi (2n + 1) k / 2N) is exactly 0 where (2n + 1) k = N mod 2N (sides with an odd factor).  std::cos returns rounding noise
+    // there (1e-17 .. 1e-15, and 1e-33 for products of two in C_N (x) C_N), whose split lo parts go down to 2^-117: multiplied by a
+    // map of small values they underflow, and the coefficients they make stop scaling with the map.
+    if (((2 * n + 1) * k) % (2 * N) == N) return 0.0;
     const double s = k == 0 ? std::sqrt(1.0 / N) : std::sqrt(2.0 / N);
     return s * std::cos(M_PI * (2.0 * n + 1.0) * k / (2.0 * N));
 }

@@ -15,7 +15,8 @@ from oracle import reference_port as port
 pytestmark = pytest.mark.gpu
 
 REL_TOL = 1e-4           # the north_star bar on scores
-ENERGY_TOL = 2e-5        # what the bf16x3 / fp32 kernels actually deliver per map
+ENERGY_TOL = 2e-5        # what the bf16x3 / fp32 kernels deliver per map on random maps (relu_maps; the rounding errors cancel),
+                         # not a bound: on maps built to line them up they reach 5e-5 (test_gpu_precision.py)
 
 
 def relu_maps(shape, seed, dead_every=0):
