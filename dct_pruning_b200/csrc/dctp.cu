@@ -1,5 +1,6 @@
 // libdctp.so - C ABI (include/dctp.h) over the sm_100a DCT importance-score kernels.
 // Host side only: argument checks, cosine-basis cache, kernel selection and launch geometry.
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -231,15 +232,24 @@ int get_stack_basis(int N, StackBasis& out) {
             img[lane * 32 + k / 2] |= static_cast<uint32_t>(part ? l : h) << (16 * (k & 1));
         }
     }
+    // folded stage 2 (stack_folded): rows h < fd of a map are paired with rows N-1-h, the middle rows [fd, N - fd) (Np / 8 odd) are not
+    const bool folded = stack_folded(KP);
+    const int fd = 8 * (Np / 16), fold = std::min(N / 2, fd);
+    // stage-2 basis: C_N[u][h] unfolded; folded, chain c (u = 2 u' + c) in rows [c W2, (c + 1) W2): C_N[2 u' + c][k] at contraction
+    // column k < N - fold (the paired rows' h, then the middle rows' h)
     std::vector<uint8_t> chi(S::C2_HALF, 0), clo(S::C2_HALF, 0);
     for (int u = 0; u < N; ++u)
-        for (int h = 0; h < N; ++h) {
+        for (int h = 0; h < (folded ? N - fold : N); ++h) {
             uint16_t hh, ll;
             split_bf16(dct_coef(u, h, N), hh, ll);
-            const size_t off = static_cast<size_t>(h / 8) * S::LBO2 + u * 16 + (h % 8) * 2;
+            const int row = folded ? (u & 1) * stack_fold_k(KP) + u / 2 : u;
+            const size_t off = static_cast<size_t>(h / 8) * S::LBO2 + row * 16 + (h % 8) * 2;
             std::memcpy(&chi[off], &hh, 2);
             std::memcpy(&clo[off], &ll, 2);
         }
+    // Bx row (= D1 column) of row h of a map: h unfolded; folded, row N-1-h' (h' < fold) at fd + h', so that each thread of epilogue 1
+    // holds both rows of a pair, and the middle rows from 2 fd on
+    auto bx_row = [&](int h) { return !folded || h < fold ? h : h >= N - fold ? fd + (N - 1 - h) : 2 * fd + (h - fold); };
     StackBasis b;
     b.kp = KP;
     b.vec = (N % 4) == 0 ? 4 : 2;
@@ -250,7 +260,7 @@ int get_stack_basis(int N, StackBasis& out) {
         for (int f = 0; f < b.tile_vec; ++f)
             for (int pc = 0; pc < pieces; ++pc) {
                 const int e = 4 * f + 2 * pc, m = e / NN, rem = e % NN, h = rem / N, w = rem % N, gI = m / J, set = m % J;
-                const int n = gI * Np + h, k = set * KP + w;
+                const int n = gI * Np + bx_row(h), k = set * KP + w;
                 tab[static_cast<size_t>(f) * pieces + pc] = static_cast<uint16_t>((k / 8) * lbo + n * 16 + (k % 8) * 2);
             }
     };
@@ -412,7 +422,7 @@ int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* 
     a.tile_elems = a.MT * a.NN; a.tile_rows = a.tile_elems / 32; a.tile_vec = basis.tile_vec;
     a.num_tiles = fill_segments(a.seg, sites, n, a.NN, a.MT);
     a.idesc1 = umma::make_idesc_bf16(128, a.ncols, false, false);
-    a.idesc2 = umma::make_idesc_bf16(128, KP, false, false);
+    a.idesc2 = umma::make_idesc_bf16(128, stack_folded(KP) ? stack_fold_k(KP) : KP, false, false);
     a.lbo1 = basis.lbo1;
     a.a_img = basis.a_img; a.c2_hi = basis.c2_hi; a.c2_lo = basis.c2_lo; a.table = basis.table; a.table_bytes = basis.table_bytes;
     a.energy_out = n == 1 ? energy_out : nullptr; a.dump = n == 1 ? coeff_out : nullptr; a.status = g.status;

@@ -19,12 +19,15 @@
 //             tcgen05.st 16x128b: A2[(q,s,r), h] for map g = 2t + s of the warp's set; never leaves TMEM
 //   stage 2   per A2 tile t:  D2[(q,s,r), u] = sum_h A2[(q,s,r), h] * C[u,h]       3 passes (hi*hi + lo*hi + hi*lo)
 //             B = C_N resident in shared memory; every lane of a tile is a live row (two maps per warp)
+//             KP >= 32 folded (stack_folded): epilogue 1 writes the row sums and differences of D1 (y + y', y - y' of rows h, N-1-h),
+//             and each pass is two chains of half the K and N, even u against the sums and odd u against the differences
 //   epi   2   tcgen05.ld 32x32b -> sum of squares per lane -> 16-lane shuffle tree -> fixed-order sum over the
 //             warps of a map -> one fp64 atomicAdd per map
 //
-// Tensor-core time per 25 KB of input: 448 + 384 cycles at 56x56 (score_tmem.cuh: 672 + 384), 512 + 192 at 28x28,
-// 512 + 96 at 14x14, against 940-1113 cycles of HBM time at the measured 6.55 TB/s (the SM clock under this load is 1.65-1.7 GHz, not the
-// 1.965 GHz nvidia-smi shows).
+// Tensor-core time per 25 KB of input: 448 + 192 cycles at 56x56 (unfolded stage 2 384; score_tmem.cuh: 672 + 384), 512 + 96 at 28x28
+// (unfolded 192), 512 + 96 at 14x14 (not folded), against 940-1113 cycles of HBM time at the measured 6.55 TB/s (the SM clock under this
+// load is 1.65-1.7 GHz, not the 1.965 GHz nvidia-smi shows).  The fold also halves the shared-memory reads of the stage-2 basis, 192 -> 96
+// wavefronts per tile at 56x56 and 28x28.
 //
 // The kernel is warp specialised (one CTA per SM), every hand-over is an mbarrier.  Roles, in warp order:
 //   converters  NCONV warps (12 in production) in NCG = 2 groups that alternate tiles: fp32 tile -> bf16 hi/lo -> Bx (two buffers),
@@ -143,6 +146,16 @@ constexpr int STACK_NCG = 2, STACK_NE1G = 1, STACK_NE2G = 2;
 // warps of a CTA with NCONV converter warps: converters, epilogue 1 (8 per group), epilogue 2 (4 per group), producer, two issuers
 constexpr int stack_warps(int nconv) { return nconv + 8 * STACK_NE1G + 4 * STACK_NE2G + 3; }
 
+// Folded stage 2 (KP >= 32; at KP = 16 one chain is already K = 16, the minimum).  The DCT-II basis has C[u][N-1-h] = (-1)^u C[u][h],
+// so  D2[., u] = sum_{h < N/2} C[u][h] (Y[., h] + (-1)^u Y[., N-1-h]):  two chains of K = N = stack_fold_k(KP) each - even u against
+// the row sums of Y = D1, odd u against the row differences - do the work of one chain of K = N = KP, with half the MMA work and half
+// the basis reads.  The converters' table puts row N-1-h of a map at D1 column fold_d + h (fold_d = 8 * (Np / 16)), so that each
+// thread of epilogue 1 holds both rows of a pair; with Np / 8 odd (N = 18..24, 36, 40, 52, 56 - whole 8-column halves would not fit
+// in Np) only rows h < fold_d are paired, and the middle rows [fold_d, N - fold_d) sit unpaired in the 8 columns from 2 * fold_d on,
+// in both chains (the basis holds C[u][h] there for every u).  A2 and D2 of a map: even chain at [0, K), odd chain at [K, 2K).
+__host__ __device__ constexpr bool stack_folded(int kp) { return kp >= 32; }
+__host__ __device__ constexpr int stack_fold_k(int kp) { return kp == 32 ? 16 : 32; }
+
 // KP: contraction length per map (N rounded up to 16); VEC: granularity of a row in the fp32 stream (4: N % 4 == 0, 2: N even)
 // NCONV: converter warps (8 or 12).
 // Every warp polls the mbarriers it depends on itself.  (Measured and dropped: one polling warp per role releasing its siblings
@@ -158,8 +171,12 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
     using namespace umma;
     constexpr int NCG = STACK_NCG, NE1G = STACK_NE1G, NE2G = STACK_NE2G;
     constexpr int J = KP <= 32 ? 64 / KP : 1;
-    constexpr int K1S = J * KP / 16, K2S = KP / 16;
+    constexpr int K1S = J * KP / 16;
     constexpr int G = KP == 16 ? 8 : KP == 32 ? 4 : 2, T2 = G / 2;
+    // stage 2: NC2 chains (two when folded) of K = N = W2; a map's A2 (hi part, in bf16 elements) and D2 take KF = NC2 * W2 columns
+    constexpr bool FOLD = stack_folded(KP);
+    constexpr int W2 = FOLD ? stack_fold_k(KP) : KP, NC2 = FOLD ? 2 : 1, KF = NC2 * W2, K2S = W2 / 16;
+    static_assert(T2 * KF <= 64, "A2 and D2 buffers are 64 columns");
     constexpr uint32_t W_E1 = NCONV, W_E2 = NCONV + 8 * NE1G, W_PROD = W_E2 + 4 * NE2G, W_MMA = W_PROD + 1, W_MMA2 = W_PROD + 2, NT = (W_MMA2 + 1) * 32;
     constexpr uint32_t NCT = NCONV * 32 / NCG;                            // threads that convert one tile
     // Bx buffers in use: with three the converters run a tile further ahead of stage 1 (same box: 56x56 4.25 -> 4.59 TB/s, 64-channel launches
@@ -371,16 +388,19 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                 TR_ADD(tr1);
                 tc_fence_after_sync();
 #pragma unroll
-                for (int t = 0; t < T2; ++t) {
-                    const uint32_t d = tmem + TM_D2 + b2 * 64 + t * KP;
-                    const uint32_t ahi = tmem + TM_A2 + b * 64 + t * KP, alo = ahi + KP / 2;
+                for (int t = 0; t < T2; ++t)
 #pragma unroll
-                    for (int pass = 0; pass < 3; ++pass)
+                    for (int c = 0; c < NC2; ++c) {                        // chain c: columns [c W2, (c + 1) W2) of the map, basis rows too
+                        const uint32_t d = tmem + TM_D2 + b2 * 64 + t * KF + c * W2;
+                        const uint32_t ahi = tmem + TM_A2 + b * 64 + t * KF + c * (W2 / 2), alo = ahi + KF / 2;
 #pragma unroll
-                        for (int ks = 0; ks < K2S; ++ks)
-                            mma_bf16_ts(d, (pass == 1 ? alo : ahi) + 8 * ks,
-                                        desc_with_lo(desc2, (pass == 2 ? lo_c2_lo : lo_c2_hi) + ks * STEP2), a.idesc2, (pass | ks) != 0);
-                }
+                        for (int pass = 0; pass < 3; ++pass)
+#pragma unroll
+                            for (int ks = 0; ks < K2S; ++ks)
+                                mma_bf16_ts(d, (pass == 1 ? alo : ahi) + 8 * ks,
+                                            desc_with_lo(desc2, (pass == 2 ? lo_c2_lo : lo_c2_hi) + c * W2 + ks * STEP2), a.idesc2,
+                                            (pass | ks) != 0);
+                    }
                 mma_commit(d2_full + b);
                 mma_commit(a2_free + b);
                 TR_ADD(tr2);
@@ -542,7 +562,8 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
             // The warp's share of D1 is T2 maps x (KP / 16) chunks of 16 columns (both lane halves: 8 + 8 registers a chunk).  Two chunks
             // are requested per TMEM round trip (a load takes hundreds of cycles while the tensor core and the other warps use the same
             // memory), whichever maps they belong to: two round trips a tile for every KP (one per map would be four at KP = 16).
-            constexpr int CPT = KP / 16, NCH = T2 * CPT;                   // chunks per map, chunks per tile
+            // (folded stage 2: the loop after this one)
+            constexpr int CPT = KP / 16, NCH = FOLD ? 0 : T2 * CPT;        // chunks per map, chunks per tile
 #pragma unroll
             for (int ch0 = 0; ch0 < NCH; ch0 += 2) {
                 uint32_t za[16], zb[16];
@@ -587,6 +608,72 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                     }
                 }
             }
+            // Folded stage 2 (stack_folded): a unit is either the 8 D1 columns of rows h with the 8 columns of their partners N-1-h
+            // fold_d further on (a fold unit: y + y' to the even chain's A2 columns at the unit's position, y - y' to the odd chain's),
+            // or the 8 columns of the unpaired middle rows (to both chains).  Two units per TMEM round trip (two fold units, a fold unit
+            // and the middle rows, or the middle rows alone): two round trips a tile, as above.
+            constexpr int D8 = NP8 / 2, MID = NP8 & 1, RT = (D8 + MID + 1) / 2, NRT = FOLD ? T2 * RT : 0;   // round trips per map, per tile
+#pragma unroll
+            for (int rt = 0; rt < NRT; ++rt) {
+                const int t = rt / RT, k0 = 2 * (rt % RT);                // the warp's map t, units k0 and k0 + 1
+                const int nf = k0 + 1 < D8 ? 2 : k0 < D8 ? 1 : 0;          // fold units of the round
+                const bool mid = MID && k0 + 1 >= D8;                      // ... and the middle rows (unit D8)
+                const uint32_t src = d1 + lane_q + (2 * t + s) * a.Np, hb = 16u << 16;    // (+ hb: the lanes of C_lo)
+                uint32_t za[16], zb[16];                                   // [0, 8): rows (fold units; or a fold unit | the middle rows), [8, 16): partners
+                if (nf == 2) {
+                    tmem_ld_frag16(src + 8 * k0, reinterpret_cast<uint32_t (&)[8]>(za[0]));
+                    tmem_ld_frag16(src + hb + 8 * k0, reinterpret_cast<uint32_t (&)[8]>(zb[0]));
+                    tmem_ld_frag16(src + 8 * (k0 + D8), reinterpret_cast<uint32_t (&)[8]>(za[8]));
+                    tmem_ld_frag16(src + hb + 8 * (k0 + D8), reinterpret_cast<uint32_t (&)[8]>(zb[8]));
+                } else {
+                    if (nf == 1) {
+                        tmem_ld_frag8(src + 8 * k0, reinterpret_cast<uint32_t (&)[4]>(za[0]));
+                        tmem_ld_frag8(src + hb + 8 * k0, reinterpret_cast<uint32_t (&)[4]>(zb[0]));
+                        tmem_ld_frag8(src + 8 * (k0 + D8), reinterpret_cast<uint32_t (&)[4]>(za[8]));
+                        tmem_ld_frag8(src + hb + 8 * (k0 + D8), reinterpret_cast<uint32_t (&)[4]>(zb[8]));
+                    }
+                    if (mid) {
+                        tmem_ld_frag8(src + 16 * D8, reinterpret_cast<uint32_t (&)[4]>(za[4]));
+                        tmem_ld_frag8(src + hb + 16 * D8, reinterpret_cast<uint32_t (&)[4]>(zb[4]));
+                    }
+                }
+                tmem_ld_wait();
+                if (rt + 1 == NRT) {                                       // every column of D1 this warp needs is in registers
+                    tc_fence_before_sync();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive(d1_free + b);
+                }
+                uint32_t sh[4], sl[4], dh[4], dl[4];
+#pragma unroll
+                for (int i = 0; i < 2 * nf; ++i) {
+                    const uint64_t y = add2_packed(pack2(za[2 * i], za[2 * i + 1]), pack2(zb[2 * i], zb[2 * i + 1]));
+                    const uint64_t yp = add2_packed(pack2(za[8 + 2 * i], za[9 + 2 * i]), pack2(zb[8 + 2 * i], zb[9 + 2 * i]));
+                    split2_packed(add2_packed(y, yp), sh[i], sl[i]);
+                    split2_packed(sub2_packed(y, yp), dh[i], dl[i]);
+                }
+                const uint32_t even = tmem + TM_A2 + b * 64 + t * KF + lane_s, odd = even + W2 / 2;      // hi parts; lo: + KF / 2
+                if (nf == 2) {
+                    tmem_st_frag8(even + 4 * k0, sh);
+                    tmem_st_frag8(even + KF / 2 + 4 * k0, sl);
+                    tmem_st_frag8(odd + 4 * k0, dh);
+                    tmem_st_frag8(odd + KF / 2 + 4 * k0, dl);
+                } else if (nf == 1) {
+                    tmem_st_frag4(even + 4 * k0, sh[0], sh[1]);
+                    tmem_st_frag4(even + KF / 2 + 4 * k0, sl[0], sl[1]);
+                    tmem_st_frag4(odd + 4 * k0, dh[0], dh[1]);
+                    tmem_st_frag4(odd + KF / 2 + 4 * k0, dl[0], dl[1]);
+                }
+                if (mid) {
+                    uint32_t h[2], l[2];
+#pragma unroll
+                    for (int i = 0; i < 2; ++i)
+                        split2_packed(add2_packed(pack2(za[4 + 2 * i], za[5 + 2 * i]), pack2(zb[4 + 2 * i], zb[5 + 2 * i])), h[i], l[i]);
+                    tmem_st_frag4(even + 4 * D8, h[0], h[1]);
+                    tmem_st_frag4(even + KF / 2 + 4 * D8, l[0], l[1]);
+                    tmem_st_frag4(odd + 4 * D8, h[0], h[1]);
+                    tmem_st_frag4(odd + KF / 2 + 4 * D8, l[0], l[1]);
+                }
+            }
             tmem_st_wait();
             tc_fence_before_sync();
             __syncwarp();
@@ -627,9 +714,9 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                 if (chan0 >= C) chan0 -= C;
             }
             float e[T2];
-            // the lane's T2 * KP (64 or 48) coefficients in two round trips of at most 32 registers; D2 is handed back as soon
-            // as the second one has landed
-            constexpr int TOT = T2 * KP, HALF = TOT >= 32 ? 32 : TOT;
+            // the lane's T2 * KF (64) coefficients in two round trips of 32 registers; D2 is handed back as soon as the second one has
+            // landed
+            constexpr int TOT = T2 * KF, HALF = TOT >= 32 ? 32 : TOT;
             float part[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
             for (int c0 = 0; c0 < TOT; c0 += HALF) {
@@ -647,7 +734,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
 #pragma unroll
                 for (int c = 0; c < HALF; c += 16) {
                     if (c0 + c < TOT) {
-                        const int t = (c0 + c) / KP;                        // A2 tile these 16 columns belong to (KP is a multiple of 16)
+                        const int t = (c0 + c) / KF;                        // A2 tile these 16 columns belong to (KF is a multiple of 16)
                         float p0 = 0.f, p1 = 0.f, p2 = 0.f, p3 = 0.f;
 #pragma unroll
                         for (int i = 0; i < 4; ++i) {
@@ -662,11 +749,13 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
                         else part[0] += p;
                         if (TRACE && a.dump != nullptr) {
                             const uint32_t m = m0 + (2 * t + s) * J + my_set;
-                            const int u0 = (c0 + c) - t * KP;
+                            const int col = (c0 + c) - t * KF;                // of the map: u = col, folded 2 (col % W2) + chain col / W2
                             if (m < seg_maps && my_v < (uint32_t)a.N)
 #pragma unroll
-                                for (int i = 0; i < 16; ++i)
-                                    if (u0 + i < a.N) a.dump[static_cast<long long>(m) * a.NN + (u0 + i) * a.N + my_v] = __uint_as_float(z[c + i]);
+                                for (int i = 0; i < 16; ++i) {
+                                    const int u = FOLD ? 2 * (col % W2 + i) + col / W2 : col + i;
+                                    if (u < a.N) a.dump[static_cast<long long>(m) * a.NN + u * a.N + my_v] = __uint_as_float(z[c + i]);
+                                }
                         }
                     }
                 }

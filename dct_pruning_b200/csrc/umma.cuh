@@ -313,6 +313,11 @@ __device__ __forceinline__ uint64_t add2_packed(uint64_t x, uint64_t y) {
     asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(x), "l"(y));
     return r;
 }
+__device__ __forceinline__ uint64_t sub2_packed(uint64_t x, uint64_t y) {
+    uint64_t r;
+    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(x), "l"(y));
+    return r;
+}
 __device__ __forceinline__ uint64_t pack2(uint32_t lo_word, uint32_t hi_word) {
     return (static_cast<uint64_t>(hi_word) << 32) | lo_word;
 }
