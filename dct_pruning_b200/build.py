@@ -12,7 +12,7 @@ REPO = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, 'csrc')
 LIB_PATH = os.path.join(HERE, 'libdctp.so')
 SOURCES = [os.path.join(CSRC, 'dctp.cu')]
-HEADERS = [os.path.join(CSRC, f) for f in ('umma.cuh', 'score_umma.cuh', 'score_tmem.cuh', 'score_stack.cuh', 'score_kron.cuh', 'score_large.cuh', 'score_simt.cuh', 'topk.cuh', 'gather.cuh', 'score_alt.cuh', 'widen.cuh')] + \
+HEADERS = [os.path.join(CSRC, f) for f in ('umma.cuh', 'score_common.cuh', 'score_umma.cuh', 'score_tmem.cuh', 'score_stack.cuh', 'score_kron.cuh', 'score_large.cuh', 'score_simt.cuh', 'topk.cuh', 'gather.cuh', 'score_alt.cuh', 'widen.cuh')] + \
           [os.path.join(REPO, 'include', 'dctp.h')]
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-shared', '-Xcompiler', '-fPIC', '-Xptxas', '-v']

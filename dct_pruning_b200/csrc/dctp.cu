@@ -81,6 +81,7 @@ struct State {
     std::map<int, StackBasis> stack;                   // N
     std::map<int, KronBasis> kron;                     // N
     std::vector<void*> bases;                          // every device allocation of the basis caches above (dctp_shutdown frees them)
+    long long* trace = nullptr;                        // cycle stamps of a traced launch (DCTP_S/L/T_TRACE), TRACE_LEN entries
     void* encode_tiled = nullptr;                      // cuTensorMapEncodeTiled, resolved through the runtime (no libcuda link dependency)
     bool pdl = true;                                   // programmatic dependent launch of the score kernels (DCTP_PDL=0 disables)
     int regs[2][6][2] = {};                            // registers/thread per (KP, load mode, prefetch) instantiation
@@ -94,6 +95,29 @@ void note_kernel(const char* fmt, ...) {
     va_start(ap, fmt);
     vsnprintf(g.last_kernel, sizeof g.last_kernel, fmt, ap);
     va_end(ap);
+}
+
+// the end of every launch: count it, report a launch error
+int launched() {
+    ++g.launches;
+    CUDA_TRY(cudaGetLastError());
+    return DCTP_OK;
+}
+
+constexpr int TRACE_LEN = 256;                        // entries of the trace buffer: the longest trace (DCTP_T_TRACE) has 32 tiles x 8 stamps
+// trace = the zeroed trace buffer when the environment variable `var` asks for a traced launch, else null
+int trace_for(const char* var, long long*& trace) {
+    trace = nullptr;
+    if (!std::getenv(var)) return DCTP_OK;
+    if (!g.trace) CUDA_TRY(cudaMalloc(&g.trace, TRACE_LEN * sizeof(long long)));
+    CUDA_TRY(cudaMemset(g.trace, 0, TRACE_LEN * sizeof(long long)));
+    trace = g.trace;
+    return DCTP_OK;
+}
+// the trace the preceding launch wrote
+int read_trace(long long (&h)[TRACE_LEN]) {
+    CUDA_TRY(cudaMemcpy(h, g.trace, sizeof h, cudaMemcpyDeviceToHost));
+    return DCTP_OK;
 }
 
 // ------------------------------------------------------------------ cosine bases
@@ -133,37 +157,45 @@ int upload(const std::vector<T>& host, T*& dev) {
     return DCTP_OK;
 }
 
-int get_umma_basis(int N, int KP, UmmaBasis& out) {
-    auto key = std::make_pair(N, KP);
-    auto it = g.umma.find(key);
-    if (it != g.umma.end()) { out = it->second; return DCTP_OK; }
-    const int Ms = (N + 7) / 8 * 8, J = KP / Ms;
-    std::vector<uint16_t> hi(static_cast<size_t>(KP) * KP, 0), lo(hi.size(), 0);
-    for (int j = 0; j < J; ++j)
-        for (int v = 0; v < N; ++v)
-            for (int w = 0; w < N; ++w)
-                split_bf16(dct_coef(v, w, N), hi[(size_t)(j * Ms + v) * KP + j * Ms + w], lo[(size_t)(j * Ms + v) * KP + j * Ms + w]);
-    UmmaBasis b;
-    int rc;
-    if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
-    // scatter table of the dense load path: where element e of a full tile (maps back to back) lands in A1
-    const int G = 128 / Ms, MT = G * J, NN = N * N;
-    if ((MT * NN) % 4 == 0) {
-        b.vpe = (N % 4 == 0) ? 1 : (N % 2 == 0) ? 2 : 4;
-        b.tile_vec = MT * NN / 4;
-        const int step = 4 / b.vpe;
-        std::vector<uint16_t> tab(static_cast<size_t>(b.tile_vec) * b.vpe + 8, 0);
-        for (int v = 0; v < b.tile_vec; ++v)
-            for (int s = 0; s < b.vpe; ++s) {
-                const int e = 4 * v + s * step, t = e / NN, r = e % NN;
-                tab[(size_t)v * b.vpe + s] =
-                    static_cast<uint16_t>(detail::kmajor_off((t / J) * Ms + r / N, (t % J) * Ms + r % N, 128));
-            }
-        if ((rc = upload(tab, b.scatter))) return rc;
-    }
-    g.umma[key] = b;
+// out = cache[key], built by build(B&) and inserted on first use (a failed build inserts nothing)
+template <class Map, class Key, class B, class Build>
+int cached(Map& cache, const Key& key, B& out, Build build) {
+    auto it = cache.find(key);
+    if (it != cache.end()) { out = it->second; return DCTP_OK; }
+    B b;
+    if (int rc = build(b)) return rc;
+    cache[key] = b;
     out = b;
     return DCTP_OK;
+}
+
+int get_umma_basis(int N, int KP, UmmaBasis& out) {
+    return cached(g.umma, std::make_pair(N, KP), out, [&](UmmaBasis& b) {
+        const int Ms = (N + 7) / 8 * 8, J = KP / Ms;
+        std::vector<uint16_t> hi(static_cast<size_t>(KP) * KP, 0), lo(hi.size(), 0);
+        for (int j = 0; j < J; ++j)
+            for (int v = 0; v < N; ++v)
+                for (int w = 0; w < N; ++w)
+                    split_bf16(dct_coef(v, w, N), hi[(size_t)(j * Ms + v) * KP + j * Ms + w], lo[(size_t)(j * Ms + v) * KP + j * Ms + w]);
+        int rc;
+        if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
+        // scatter table of the dense load path: where element e of a full tile (maps back to back) lands in A1
+        const int G = 128 / Ms, MT = G * J, NN = N * N;
+        if ((MT * NN) % 4 == 0) {
+            b.vpe = (N % 4 == 0) ? 1 : (N % 2 == 0) ? 2 : 4;
+            b.tile_vec = MT * NN / 4;
+            const int step = 4 / b.vpe;
+            std::vector<uint16_t> tab(static_cast<size_t>(b.tile_vec) * b.vpe + 8, 0);
+            for (int v = 0; v < b.tile_vec; ++v)
+                for (int s = 0; s < b.vpe; ++s) {
+                    const int e = 4 * v + s * step, t = e / NN, r = e % NN;
+                    tab[(size_t)v * b.vpe + s] =
+                        static_cast<uint16_t>(detail::kmajor_off((t / J) * Ms + r / N, (t % J) * Ms + r % N, 128));
+                }
+            if ((rc = upload(tab, b.scatter))) return rc;
+        }
+        return DCTP_OK;
+    });
 }
 
 // D columns per tile slot of the TMEM-operand kernel; maps of side <= 16 sit two side by side (J = 2) in a 32-column slot
@@ -171,40 +203,37 @@ inline int t_n1max(int N) { return N <= 32 ? 32 : 64; }
 inline int t_groups(int N) { return N <= 8 ? 4 : N <= 16 ? 2 : 1; }
 
 int get_t_basis(int N, TBasis& out) {
-    auto it = g.tmem.find(N);
-    if (it != g.tmem.end()) { out = it->second; return DCTP_OK; }
-    const int Ms = (N + 7) / 8 * 8, G = 128 / Ms, NN = N * N, rows = t_n1max(N), J = t_groups(N);
-    std::vector<uint32_t> ahi(128 * 64, 0), alo(128 * 64, 0);
-    std::vector<uint16_t> chi(64 * 64, 0), clo(64 * 64, 0);
-    for (int gI = 0; gI < G; ++gI)
-        for (int v = 0; v < N; ++v)
-            for (int w = 0; w < N; ++w) {
-                uint16_t h, l;
-                split_bf16(dct_coef(v, w, N), h, l);
-                const int row = gI * Ms + v, k = gI * N + w;          // element k of the row sits in half (k & 1) of packed column k / 2
-                ahi[row * 64 + k / 2] |= static_cast<uint32_t>(h) << (16 * (k & 1));
-                alo[row * 64 + k / 2] |= static_cast<uint32_t>(l) << (16 * (k & 1));
+    return cached(g.tmem, N, out, [&](TBasis& b) {
+        const int Ms = (N + 7) / 8 * 8, G = 128 / Ms, NN = N * N, rows = t_n1max(N), J = t_groups(N);
+        std::vector<uint32_t> ahi(128 * 64, 0), alo(128 * 64, 0);
+        std::vector<uint16_t> chi(64 * 64, 0), clo(64 * 64, 0);
+        for (int gI = 0; gI < G; ++gI)
+            for (int v = 0; v < N; ++v)
+                for (int w = 0; w < N; ++w) {
+                    uint16_t h, l;
+                    split_bf16(dct_coef(v, w, N), h, l);
+                    const int row = gI * Ms + v, k = gI * N + w;          // element k of the row sits in half (k & 1) of packed column k / 2
+                    ahi[row * 64 + k / 2] |= static_cast<uint32_t>(h) << (16 * (k & 1));
+                    alo[row * 64 + k / 2] |= static_cast<uint32_t>(l) << (16 * (k & 1));
+                }
+        for (int rep = 0; rep < (Ms == 8 ? 2 : 1); ++rep)           // Ms = 8: two maps share a 16-column stage-2 group -> I_2 (x) C_N
+            for (int u = 0; u < N; ++u)
+                for (int h = 0; h < N; ++h) split_bf16(dct_coef(u, h, N), chi[(rep * 8 + u) * 64 + rep * 8 + h], clo[(rep * 8 + u) * 64 + rep * 8 + h]);
+        b.vpe = (N % 4 == 0) ? 1 : (N % 2 == 0) ? 2 : 4;
+        b.tile_vec = G * J * NN / 4;
+        const int step = 4 / b.vpe;
+        std::vector<uint16_t> tab(static_cast<size_t>(b.tile_vec) * b.vpe + 8, 0);
+        for (int v = 0; v < b.tile_vec; ++v)
+            for (int sI = 0; sI < b.vpe; ++sI) {               // map t = (g, j) of the tile: operand row (j, h), contraction column (g, w)
+                const int e = 4 * v + sI * step, t = e / NN, r = e % NN, gI = t / J, j = t % J;
+                tab[(size_t)v * b.vpe + sI] = static_cast<uint16_t>(detail::kmajor_off(j * Ms + r / N, gI * N + r % N, rows));
             }
-    for (int rep = 0; rep < (Ms == 8 ? 2 : 1); ++rep)           // Ms = 8: two maps share a 16-column stage-2 group -> I_2 (x) C_N
-        for (int u = 0; u < N; ++u)
-            for (int h = 0; h < N; ++h) split_bf16(dct_coef(u, h, N), chi[(rep * 8 + u) * 64 + rep * 8 + h], clo[(rep * 8 + u) * 64 + rep * 8 + h]);
-    TBasis b;
-    b.vpe = (N % 4 == 0) ? 1 : (N % 2 == 0) ? 2 : 4;
-    b.tile_vec = G * J * NN / 4;
-    const int step = 4 / b.vpe;
-    std::vector<uint16_t> tab(static_cast<size_t>(b.tile_vec) * b.vpe + 8, 0);
-    for (int v = 0; v < b.tile_vec; ++v)
-        for (int sI = 0; sI < b.vpe; ++sI) {               // map t = (g, j) of the tile: operand row (j, h), contraction column (g, w)
-            const int e = 4 * v + sI * step, t = e / NN, r = e % NN, gI = t / J, j = t % J;
-            tab[(size_t)v * b.vpe + sI] = static_cast<uint16_t>(detail::kmajor_off(j * Ms + r / N, gI * N + r % N, rows));
-        }
-    int rc;
-    if ((rc = upload(ahi, b.a_hi)) || (rc = upload(alo, b.a_lo)) || (rc = upload(chi, b.c_hi)) || (rc = upload(clo, b.c_lo)) ||
-        (rc = upload(tab, b.scatter)))
-        return rc;
-    g.tmem[N] = b;
-    out = b;
-    return DCTP_OK;
+        int rc;
+        if ((rc = upload(ahi, b.a_hi)) || (rc = upload(alo, b.a_lo)) || (rc = upload(chi, b.c_hi)) || (rc = upload(clo, b.c_lo)) ||
+            (rc = upload(tab, b.scatter)))
+            return rc;
+        return DCTP_OK;
+    });
 }
 
 // ------------------------------------------------------------------ stacked-basis kernel (score_stack.cuh)
@@ -215,86 +244,82 @@ inline int stack_g(int kp) { return kp == 16 ? 8 : kp == 32 ? 4 : 2; }
 bool stack_shape_supported(int N) { return N >= 10 && N <= 64 && (N % 2) == 0 && (N <= 32 || (N % 4) == 0); }
 
 int get_stack_basis(int N, StackBasis& out) {
-    auto it = g.stack.find(N);
-    if (it != g.stack.end()) { out = it->second; return DCTP_OK; }
-    using S = StackSmem;
-    const int KP = stack_kp(N), J = stack_sets(KP), G = stack_g(KP), NN = N * N, Np = (N + 7) / 8 * 8, MT = G * J;
-    std::vector<uint32_t> img(128 * 32, 0);
-    for (int lane = 0; lane < 128; ++lane) {
-        const int q = lane >> 5, part = (lane >> 4) & 1, r = lane & 15;
-        const int set = J == 4 ? q : J == 2 ? q >> 1 : 0;
-        const int v = J == 4 ? r : J == 2 ? 16 * (q & 1) + r : 16 * q + r;
-        if (v >= N) continue;
-        for (int w = 0; w < N; ++w) {
-            uint16_t h, l;
-            split_bf16(dct_coef(v, w, N), h, l);
-            const int k = set * KP + w;
-            img[lane * 32 + k / 2] |= static_cast<uint32_t>(part ? l : h) << (16 * (k & 1));
-        }
-    }
-    // folded stage 2 (stack_folded): rows h < fd of a map are paired with rows N-1-h, the middle rows [fd, N - fd) (Np / 8 odd) are not
-    const bool folded = stack_folded(KP);
-    const int fd = 8 * (Np / 16), fold = std::min(N / 2, fd);
-    // stage-2 basis: C_N[u][h] unfolded; folded, chain c (u = 2 u' + c) in rows [c W2, (c + 1) W2): C_N[2 u' + c][k] at contraction
-    // column k < N - fold (the paired rows' h, then the middle rows' h)
-    std::vector<uint8_t> chi(S::C2_HALF, 0), clo(S::C2_HALF, 0);
-    for (int u = 0; u < N; ++u)
-        for (int h = 0; h < (folded ? N - fold : N); ++h) {
-            uint16_t hh, ll;
-            split_bf16(dct_coef(u, h, N), hh, ll);
-            const int row = folded ? (u & 1) * stack_fold_k(KP) + u / 2 : u;
-            const size_t off = static_cast<size_t>(h / 8) * S::LBO2 + row * 16 + (h % 8) * 2;
-            std::memcpy(&chi[off], &hh, 2);
-            std::memcpy(&clo[off], &ll, 2);
-        }
-    // Bx row (= D1 column) of row h of a map: h unfolded; folded, row N-1-h' (h' < fold) at fd + h', so that each thread of epilogue 1
-    // holds both rows of a pair, and the middle rows from 2 fd on
-    auto bx_row = [&](int h) { return !folded || h < fold ? h : h >= N - fold ? fd + (N - 1 - h) : 2 * fd + (h - fold); };
-    StackBasis b;
-    b.kp = KP;
-    b.vec = (N % 4) == 0 ? 4 : 2;
-    b.tile_vec = MT * NN / 4;
-    const int pieces = b.vec == 4 ? 1 : 2;
-    std::vector<uint16_t> tab(static_cast<size_t>(b.tile_vec) * pieces + 8, 0);
-    auto fill = [&](uint32_t lbo) {
-        for (int f = 0; f < b.tile_vec; ++f)
-            for (int pc = 0; pc < pieces; ++pc) {
-                const int e = 4 * f + 2 * pc, m = e / NN, rem = e % NN, h = rem / N, w = rem % N, gI = m / J, set = m % J;
-                const int n = gI * Np + bx_row(h), k = set * KP + w;
-                tab[static_cast<size_t>(f) * pieces + pc] = static_cast<uint16_t>((k / 8) * lbo + n * 16 + (k % 8) * 2);
+    return cached(g.stack, N, out, [&](StackBasis& b) {
+        const int KP = stack_kp(N), J = stack_sets(KP), G = stack_g(KP), NN = N * N, Np = (N + 7) / 8 * 8, MT = G * J;
+        std::vector<uint32_t> img(128 * 32, 0);
+        for (int lane = 0; lane < 128; ++lane) {
+            const int q = lane >> 5, part = (lane >> 4) & 1, r = lane & 15;
+            const int set = J == 4 ? q : J == 2 ? q >> 1 : 0;
+            const int v = J == 4 ? r : J == 2 ? 16 * (q & 1) + r : 16 * q + r;
+            if (v >= N) continue;
+            for (int w = 0; w < N; ++w) {
+                uint16_t h, l;
+                split_bf16(dct_coef(v, w, N), h, l);
+                const int k = set * KP + w;
+                img[lane * 32 + k / 2] |= static_cast<uint32_t>(part ? l : h) << (16 * (k & 1));
             }
-    };
-    // shared-memory wavefronts of the converters' stores (thread t of a warp stores the pieces of vector f0 + t: 8-byte stores
-    // are served per half-warp, 4-byte stores per warp) for a given chunk distance: pick the bank spread with the fewest
-    auto store_wavefronts = [&]() {
-        long long total = 0;
-        const int width = b.vec == 4 ? 2 : 1, lanes = b.vec == 4 ? 16 : 32;      // banks per store, threads per phase
-        for (int f0 = 0; f0 < b.tile_vec; f0 += lanes)
-            for (int pc = 0; pc < pieces; ++pc) {
-                int cnt[32] = {0}, worst = 0;
-                for (int t = 0; t < lanes && f0 + t < b.tile_vec; ++t)
-                    for (int w = 0; w < width; ++w) {
-                        const int bank = (tab[static_cast<size_t>(f0 + t) * pieces + pc] / 4 + w) % 32;
-                        if (++cnt[bank] > worst) worst = cnt[bank];
-                    }
-                total += worst;
+        }
+        // folded stage 2 (stack_folded): rows h < fd of a map are paired with rows N-1-h, the middle rows [fd, N - fd) (Np / 8 odd) are not
+        const bool folded = stack_folded(KP);
+        const int fd = 8 * (Np / 16), fold = std::min(N / 2, fd);
+        // stage-2 basis: C_N[u][h] unfolded; folded, chain c (u = 2 u' + c) in rows [c W2, (c + 1) W2): C_N[2 u' + c][k] at contraction
+        // column k < N - fold (the paired rows' h, then the middle rows' h)
+        std::vector<uint8_t> chi(OperandImage64::BYTES, 0), clo(OperandImage64::BYTES, 0);
+        for (int u = 0; u < N; ++u)
+            for (int h = 0; h < (folded ? N - fold : N); ++h) {
+                uint16_t hh, ll;
+                split_bf16(dct_coef(u, h, N), hh, ll);
+                const int row = folded ? (u & 1) * stack_fold_k(KP) + u / 2 : u;
+                const size_t off = static_cast<size_t>(h / 8) * OperandImage64::LBO + row * 16 + (h % 8) * 2;
+                std::memcpy(&chi[off], &hh, 2);
+                std::memcpy(&clo[off], &ll, 2);
             }
-        return total;
-    };
-    long long best = -1;
-    for (uint32_t u = 0; u < 8; ++u) {
-        fill(2048u + 16u * u);
-        const long long wf = store_wavefronts();
-        if (best < 0 || wf < best) { best = wf; b.lbo1 = 2048u + 16u * u; }
-    }
-    fill(b.lbo1);
-    b.table_bytes = static_cast<uint32_t>((static_cast<size_t>(b.tile_vec) * pieces * 2 + 15) / 16 * 16);
-    if (b.table_bytes > S::TABLE_MAX) return fail(DCTP_E_UNSUPPORTED, "stacked-basis kernel: offset table of side %d does not fit", N);
-    int rc;
-    if ((rc = upload(img, b.a_img)) || (rc = upload(chi, b.c2_hi)) || (rc = upload(clo, b.c2_lo)) || (rc = upload(tab, b.table))) return rc;
-    g.stack[N] = b;
-    out = b;
-    return DCTP_OK;
+        // Bx row (= D1 column) of row h of a map: h unfolded; folded, row N-1-h' (h' < fold) at fd + h', so that each thread of epilogue 1
+        // holds both rows of a pair, and the middle rows from 2 fd on
+        auto bx_row = [&](int h) { return !folded || h < fold ? h : h >= N - fold ? fd + (N - 1 - h) : 2 * fd + (h - fold); };
+        b.kp = KP;
+        b.vec = (N % 4) == 0 ? 4 : 2;
+        b.tile_vec = MT * NN / 4;
+        const int pieces = b.vec == 4 ? 1 : 2;
+        std::vector<uint16_t> tab(static_cast<size_t>(b.tile_vec) * pieces + 8, 0);
+        auto fill = [&](uint32_t lbo) {
+            for (int f = 0; f < b.tile_vec; ++f)
+                for (int pc = 0; pc < pieces; ++pc) {
+                    const int e = 4 * f + 2 * pc, m = e / NN, rem = e % NN, h = rem / N, w = rem % N, gI = m / J, set = m % J;
+                    const int n = gI * Np + bx_row(h), k = set * KP + w;
+                    tab[static_cast<size_t>(f) * pieces + pc] = static_cast<uint16_t>((k / 8) * lbo + n * 16 + (k % 8) * 2);
+                }
+        };
+        // shared-memory wavefronts of the converters' stores (thread t of a warp stores the pieces of vector f0 + t: 8-byte stores
+        // are served per half-warp, 4-byte stores per warp) for a given chunk distance: pick the bank spread with the fewest
+        auto store_wavefronts = [&]() {
+            long long total = 0;
+            const int width = b.vec == 4 ? 2 : 1, lanes = b.vec == 4 ? 16 : 32;      // banks per store, threads per phase
+            for (int f0 = 0; f0 < b.tile_vec; f0 += lanes)
+                for (int pc = 0; pc < pieces; ++pc) {
+                    int cnt[32] = {0}, worst = 0;
+                    for (int t = 0; t < lanes && f0 + t < b.tile_vec; ++t)
+                        for (int w = 0; w < width; ++w) {
+                            const int bank = (tab[static_cast<size_t>(f0 + t) * pieces + pc] / 4 + w) % 32;
+                            if (++cnt[bank] > worst) worst = cnt[bank];
+                        }
+                    total += worst;
+                }
+            return total;
+        };
+        long long best = -1;
+        for (uint32_t u = 0; u < 8; ++u) {
+            fill(2048u + 16u * u);
+            const long long wf = store_wavefronts();
+            if (best < 0 || wf < best) { best = wf; b.lbo1 = 2048u + 16u * u; }
+        }
+        fill(b.lbo1);
+        b.table_bytes = static_cast<uint32_t>((static_cast<size_t>(b.tile_vec) * pieces * 2 + 15) / 16 * 16);
+        if (b.table_bytes > StackSmem::TABLE_MAX) return fail(DCTP_E_UNSUPPORTED, "stacked-basis kernel: offset table of side %d does not fit", N);
+        int rc;
+        if ((rc = upload(img, b.a_img)) || (rc = upload(chi, b.c2_hi)) || (rc = upload(clo, b.c2_lo)) || (rc = upload(tab, b.table))) return rc;
+        return DCTP_OK;
+    });
 }
 
 // instantiations: variant v = (KP, VEC, Np / 8) - (16,4,2) (16,2,2) (32,4,3) (32,4,4) (32,2,3) (32,2,4) (48,4,5) (48,4,6) (64,4,7) (64,4,8);
@@ -334,6 +359,8 @@ StackKernel stack_kernel_fn(bool debug, int v, int in) {
     return in == IN_BF16 ? stack_kernel_in<IN_BF16>(debug, v) : in == IN_F16 ? stack_kernel_in<IN_F16>(debug, v) : stack_kernel_in<IN_F32>(debug, v);
 }
 const char* in_name(int in) { return in == IN_BF16 ? "bf16" : in == IN_F16 ? "f16" : "f32"; }
+// what a 16-bit instantiation adds to its template arguments in dctp_last_kernel()
+const char* in_suffix(int in) { return in == IN_BF16 ? ",IN=bf16" : in == IN_F16 ? ",IN=f16" : ""; }
 int stack_variant(int KP, int vec, int np8) {
     if (KP == 16) return vec == 4 ? 0 : 1;
     if (KP == 32) return (vec == 4 ? 2 : 4) + (np8 == 4 ? 1 : 0);
@@ -392,8 +419,9 @@ cudaError_t launch_pdl(void (*kern)(Params...), int grid, int block, size_t smem
 
 struct SiteDesc { const void* first; int B; int c_count; double* accum; };      // one dense activation: B * c_count maps back to back
 
-// fills seg (tile ranges, per-site sizes); returns the launch's tile count
-int fill_segments(ScoreSegments& seg, const SiteDesc* sites, int n, int NN, int maps_per_tile) {
+// fills seg (tile ranges, per-site sizes); returns the launch's tile count.  A map is items_per_map work items (score_large.cuh:
+// its v-chunks), and a tile holds up to `per_tile` of them.
+int fill_segments(ScoreSegments& seg, const SiteDesc* sites, int n, int NN, int items_per_map, int per_tile) {
     seg.n_seg = n;
     int tiles = 0;
     for (int i = 0; i < n; ++i) {
@@ -403,10 +431,19 @@ int fill_segments(ScoreSegments& seg, const SiteDesc* sites, int n, int NN, int 
         seg.total_elems[i] = static_cast<long long>(seg.n_maps[i]) * NN;
         seg.x[i] = sites[i].first;
         seg.accum[i] = sites[i].accum;
-        tiles += (seg.n_maps[i] + maps_per_tile - 1) / maps_per_tile;
+        tiles += (seg.n_maps[i] * items_per_map + per_tile - 1) / per_tile;
     }
     for (int i = n; i <= SCORE_MAX_SEG; ++i) seg.tile0[i] = tiles;
     return tiles;
+}
+
+// the tensor maps of a multi-site launch: encode(i, map) for each of the n sites, the unused entries copies of the first
+template <class Encode>
+int fill_maps(ScoreTensorMaps& maps, int n, Encode encode) {
+    for (int i = 0; i < n; ++i)
+        if (int rc = encode(i, maps.m[i])) return rc;
+    for (int i = n; i < SCORE_MAX_SEG; ++i) maps.m[i] = maps.m[0];
+    return DCTP_OK;
 }
 
 // up to SCORE_MAX_SEG dense activations of side N in ONE launch (energy_out / coeff_out: single-site launches only)
@@ -420,40 +457,28 @@ int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* 
     a.N = N; a.NN = N * N; a.Np = (N + 7) / 8 * 8; a.G = stack_g(KP); a.MT = a.G * J;
     a.ncols = a.G * a.Np;
     a.tile_elems = a.MT * a.NN; a.tile_rows = a.tile_elems / 32; a.tile_vec = basis.tile_vec;
-    a.num_tiles = fill_segments(a.seg, sites, n, a.NN, a.MT);
+    a.num_tiles = fill_segments(a.seg, sites, n, a.NN, 1, a.MT);
     a.idesc1 = umma::make_idesc_bf16(128, a.ncols, false, false);
     a.idesc2 = umma::make_idesc_bf16(128, stack_folded(KP) ? stack_fold_k(KP) : KP, false, false);
     a.lbo1 = basis.lbo1;
     a.a_img = basis.a_img; a.c2_hi = basis.c2_hi; a.c2_lo = basis.c2_lo; a.table = basis.table; a.table_bytes = basis.table_bytes;
     a.energy_out = n == 1 ? energy_out : nullptr; a.dump = n == 1 ? coeff_out : nullptr; a.status = g.status;
     ScoreTensorMaps maps;
-    for (int i = 0; i < n; ++i)
-        if ((rc = encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.tile_rows, in))) return rc;
-    for (int i = n; i < SCORE_MAX_SEG; ++i) maps.m[i] = maps.m[0];
+    if ((rc = fill_maps(maps, n, [&](int i, CUtensorMap& m) { return encode_flat_map(m, sites[i].first, a.seg.total_elems[i], a.tile_rows, in); })))
+        return rc;
     int grid = g.sm_count < a.num_tiles ? g.sm_count : a.num_tiles;
     const size_t smem = StackSmem::TOTAL;
-    const bool v4 = basis.vec == 4;
-    static long long* trace_buf = nullptr;
-    const bool tracing = std::getenv("DCTP_S_TRACE") != nullptr;
-    if (tracing) {
-        if (!trace_buf) CUDA_TRY(cudaMalloc(&trace_buf, 64 * sizeof(long long)));
-        CUDA_TRY(cudaMemset(trace_buf, 0, 64 * sizeof(long long)));
-        a.trace = trace_buf;
-    }
-    const int variant = stack_variant(KP, v4 ? 4 : 2, a.Np / 8);
+    if ((rc = trace_for("DCTP_S_TRACE", a.trace))) return rc;
+    const int variant = stack_variant(KP, basis.vec, a.Np / 8);
     // per-map energies, coefficients and the cycle trace live in the debug instantiation (cfg6) only
-    const bool debug = a.energy_out || a.dump || tracing;
+    const bool debug = a.energy_out || a.dump || a.trace;
     CUDA_TRY(launch_pdl(stack_kernel_fn(debug, variant, in), grid, 32 * stack_warps(debug ? STACK_NCONV_DEBUG : STACK_NCONV), smem, stream,
                         maps, a));
-    if (in == IN_F32)
-        note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP, basis.vec,
-                    debug ? 6 : 7);
-    else
-        note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d,IN=%s> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP,
-                    basis.vec, debug ? 6 : 7, in_name(in));
-    if (tracing) {
-        long long h[64];
-        CUDA_TRY(cudaMemcpy(h, trace_buf, sizeof h, cudaMemcpyDeviceToHost));
+    note_kernel("score_stack_kernel<KP=%d,VEC=%d,cfg%d%s> (tcgen05, stacked hi/lo basis in TMEM, TMA tile ring, warp specialised)", KP, basis.vec,
+                debug ? 6 : 7, in_suffix(in));
+    if (a.trace) {
+        long long h[TRACE_LEN];
+        if ((rc = read_trace(h))) return rc;
         const double nt = h[14] > 0 ? double(h[14]) : 1.0;
         fprintf(stderr, "[dctp trace] stack N=%d, CTA 0, %lld tiles, cycles per tile | producer: wait slot %.0f | converter: wait Bx free %.0f, "
                         "wait TMA %.0f, convert %.0f, fence+arrive %.0f | issuer 1: wait Bx %.0f, wait D1 free %.0f, issue %.0f | issuer 2: wait A2 %.0f, "
@@ -465,34 +490,28 @@ int launch_stack(const SiteDesc* sites, int n, int N, float* energy_out, float* 
         fprintf(stderr, "[dctp trace] tile loop of CTA 0: %lld SM cycles in %lld ns = %.0f MHz, %.0f cycles per tile\n", h[50], h[51],
                 h[51] > 0 ? 1e3 * double(h[50]) / double(h[51]) : 0.0, double(h[50]) / nt);
     }
-    g.launches += 1;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 // ------------------------------------------------------------------ Kronecker kernel (score_kron.cuh), sides 1..8
 int get_kron_basis(int N, KronBasis& out) {
-    auto it = g.kron.find(N);
-    if (it != g.kron.end()) { out = it->second; return DCTP_OK; }
-    using S = StackSmem;
-    std::vector<uint8_t> hi(S::C2_HALF, 0), lo(S::C2_HALF, 0);
-    for (int u = 0; u < N; ++u)
-        for (int v = 0; v < N; ++v)
-            for (int h = 0; h < N; ++h)
-                for (int w = 0; w < N; ++w) {
-                    uint16_t hh, ll;
-                    split_bf16(dct_coef(u, h, N) * dct_coef(v, w, N), hh, ll);
-                    const int n = u * N + v, k = h * N + w;
-                    const size_t off = static_cast<size_t>(k / 8) * S::LBO2 + n * 16 + (k % 8) * 2;
-                    std::memcpy(&hi[off], &hh, 2);
-                    std::memcpy(&lo[off], &ll, 2);
-                }
-    KronBasis b;
-    int rc;
-    if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
-    g.kron[N] = b;
-    out = b;
-    return DCTP_OK;
+    return cached(g.kron, N, out, [&](KronBasis& b) {
+        std::vector<uint8_t> hi(OperandImage64::BYTES, 0), lo(OperandImage64::BYTES, 0);
+        for (int u = 0; u < N; ++u)
+            for (int v = 0; v < N; ++v)
+                for (int h = 0; h < N; ++h)
+                    for (int w = 0; w < N; ++w) {
+                        uint16_t hh, ll;
+                        split_bf16(dct_coef(u, h, N) * dct_coef(v, w, N), hh, ll);
+                        const int n = u * N + v, k = h * N + w;
+                        const size_t off = static_cast<size_t>(k / 8) * OperandImage64::LBO + n * 16 + (k % 8) * 2;
+                        std::memcpy(&hi[off], &hh, 2);
+                        std::memcpy(&lo[off], &ll, 2);
+                    }
+        int rc;
+        if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
+        return DCTP_OK;
+    });
 }
 
 typedef void (*KronKernel)(const ScoreTensorMaps, const KronArgs);
@@ -546,27 +565,21 @@ int launch_kron(const SiteDesc* sites, int n, int N, float* energy_out, float* c
         a.box_rows = a.tile_maps * NN / 32;
         a.tile_bytes = static_cast<uint32_t>(a.box_rows) * 32u * eb;
     }
-    a.num_tiles = fill_segments(a.seg, sites, n, NN, a.tile_maps);
+    a.num_tiles = fill_segments(a.seg, sites, n, NN, 1, a.tile_maps);
     ScoreTensorMaps maps;
-    for (int i = 0; i < n; ++i) {
-        // even sides: one map per row of the box, padded to row_elems; odd sides: the flat stream
-        rc = even ? encode_2d(maps.m[i], sites[i].first, NN, a.seg.n_maps[i], static_cast<long long>(eb) * NN, a.row_elems, a.tile_maps,
-                              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, in)
-                  : encode_flat_map(maps.m[i], sites[i].first, a.seg.total_elems[i], a.box_rows, in);
-        if (rc) return rc;
-    }
-    for (int i = n; i < SCORE_MAX_SEG; ++i) maps.m[i] = maps.m[0];
+    // even sides: one map per row of the box, padded to row_elems; odd sides: the flat stream
+    rc = fill_maps(maps, n, [&](int i, CUtensorMap& m) {
+        return even ? encode_2d(m, sites[i].first, NN, a.seg.n_maps[i], static_cast<long long>(eb) * NN, a.row_elems, a.tile_maps,
+                                CU_TENSOR_MAP_L2_PROMOTION_L2_128B, in)
+                    : encode_flat_map(m, sites[i].first, a.seg.total_elems[i], a.box_rows, in);
+    });
+    if (rc) return rc;
     const int grid = g.sm_count < a.num_tiles ? g.sm_count : a.num_tiles;
     const size_t smem = KronSmem::TOTAL;
     CUDA_TRY(launch_pdl(kron_kernel_fn(K2, even, in), grid, KRON_NT, smem, stream, maps, a));
-    if (in == IN_F32)
-        note_kernel("score_kron_kernel<K2=%d,%s> (tcgen05, single-stage Kronecker, TMA tile ring, warp specialised)", K2, even ? "even" : "odd");
-    else
-        note_kernel("score_kron_kernel<K2=%d,%s,IN=%s> (tcgen05, single-stage Kronecker, TMA tile ring, warp specialised)", K2,
-                    even ? "even" : "odd", in_name(in));
-    g.launches += 1;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    note_kernel("score_kron_kernel<K2=%d,%s%s> (tcgen05, single-stage Kronecker, TMA tile ring, warp specialised)", K2, even ? "even" : "odd",
+                in_suffix(in));
+    return launched();
 }
 
 // stage-2 output chunks of the large-map kernel: NUC chunks of NU columns (multiple of 16, at most 128: one basis slab)
@@ -576,47 +589,47 @@ void large_u_chunks(int N, int& nu, int& nuc) {
 }
 
 int get_large_basis(int N, LargeBasis& out) {
-    auto it = g.large.find(N);
-    if (it != g.large.end()) { out = it->second; return DCTP_OK; }
-    LargeBasis b;
-    b.NP = (N + 63) / 64 * 64;
-    // operand image: [column block cb][row k][64 columns], the eight 16-byte chunks of a row XOR-swizzled by (k & 7);
-    // rows padded so that every u-chunk slab of the kernel stays inside its column block
-    int nu, nuc;
-    large_u_chunks(N, nu, nuc);
-    b.NPR = b.NP > nu * nuc ? b.NP : nu * nuc;
-    std::vector<uint16_t> hi(static_cast<size_t>(b.NP / 64) * b.NPR * 64, 0), lo(hi.size(), 0);
-    for (int k = 0; k < N; ++k)
-        for (int n = 0; n < N; ++n) {
-            const size_t at = (static_cast<size_t>(n >> 6) * b.NPR + k) * 64 + ((((n & 63) >> 3) ^ (k & 7)) << 3) + (n & 7);
-            split_bf16(dct_coef(k, n, N), hi[at], lo[at]);
-        }
-    int rc;
-    if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
-    g.large[N] = b;
-    out = b;
-    return DCTP_OK;
+    return cached(g.large, N, out, [&](LargeBasis& b) {
+        b.NP = (N + 63) / 64 * 64;
+        // operand image: [column block cb][row k][64 columns], the eight 16-byte chunks of a row XOR-swizzled by (k & 7);
+        // rows padded so that every u-chunk slab of the kernel stays inside its column block
+        int nu, nuc;
+        large_u_chunks(N, nu, nuc);
+        b.NPR = b.NP > nu * nuc ? b.NP : nu * nuc;
+        std::vector<uint16_t> hi(static_cast<size_t>(b.NP / 64) * b.NPR * 64, 0), lo(hi.size(), 0);
+        for (int k = 0; k < N; ++k)
+            for (int n = 0; n < N; ++n) {
+                const size_t at = (static_cast<size_t>(n >> 6) * b.NPR + k) * 64 + ((((n & 63) >> 3) ^ (k & 7)) << 3) + (n & 7);
+                split_bf16(dct_coef(k, n, N), hi[at], lo[at]);
+            }
+        int rc;
+        if ((rc = upload(hi, b.hi)) || (rc = upload(lo, b.lo))) return rc;
+        return DCTP_OK;
+    });
 }
 
 int get_simt_basis(int N, SimtBasis& out) {
-    auto it = g.simt.find(N);
-    if (it != g.simt.end()) { out = it->second; return DCTP_OK; }
-    std::vector<float> t(static_cast<size_t>(N) * N);
-    for (int n = 0; n < N; ++n)
-        for (int k = 0; k < N; ++k) t[(size_t)n * N + k] = static_cast<float>(dct_coef(k, n, N));
-    SimtBasis b;
-    if (int rc = upload(t, b.t)) return rc;
-    g.simt[N] = b;
-    out = b;
-    return DCTP_OK;
+    return cached(g.simt, N, out, [&](SimtBasis& b) {
+        std::vector<float> t(static_cast<size_t>(N) * N);
+        for (int n = 0; n < N; ++n)
+            for (int k = 0; k < N; ++k) t[(size_t)n * N + k] = static_cast<float>(dct_coef(k, n, N));
+        return upload(t, b.t);
+    });
 }
 
 // ------------------------------------------------------------------ init
+// fn may use `bytes` of dynamic shared memory, and prefers the largest shared-memory carveout
+template <class F>
+int allow_smem(F* fn, int bytes) {
+    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    return DCTP_OK;
+}
+
 template <int KP, int MODE, bool PF>
 int setup_umma(int& regs) {
     auto* fn = score_umma_kernel<KP, MODE, PF>;
-    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, KP == 64 ? 100 * 1024 : 200 * 1024));
-    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    if (int rc = allow_smem(fn, KP == 64 ? 100 * 1024 : 200 * 1024)) return rc;
     cudaFuncAttributes fa;
     CUDA_TRY(cudaFuncGetAttributes(&fa, fn));
     regs = fa.numRegs;
@@ -679,26 +692,18 @@ int ensure_init() {
         const void* fns[] = {reinterpret_cast<const void*>(score_t_kernel<64, 3, 1>), reinterpret_cast<const void*>(score_t_kernel<64, 3, 2>),
                              reinterpret_cast<const void*>(score_t_kernel<32, 6, 1>), reinterpret_cast<const void*>(score_t_kernel<32, 6, 2>),
                              reinterpret_cast<const void*>(score_t_kernel<32, 6, 4>), reinterpret_cast<const void*>(score_t_kernel<64, 3, 1, 2>)};
-        for (const void* fn : fns) {
-            CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-            CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-        }
+        for (const void* fn : fns)
+            if ((rc = allow_smem(fn, 227 * 1024))) return rc;
     }
     {
         for (const int in : {IN_F32, IN_BF16, IN_F16}) {
             for (const bool debug : {false, true})
-                for (int v = 0; v < STACK_VARIANTS; ++v) {
-                    const void* fn = reinterpret_cast<const void*>(stack_kernel_fn(debug, v, in));
-                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(StackSmem::TOTAL)));
-                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                }
+                for (int v = 0; v < STACK_VARIANTS; ++v)
+                    if ((rc = allow_smem(stack_kernel_fn(debug, v, in), static_cast<int>(StackSmem::TOTAL)))) return rc;
             for (const int k2 : {16, 32, 48, 64})
-                for (const bool even : {true, false}) {
-                    if (!kron_kernel_built(k2, even, in)) continue;
-                    const void* fn = reinterpret_cast<const void*>(kron_kernel_fn(k2, even, in));
-                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(KronSmem::TOTAL)));
-                    CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-                }
+                for (const bool even : {true, false})
+                    if (kron_kernel_built(k2, even, in) && (rc = allow_smem(kron_kernel_fn(k2, even, in), static_cast<int>(KronSmem::TOTAL))))
+                        return rc;
         }
         cudaDriverEntryPointQueryResult qres;
         CUDA_TRY(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &g.encode_tiled, cudaEnableDefault, &qres));
@@ -738,7 +743,7 @@ int pick_vec(const float* x, long long stride_b, long long stride_c, int N) {
 // instructions), 96 1.22 vs 0.73
 bool large_shape_supported(int H, int W, long long stride_h) { return H == W && H >= 80 && H <= 320 && (H % 16) == 0 && stride_h == W; }
 
-// up to LARGE_MAX_SEG dense activations of side N in ONE launch (energy_out / coeff_out: single-site launches only)
+// up to SCORE_MAX_SEG dense activations of side N in ONE launch (energy_out / coeff_out: single-site launches only)
 int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* coeff_out, cudaStream_t stream) {
     LargeBasis basis;
     int rc = get_large_basis(N, basis);
@@ -747,38 +752,27 @@ int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* 
     std::memset(&a, 0, sizeof a);
     a.N = N; a.NPR = basis.NPR; a.NVC = (N + 127) / 128;
     large_u_chunks(N, a.NU, a.NUC);
-    a.seg.n_seg = n;
     long long items = 0;
     for (int i = 0; i < n; ++i) {
         const long long maps = static_cast<long long>(sites[i].B) * sites[i].c_count;
         if (maps * N >= (1ll << 31) || items + maps * a.NVC >= (1ll << 31))
             return fail(DCTP_E_INVALID, "too many maps of side %d in one launch (tensor-map row coordinates and work-item numbers are 32-bit)", N);
-        a.seg.item0[i] = static_cast<int>(items);
-        a.seg.c_count[i] = sites[i].c_count;
-        a.seg.accum[i] = sites[i].accum;
         a.n_maps += static_cast<int>(maps);
         items += maps * a.NVC;
     }
-    for (int i = n; i <= LARGE_MAX_SEG; ++i) a.seg.item0[i] = static_cast<int>(items);
-    a.n_items = static_cast<int>(items);
+    a.n_items = fill_segments(a.seg, sites, n, N * N, a.NVC, 1);
     a.c_hi = reinterpret_cast<const uint8_t*>(basis.hi); a.c_lo = reinterpret_cast<const uint8_t*>(basis.lo);
     a.energy_out = n == 1 ? energy_out : nullptr; a.dump = n == 1 ? coeff_out : nullptr; a.status = g.status;
     energy_out = a.energy_out;
     if (energy_out) CUDA_TRY(cudaMallocAsync(&a.energy_parts, sizeof(float) * a.n_maps * a.NVC, stream));   // (debug / parity output only)
     int grid = g.sm_count < a.n_items ? g.sm_count : a.n_items;
-    static long long* trace_buf = nullptr;
-    const bool tracing = std::getenv("DCTP_L_TRACE") != nullptr;
-    if (tracing) {
-        if (!trace_buf) CUDA_TRY(cudaMalloc(&trace_buf, 16 * sizeof(long long)));
-        a.trace = trace_buf;
-    }
+    if ((rc = trace_for("DCTP_L_TRACE", a.trace))) return rc;
     // every activation as a 2-D tensor [n_maps * N rows, N floats]; a map slab is the box {64 floats, 128 rows}, out-of-range parts zero
-    LargeTensorMap xmap;
-    for (int i = 0; i < n; ++i)
-        if ((rc = encode_2d(xmap.m[i], sites[i].first, N, static_cast<long long>(sites[i].B) * sites[i].c_count * N, 4ll * N, 64, 128,
-                            CU_TENSOR_MAP_L2_PROMOTION_L2_256B)))
-            return rc;
-    for (int i = n; i < LARGE_MAX_SEG; ++i) xmap.m[i] = xmap.m[0];
+    ScoreTensorMaps xmap;
+    if ((rc = fill_maps(xmap, n, [&](int i, CUtensorMap& m) {
+             return encode_2d(m, sites[i].first, N, static_cast<long long>(a.seg.n_maps[i]) * N, 4ll * N, 64, 128, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+         })))
+        return rc;
     CUDA_TRY(launch_pdl((a.trace || a.dump) ? score_large_kernel<true> : score_large_kernel<false>, grid, LARGE_NT, LargeSmem::TOTAL, stream,
                         xmap, a));
     if (energy_out) {
@@ -786,9 +780,9 @@ int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* 
         CUDA_TRY(cudaFreeAsync(a.energy_parts, stream));
     }
     note_kernel("score_large_kernel (tcgen05, tiled two-stage, TMA-staged map slabs, 19 warps)");
-    if (tracing) {
-        long long h[16];
-        CUDA_TRY(cudaMemcpy(h, trace_buf, sizeof h, cudaMemcpyDeviceToHost));
+    if (a.trace) {
+        long long h[TRACE_LEN];
+        if ((rc = read_trace(h))) return rc;
         const double n = h[7] > 0 ? double(h[7]) : 1.0;
         fprintf(stderr, "[dctp trace] large N=%d steps=%lld, issuer thread cycles/step: total %.0f | waiting for: map slab %.0f, "
                         "basis slab %.0f (+%.0f look-ahead), A2 %.0f, D2 free %.0f\n",
@@ -797,9 +791,7 @@ int launch_large(const SiteDesc* sites, int n, int N, float* energy_out, float* 
         fprintf(stderr, "[dctp trace] converter thread 0, cycles per map slab (%lld slabs): operand buffer wait %.0f, staged slab wait %.0f, "
                         "convert + store + hand-over %.0f\n", h[12], h[8] / m, h[11] / m, h[9] / m);
     }
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 // which maps the TMEM-operand kernel takes at all (dense; side 5..64, odd sides up to 13 and only when the whole stream is a
@@ -848,13 +840,7 @@ int launch_t(const float* first, int B, int N, int c_count, double* accum, float
     a.scatter = basis.scatter; a.scatter_bytes = static_cast<uint32_t>(basis.tile_vec) * basis.vpe * 2u;
     a.a_hi = basis.a_hi; a.a_lo = basis.a_lo; a.c_hi = basis.c_hi; a.c_lo = basis.c_lo;
     a.accum = accum; a.energy_out = energy_out; a.dump = coeff_out; a.status = g.status;
-    static long long* trace_buf = nullptr;
-    const bool tracing = std::getenv("DCTP_T_TRACE") != nullptr;
-    if (tracing) {
-        if (!trace_buf) CUDA_TRY(cudaMalloc(&trace_buf, 256 * sizeof(long long)));
-        CUDA_TRY(cudaMemset(trace_buf, 0, 256 * sizeof(long long)));
-        a.trace = trace_buf;
-    }
+    if ((rc = trace_for("DCTP_T_TRACE", a.trace))) return rc;
     a.div_ms.set(a.Ms);
     const int n1max = t_n1max(N), ns = n1max == 64 ? 3 : 6;
     const size_t smem = n1max == 64 ? TScoreSmem<64>::total(ns, a.scatter_bytes) : TScoreSmem<32>::total(ns, a.scatter_bytes);
@@ -878,9 +864,9 @@ int launch_t(const float* first, int B, int N, int c_count, double* accum, float
     }
     note_kernel("score_t_kernel<%d,%d,VPE=%d%s> (tcgen05, block-diagonal basis in TMEM)", n1max, ns, basis.vpe,
                 producers ? ",2 producer warpgroups" : "");
-    if (tracing) {
-        long long h[256];
-        CUDA_TRY(cudaMemcpy(h, trace_buf, sizeof h, cudaMemcpyDeviceToHost));
+    if (a.trace) {
+        long long h[TRACE_LEN];
+        if ((rc = read_trace(h))) return rc;
         const char* names[7] = {"convert", "fence+bar", "issue1+prefetch", "wait1", "epi1+bar", "issue2+wait2", "epi2+reduce"};
         double sum[7] = {0}; int n = 0; double gap = 0;
         for (int t = 2; t < 32 && h[t * 8 + 7]; ++t, ++n) {
@@ -894,9 +880,7 @@ int launch_t(const float* first, int B, int N, int c_count, double* accum, float
             fprintf(stderr, " loop-gap %.0f total %.0f\n", gap / n, tot + gap / n);
         }
     }
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 struct Call {                                            // the arguments of one dctp_score_accum_ex call
@@ -989,9 +973,7 @@ int launch_umma(const Call& c, cudaStream_t stream) {
         default: CUDA_TRY(launch_pdl(score_umma_kernel<KP, LOAD_GEN1, false>, grid, 128, smem, stream, a)); break;
     }
     note_kernel("score_umma_kernel<%d,%d,%d> (tcgen05 bf16x3, operands in shared memory)", KP, mode, pf ? 1 : 0);
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 int launch_simt(const Call& c, cudaStream_t stream) {
@@ -1020,9 +1002,7 @@ int launch_simt(const Call& c, cudaStream_t stream) {
         score_simt_large_kernel<<<grid, 256, smem, stream>>>(a);
         note_kernel("score_simt_large_kernel (fp32 CUDA cores)");
     }
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 // ------------------------------------------------------------------ routing
@@ -1062,7 +1042,6 @@ Call dense_call(int H, int W, long long stride_h) {
 }
 
 // the kernels that score up to SCORE_MAX_SEG activations in one launch
-static_assert(SCORE_MAX_SEG == LARGE_MAX_SEG, "one multi-site batch size");
 bool multi_site(Route r) { return r == R_KRON || r == R_STACK || r == R_LARGE; }
 // the kernels that read 16-bit input themselves; every other route scores a widened fp32 copy of the window (score_accum)
 bool reads_16bit(Route r) { return r == R_KRON || r == R_STACK; }
@@ -1102,7 +1081,7 @@ int dctp_shutdown(void) {
     std::lock_guard<std::mutex> lk(g_mu);
     if (!g.ready) return DCTP_OK;
     for (void* p : g.bases) cudaFree(p);
-    cudaFree(g.status); cudaFree(g.hx); cudaFree(g.hacc); cudaFree(g.hout);
+    cudaFree(g.status); cudaFree(g.trace); cudaFree(g.hx); cudaFree(g.hacc); cudaFree(g.hout);
     g = State();
     return DCTP_OK;
 }
@@ -1295,9 +1274,7 @@ static int dct3_energy(const float* x, int B, int H, int W, long long stride_b, 
     std::lock_guard<std::mutex> lk(g_mu);
     if (values_out) dct3_reduce_kernel<<<B, 256, 0, s>>>(energy, c_count, values_out, accum);
     else sum_to_one_kernel<<<1, 256, 0, s>>>(part, c_count, accum);
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 int dctp_score_op(int op, const float* x, int B, int H, int W, long long stride_b, long long stride_c, long long stride_h,
@@ -1341,10 +1318,8 @@ int dctp_score_op(int op, const float* x, int B, int H, int W, long long stride_
         const long long cap = static_cast<long long>(g.sm_count) * 32;
         if (blocks > cap) blocks = cap;
         rank_jacobi_kernel<<<static_cast<unsigned>(blocks), threads, smem, s>>>(a);
-        ++g.launches;
         note_kernel("rank_jacobi_kernel (fp32 one-sided Jacobi SVD in shared memory, %d lanes per pair, %d maps per CTA)", L, a.G);
-        CUDA_TRY(cudaGetLastError());
-        return DCTP_OK;
+        return launched();
     }
     if (op != DCTP_OP_DCT3) return fail(DCTP_E_INVALID, "dctp_score_op: unknown op %d", op);
     // dct_3d energy of x[b, window] = sum over the window's channels of the 2-D energies (the channel-axis DCT is orthonormal)
@@ -1377,9 +1352,7 @@ int dctp_finalize(const double* accum, double n_images, float* out, int n, void*
     if (n < 0 || (n > 0 && (!accum || !out)) || !(n_images > 0)) return fail(DCTP_E_INVALID, "dctp_finalize: n=%d n_images=%g", n, n_images);
     if (n == 0) return DCTP_OK;
     finalize_kernel<<<(n + 255) / 256, 256, 0, static_cast<cudaStream_t>(stream)>>>(accum, n_images, out, n);
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 int dctp_topk_segmented(const float* scores, const int* seg_offsets, const int* seg_k, int n_seg, long long* out_idx,
@@ -1392,9 +1365,7 @@ int dctp_topk_segmented(const float* scores, const int* seg_offsets, const int* 
     if (n_seg == 0) return DCTP_OK;
     topk_segmented_kernel<<<n_seg, TOPK_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(scores, seg_offsets, seg_k, out_idx,
                                                                                          out_offsets);
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 int dctp_gather_weight(const float* w, int c_out, int c_in, int inner, const long long* sel_out, int k_out,
@@ -1419,9 +1390,7 @@ int dctp_gather_weight(const float* w, int c_out, int c_in, int inner, const lon
     const long long cap = static_cast<long long>(g.sm_count) * 16;
     if (blocks > cap) blocks = cap;
     gather_weight_kernel<<<static_cast<unsigned>(blocks), GATHER_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(a);
-    ++g.launches;
-    CUDA_TRY(cudaGetLastError());
-    return DCTP_OK;
+    return launched();
 }
 
 int dctp_check(void* stream) {

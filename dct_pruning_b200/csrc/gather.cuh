@@ -15,7 +15,7 @@
 namespace dctp {
 
 constexpr int GATHER_THREADS = 256;
-enum : int { DCTP_DEV_BAD_INDEX = 3 };         // (continues DCTP_DEV_* of score_umma.cuh)
+enum : int { DCTP_DEV_BAD_INDEX = 3 };         // (continues DCTP_DEV_* of score_common.cuh)
 
 struct GatherArgs {
     const float* w;                 // [c_out][c_in][inner]

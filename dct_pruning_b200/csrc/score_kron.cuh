@@ -24,13 +24,13 @@
 // 4 and 8 only (box width padded to an odd number of 16-byte units); every other side uses the flat [rows, 32 elements] view.  bf16
 // maps are their own hi part: A_lo is not written and the MMA issuer runs the hi*hi and hi*lo passes only; fp16 is split as fp32.
 #pragma once
-#include <cuda.h>
-#include "score_stack.cuh"
+#include "score_common.cuh"
+#include "umma.cuh"
 
 namespace dctp {
 
 struct KronArgs {
-    ScoreSegments seg;              // the activations of the launch (score_stack.cuh)
+    ScoreSegments seg;              // the activations of the launch
     int N, NN;
     int sub_tiles;                  // 128-map sub-tiles per TMA tile (1, 2 or 4)
     int row_elems;                  // shared-memory stride of a map's row in elements (EVEN: box width, ODD: NN)
@@ -38,7 +38,7 @@ struct KronArgs {
     uint32_t tile_bytes;            // bytes one TMA tile lands
     int box_rows;                   // second box dimension (EVEN: maps per tile, ODD: 128-byte rows per tile)
     uint32_t idesc;
-    const uint8_t* k_hi;            // Kr operand images (StackSmem::LBO2 layout)
+    const uint8_t* k_hi;            // Kr operand images (OperandImage64 layout)
     const uint8_t* k_lo;
     float* energy_out;              // optional, single-segment launches only
     float* dump;                    // optional, single-segment launches only
@@ -48,7 +48,7 @@ struct KronArgs {
 struct KronSmem {
     static constexpr uint32_t NSTG = 3, STG_STRIDE = 36 * 1024;
     static constexpr uint32_t OFF_K = NSTG * STG_STRIDE;
-    static constexpr uint32_t OFF_BARS = OFF_K + 2 * StackSmem::C2_HALF;
+    static constexpr uint32_t OFF_BARS = OFF_K + 2 * OperandImage64::BYTES;
     static constexpr uint32_t OFF_SLOT = OFF_BARS + 256;
     static constexpr uint32_t TOTAL = OFF_SLOT + 128;
 };
@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
     using S = KronSmem;
     using namespace umma;
     constexpr int KS = K2 / 16;
-    constexpr uint32_t LBO = StackSmem::LBO2, HALF = StackSmem::C2_HALF, STEP = (2 * LBO) >> 4;
+    constexpr uint32_t LBO = OperandImage64::LBO, HALF = OperandImage64::BYTES, STEP = (2 * LBO) >> 4;
     constexpr uint32_t TM_A = 0, TM_D = 256;
 
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -102,9 +102,6 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
 
     const int first = blockIdx.x, stride = gridDim.x;
     bool dead = false;
-    auto seg_of = [&](int tile, int& sg) {
-        while (tile >= a.seg.tile0[sg + 1]) ++sg;
-    };
     auto is_tail = [&](int tile, int sg) {               // (ODD) a stream that does not end on a 32-element row: last tile from global memory
         return !EVEN && tile == a.seg.tile0[sg + 1] - 1 && (a.seg.total_elems[sg] & 31) != 0;
     };
@@ -120,7 +117,7 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
             uint32_t it = 0;
             int sg = 0;
             for (int tile = first; tile < a.num_tiles; tile += stride) {
-                seg_of(tile, sg);
+                advance_segment(a.seg, tile, sg);
                 if (is_tail(tile, sg)) continue;
                 const uint32_t s = it % S::NSTG;
                 if (it >= S::NSTG) KRON_WAIT(stg_free + s, ((it / S::NSTG) - 1u) & 1u);
@@ -163,7 +160,7 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
         uint32_t it = 0, j = 0;
         int sg = 0;
         for (int tile = first; tile < a.num_tiles && !dead; tile += stride) {
-            seg_of(tile, sg);
+            advance_segment(a.seg, tile, sg);
             const bool from_global = is_tail(tile, sg);
             uint32_t s = 0;
             if (!from_global) {
@@ -288,7 +285,7 @@ __global__ void __launch_bounds__(KRON_NT, 1) score_kron_kernel(const __grid_con
         uint32_t j = 0;
         int sg = 0;
         for (int tile = first; tile < a.num_tiles && !dead; tile += stride) {
-            seg_of(tile, sg);
+            advance_segment(a.seg, tile, sg);
             const uint32_t C = static_cast<uint32_t>(a.seg.c_count[sg]), seg_maps = static_cast<uint32_t>(a.seg.n_maps[sg]);
             double* const accum = a.seg.accum[sg];
             for (int st = 0; st < a.sub_tiles; ++st, ++j) {

@@ -33,25 +33,13 @@
 //                                       No block-wide barrier inside the pipeline, only mbarriers.
 // One resident CTA of 19 warps per SM (226 KB of shared memory, 512 TMEM columns).
 #pragma once
-#include <cuda.h>
-#include "score_umma.cuh"
+#include "score_common.cuh"
+#include "umma.cuh"
 
 namespace dctp {
 
-constexpr int LARGE_MAX_SEG = 16;           // activations (hook sites of the same map side) one launch can score
-// one tensor map per activation of the launch: [n_maps * N rows, N floats], box {64, 128}
-struct LargeTensorMap { CUtensorMap m[LARGE_MAX_SEG]; };
-// The activations of a launch, all their scored maps back to back.  Work item i belongs to segment s with item0[s] <= i < item0[s + 1]
-// (every segment holds a whole number of NVC-item maps, so i % NVC is still the v-chunk).
-struct LargeSegments {
-    int n_seg;
-    int item0[LARGE_MAX_SEG + 1];
-    int c_count[LARGE_MAX_SEG];
-    double* accum[LARGE_MAX_SEG];
-};
-
 struct LargeScoreArgs {
-    LargeSegments seg;
+    ScoreSegments seg;              // the activations of the launch; a tile of the table is a work item (map, v-chunk)
     int n_maps;                     // all segments together
     int N, NPR;                     // map side; rows per column block of the basis image (>= N and >= NU * NUC, zero padded)
     int NVC;                        // v-chunks per map = ceil(N / 128)
@@ -91,7 +79,7 @@ constexpr int LARGE_NT = LARGE_CONV + 96;   // + the MMA issuer, basis producer 
 
 // TRACE: the cycle accounting of DCTP_L_TRACE and the coefficient dump; the production instantiation carries neither
 template <bool TRACE>
-__global__ void __launch_bounds__(LARGE_NT, 1) score_large_kernel(const __grid_constant__ LargeTensorMap xmap, const LargeScoreArgs a) {
+__global__ void __launch_bounds__(LARGE_NT, 1) score_large_kernel(const __grid_constant__ ScoreTensorMaps xmap, const LargeScoreArgs a) {
     constexpr int NC = LARGE_CONV;
     constexpr int XV = 2048 / NC;                                  // float4 per thread and map slab
     using S = LargeSmem;
@@ -285,8 +273,8 @@ __global__ void __launch_bounds__(LARGE_NT, 1) score_large_kernel(const __grid_c
             uint32_t k = 0;
             int sg = 0;
             for (int item = blockIdx.x; item < a.n_items; item += gridDim.x) {
-                while (item >= a.seg.item0[sg + 1]) ++sg;
-                const int row0 = ((item - a.seg.item0[sg]) / a.NVC) * N;
+                advance_segment(a.seg, item, sg);
+                const int row0 = ((item - a.seg.tile0[sg]) / a.NVC) * N;
                 for (int h0 = 0; h0 < N; h0 += 128)
                     for (int w0 = 0; w0 < N; w0 += 64, ++k) {
                         const uint32_t set = k & 1u;
@@ -350,8 +338,8 @@ __global__ void __launch_bounds__(LARGE_NT, 1) score_large_kernel(const __grid_c
         int first_block = 0;                                       // this tile's slabs [0, first_block) are already stored
         int sg = 0;
         for (; item < a.n_items; item += gridDim.x) {
-            while (item >= a.seg.item0[sg + 1]) ++sg;
-            const int map = (item - a.seg.item0[sg]) / a.NVC, vc = item % a.NVC;       // map within its segment, v-chunk
+            advance_segment(a.seg, item, sg);
+            const int map = (item - a.seg.tile0[sg]) / a.NVC, vc = item % a.NVC;       // map within its segment, v-chunk
             const int v0 = vc * 128, MV = min(128, N - v0);
             const int nitem = item + (int)gridDim.x;               // what this CTA works on next
 

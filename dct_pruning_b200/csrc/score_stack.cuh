@@ -47,61 +47,11 @@
 // the Bx_hi pass only (the Bx_lo pass would add exact zeros).  fp16 (11 significant bits) splits exactly into a bf16 hi / lo pair: it
 // is widened in registers and runs the fp32 split.
 #pragma once
-#include <cuda.h>
-#include <cuda_fp16.h>
 #include <type_traits>
-#include "score_umma.cuh"
+#include "score_common.cuh"
+#include "umma.cuh"
 
 namespace dctp {
-
-// element type of the activation a score kernel reads (the values of DCTP_DTYPE_* in include/dctp.h)
-constexpr int IN_F32 = 0, IN_BF16 = 1, IN_F16 = 2;
-__host__ __device__ constexpr int in_bytes(int in) { return in == IN_F32 ? 4 : 2; }
-
-// element i of a 16-bit stream as fp32 (exact)
-template <int IN>
-__device__ __forceinline__ float in16_to_float(const uint16_t* x, long long i) {
-    if constexpr (IN == IN_BF16) return __uint_as_float(static_cast<uint32_t>(x[i]) << 16);
-    else return __half2float(__ushort_as_half(x[i]));
-}
-// two packed fp16 values (the first in the low half) as fp32
-__device__ __forceinline__ float2 f16x2_to_float2(uint32_t p) {
-    __half2 h;
-    memcpy(&h, &p, 4);
-    return __half22float2(h);
-}
-
-// detail::map_energy64 of map m of a dense stream of element type IN (x: the stream's first element)
-template <int IN>
-__device__ __forceinline__ double map_energy64_in(const void* x, long long m, int NN, int N) {
-    if constexpr (IN == IN_F32) {
-        return detail::map_energy64(static_cast<const float*>(x) + m * NN, N);
-    } else {
-        const uint16_t* p = static_cast<const uint16_t*>(x) + m * NN;
-        double s = 0.0;
-#pragma unroll 1
-        for (int i = 0; i < N * N; ++i) {
-            const double e = in16_to_float<IN>(p, i);
-            if (!isfinite(e)) return __longlong_as_double(0x7FF8000000000000ll);
-            s = fma(e, e, s);
-        }
-        return s;
-    }
-}
-
-constexpr int SCORE_MAX_SEG = 16;   // activations (hook sites of the same map side) one launch can score
-
-// One dense activation of a launch: all its scored maps back to back.  A launch walks the tiles of its segments in order;
-// tile t belongs to segment s with tile0[s] <= t < tile0[s + 1].
-struct ScoreSegments {
-    int n_seg;
-    int tile0[SCORE_MAX_SEG + 1];
-    int n_maps[SCORE_MAX_SEG], c_count[SCORE_MAX_SEG];
-    long long total_elems[SCORE_MAX_SEG];                // n_maps * NN
-    const void* x[SCORE_MAX_SEG];                        // first scored element (of the kernel's IN type), 16-B aligned
-    double* accum[SCORE_MAX_SEG];                        // fp64 [c_count] of the site
-};
-struct ScoreTensorMaps { CUtensorMap m[SCORE_MAX_SEG]; };
 
 struct StackArgs {
     ScoreSegments seg;
@@ -112,7 +62,7 @@ struct StackArgs {
     uint32_t idesc1, idesc2;
     uint32_t lbo1;                  // Bx: byte distance between consecutive 8-element k-chunks (2048 + 16 u, u chosen per side for conflict-free stores)
     const uint32_t* a_img;          // [128][32] packed bf16 pairs: the stacked basis as it sits in TMEM
-    const uint8_t* c2_hi;           // stage-2 basis as a shared-memory operand image (hi, lo): C2_HALF bytes each
+    const uint8_t* c2_hi;           // stage-2 basis as a shared-memory operand image (hi, lo): OperandImage64::BYTES each
     const uint8_t* c2_lo;
     const uint16_t* table;          // [tile_vec] (VEC 4) / [2 * tile_vec] (VEC 2) byte offsets of a float4's pieces in Bx
     uint32_t table_bytes;
@@ -126,19 +76,16 @@ struct StackSmem {
     static constexpr uint32_t NSTG = 3, STG_STRIDE = 32768;              // TMA ring: fp32 tiles of at most 32 KB
     static constexpr uint32_t LBO1_MAX = 128 * 16 + 16 * 7;              // Bx: k-chunk c of row n at c * lbo1 + n * 16; lbo1 = 2048 + 16 u spreads the banks
     static constexpr uint32_t BX_HALF = 8 * LBO1_MAX;                    // 17280
-    static constexpr uint32_t LBO2 = 64 * 16 + 16;                       // stage-2 basis, same layout
-    static constexpr uint32_t C2_HALF = 8 * LBO2;                        // 8320
     static constexpr uint32_t OFF_BX = NSTG * STG_STRIDE;
     static constexpr uint32_t NBX = 3;                                   // room for three Bx buffers (hi | lo each); how many a kernel uses: see NBXK
     static constexpr uint32_t OFF_C2 = OFF_BX + 2 * NBX * BX_HALF;
-    static constexpr uint32_t OFF_TABLE = OFF_C2 + 2 * C2_HALF;
+    static constexpr uint32_t OFF_TABLE = OFF_C2 + 2 * OperandImage64::BYTES;   // stage-2 basis (hi | lo)
     static constexpr uint32_t TABLE_MAX = 8192;
     static constexpr uint32_t OFF_RED = OFF_TABLE + TABLE_MAX;
     static constexpr uint32_t OFF_BARS = OFF_RED + 256;
     static constexpr uint32_t OFF_SLOT = OFF_BARS + 256;
     static constexpr uint32_t TOTAL = OFF_SLOT + 128;
 };
-
 
 // Role groups: converters in NCG groups (group g converts the CTA's tiles g, g + NCG, ...), NE1G epilogue-1 groups and NE2G
 // epilogue-2 groups (group g takes the CTA's tiles g, g + NE1G / NE2G, ...).
@@ -187,7 +134,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
     const uint32_t TM_A2 = TM_D1 + 2 * d1_stride, TM_D2 = TM_A2 + 128;
     const uint32_t nb2 = TM_D2 + 128 <= 512 ? 2u : 1u;                    // a second D2 buffer when D1 is at most 112 columns wide
     const uint32_t STEP1 = (2 * a.lbo1) >> 4;                             // one k-step (two 8-element chunks) in descriptor units
-    constexpr uint32_t STEP2 = (2 * S::LBO2) >> 4;
+    constexpr uint32_t STEP2 = (2 * OperandImage64::LBO) >> 4;
 
     extern __shared__ __align__(1024) uint8_t smem[];
     // (the warp index comes out of a shuffle so that the compiler knows it is warp-uniform: role addresses stay in uniform registers)
@@ -238,12 +185,12 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         // Every global load of the prologue is issued before the first store (the stores are to shared memory / TMEM, which the compiler
         // will not move loads across): one exposed L2 / HBM latency instead of four - 3.4 -> ~1.5 us of the ~10 us a launch costs beyond
         // its bytes, which is what the 6-50 MB launches of the small layers are made of.
-        static_assert(2 * PNT * 16 >= S::C2_HALF && PNT * 16 >= S::TABLE_MAX, "prologue loads are unrolled for these sizes");
+        static_assert(2 * PNT * 16 >= OperandImage64::BYTES && PNT * 16 >= S::TABLE_MAX, "prologue loads are unrolled for these sizes");
         uint4 c2h[2], c2l[2], tb = make_uint4(0, 0, 0, 0), ai[8];
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             const uint32_t off = (ptid + i * PNT) * 16;
-            if (off < S::C2_HALF) {
+            if (off < OperandImage64::BYTES) {
                 c2h[i] = *reinterpret_cast<const uint4*>(a.c2_hi + off);
                 c2l[i] = *reinterpret_cast<const uint4*>(a.c2_lo + off);
             }
@@ -257,9 +204,9 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
 #pragma unroll
         for (int i = 0; i < 2; ++i) {
             const uint32_t off = (ptid + i * PNT) * 16;
-            if (off < S::C2_HALF) {
+            if (off < OperandImage64::BYTES) {
                 *reinterpret_cast<uint4*>(c2 + off) = c2h[i];
-                *reinterpret_cast<uint4*>(c2 + S::C2_HALF + off) = c2l[i];
+                *reinterpret_cast<uint4*>(c2 + OperandImage64::BYTES + off) = c2l[i];
             }
         }
         if (ptid * 16 < a.table_bytes) *reinterpret_cast<uint4*>(smem + S::OFF_TABLE + ptid * 16) = tb;
@@ -301,9 +248,6 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
     bool dead = false;
     // segment of a tile: the roles walk the tiles in increasing order, so each keeps a cursor.  A segment whose stream does not end
     // on a 32-element row (128 bytes in fp32, 64 in 16-bit) has its last tile converted from global memory (that row is not in the tensor map).
-    auto seg_of = [&](int tile, int& sg) {
-        while (tile >= a.seg.tile0[sg + 1]) ++sg;
-    };
     auto is_tail = [&](int tile, int sg) {
         return tile == a.seg.tile0[sg + 1] - 1 && (a.seg.total_elems[sg] & 31) != 0;
     };
@@ -322,7 +266,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
             uint32_t it = 0;
             int sg = 0;
             for (int tile = first; tile < a.num_tiles; tile += stride) {
-                seg_of(tile, sg);
+                advance_segment(a.seg, tile, sg);
                 if (is_tail(tile, sg)) continue;
                 const uint32_t s = it % S::NSTG;
                 TR_START();
@@ -371,9 +315,9 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         // ================================================================ MMA issuer, stage 2: D2 = A2 * C^T (hi*hi + lo*hi + hi*lo)
         if (elect_one()) {
             tr_me = tr_on;
-            const uint64_t desc2 = make_smem_desc(0, S::LBO2, 128, SWIZZLE_NONE);
+            const uint64_t desc2 = make_smem_desc(0, OperandImage64::LBO, 128, SWIZZLE_NONE);
             const uint32_t lo_c2_hi = static_cast<uint32_t>(desc2) + (smem_u32(c2) >> 4);
-            const uint32_t lo_c2_lo = lo_c2_hi + (S::C2_HALF >> 4);
+            const uint32_t lo_c2_lo = lo_c2_hi + (OperandImage64::BYTES >> 4);
             uint32_t m = 0;
             for (int tile = first; tile < a.num_tiles; tile += stride, ++m) {
                 const uint32_t b = m & 1u;
@@ -415,7 +359,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         int sg = 0;
         tr_me = tr_on && tid == 0;
         for (int tile = first; tile < a.num_tiles; tile += stride, ++n) {
-            seg_of(tile, sg);
+            advance_segment(a.seg, tile, sg);
             const bool tail = is_tail(tile, sg);
             if (n % NCG != cg) {                                           // the other group's tile: only keep the TMA count in step
                 if (!tail) ++it;
@@ -694,7 +638,7 @@ __global__ void __launch_bounds__(stack_warps(NCONV) * 32, 1) score_stack_kernel
         uint32_t chan0 = 0, chan_step = 0;
         tr_me = tr_on && warp == W_E2 && lane == 0;
         for (int tile = first + (int)eg2 * stride; tile < a.num_tiles; tile += NE2G * stride, n += NE2G) {
-            seg_of(tile, sg);
+            advance_segment(a.seg, tile, sg);
             const uint32_t C = static_cast<uint32_t>(a.seg.c_count[sg]), seg_maps = static_cast<uint32_t>(a.seg.n_maps[sg]);
             double* const accum = a.seg.accum[sg];
             const uint32_t pb = n & 1u, b2 = nb2 == 2 ? pb : 0u;           // barrier pair by tile parity, buffer

@@ -25,7 +25,8 @@
 // TMEM lanes) each, sharing A' and C: 3 slots for maps up to 64 wide, 6 for maps up to 32 or 16 wide (the
 // per-tile dependency chain is what bounds this kernel, so smaller tiles get more slots).
 #pragma once
-#include "score_umma.cuh"
+#include "score_common.cuh"
+#include "umma.cuh"
 
 namespace dctp {
 

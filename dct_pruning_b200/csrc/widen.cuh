@@ -2,7 +2,7 @@
 // fp32 copy (scratch on the caller's stream), and the fp32 kernels score that copy.  Only the stacked-basis and Kronecker kernels read
 // 16-bit input themselves (score_stack.cuh, score_kron.cuh).
 #pragma once
-#include "score_stack.cuh"
+#include "score_common.cuh"
 
 namespace dctp {
 
